@@ -2,8 +2,11 @@
 """Benchmark of the fast WordPiece encode path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload en|ru|ja|zh|adv]
+                    [--dump-outputs DIR]
 
-One step = one pass of the encode path over one batch of synthetic text.
+One step = one pass of the encode path over one batch of synthetic text.  The text and the vocabulary come
+from fixed seeds, so the same arguments give the same inputs in every run; --dump-outputs DIR writes what the
+last timed step returned (see dump_outputs) so that two builds can be compared output for output.
 
 * N = 1: the batch is BASELINE.json configs[1] — 1 GiB of English-like text, the 29k-entry bert-shaped
   vocabulary, resident in HBM before the timed region.  The line also carries a compact `configs` object
@@ -57,7 +60,13 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the other configurations / latency / drop-in legs")
     ap.add_argument("--no-gather", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the ids of the last timed step as DIR/*.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU path; it is not available with --impl reference")
+    return args
 
 
 def workload_name(args, world: int = 1) -> str:
@@ -263,6 +272,35 @@ def emit(line: dict):
         sys.stdout.flush()
     else:
         os.write(_REAL_STDOUT, data)
+
+
+DUMP_SAMPLE = 1 << 21  # ids kept by --dump-outputs over all ranks: 2 x 16 MiB of float64 (ids and positions)
+
+
+def dump_outputs(out_dir: str, d_ids, n_ids: int, vocab_size: int, sample: int = DUMP_SAMPLE, first_id: int = 0):
+    """--dump-outputs: what a caller of the timed path receives, the id count and the id array (float64, which
+    holds every id and position exactly).  A 1 GiB step yields ~300 M ids, so the array is written as a fixed
+    seeded sample of at most `sample` positions (all of them for smaller outputs), next to the histogram of
+    ALL ids, which a single changed id anywhere alters:
+        n_ids.npy                 [n_ids]
+        ids_sample.npy            ids at the positions below
+        ids_sample_positions.npy  sorted positions, first_id + index into this call's id array
+        id_histogram.npy          occurrences of id -1 (no [UNK] in the vocabulary), 0, 1, ..., vocab_size - 1
+    N > 1: every rank writes its shard's files; first_id is the shard's offset in the whole corpus's ids, so
+    the positions of all ranks index one array, and `sample` is DUMP_SAMPLE / N to keep the total bounded."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    ids = d_ids[:n_ids]
+    if n_ids <= sample:
+        pos = np.arange(n_ids, dtype=np.int64)
+    else:
+        pos = np.unique(np.random.default_rng(0).integers(0, n_ids, sample))
+    values = ids[torch.from_numpy(pos).to(ids.device)].cpu().numpy()
+    hist = torch.bincount(ids.long() + 1, minlength=vocab_size + 1).cpu().numpy()
+    for name, a in (("n_ids", np.array([n_ids])), ("ids_sample", values), ("ids_sample_positions", first_id + pos),
+                    ("id_histogram", hist)):
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float64))
 
 
 # ------------------------------------------------------------------ helper legs (N = 1)
@@ -601,6 +639,11 @@ def main():
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     ms_step = ms_total / args.steps
     assert int(d_cnt.item()) == n_ids or world > 1
+    if args.dump_outputs:
+        # the last timed step's own count (d_cnt, or this rank's gathered count) and ids
+        n_last = int(d_cnt.item()) if world == 1 else int(counts_t[rank].item())
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"),
+                     d_ids, n_last, len(vocab_tokens), sample=DUMP_SAMPLE // world, first_id=offsets[rank])
 
     total_bytes = sum_over_ranks(float(n_bytes))
     total_ids = sum_over_ranks(float(n_ids))

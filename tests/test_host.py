@@ -42,33 +42,6 @@ def test_cpp_entry_points_are_exported():
         assert sig in out, sig
 
 
-def test_reference_drivers_compile_against_the_drop_in_headers(tmp_path):
-    """SURVEY 8(b): the reference's own drivers (tests/tests.cpp, tests/runner.cpp) include "src/utils.hpp" and
-    "src/word_piece.hpp" and use word_piece::fast::*, utils::globalThreadPool, utils::writeToFile and
-    WordPieceVocabulary::kDefaultUnkTokenId.  Both must compile UNCHANGED with include/ on the include path.  The
-    only thing added is a declaration of the out-of-scope `linear` half they also call (a test-only header).
-    Build container only: /root/reference does not exist on the GPU box."""
-    import shutil
-    import subprocess
-
-    ref_tests = "/root/reference/tests"
-    cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else shutil.which("g++")
-    if not os.path.isdir(ref_tests) or not cxx:
-        pytest.skip("reference sources (or g++) not present")
-    stub = tmp_path / "linear_decl.hpp"
-    stub.write_text(
-        "#include <cstddef>\n#include <string>\n#include <vector>\n"
-        "namespace word_piece { namespace linear {\n"
-        "std::vector<int> encode(const std::string &, const std::vector<std::string> &);\n"
-        "std::vector<int> encode(const std::string &, const std::string &);\n"
-        "void encodeExternal(const std::string &, const std::string &, const std::string &, size_t);\n"
-        "} }\n")
-    for driver in ("runner.cpp", "tests.cpp"):
-        r = subprocess.run([cxx, "-std=c++17", "-fsyntax-only", "-include", str(stub), "-I", os.path.join(ROOT, "include"),
-                            os.path.join(ref_tests, driver)], capture_output=True, text=True)
-        assert r.returncode == 0, f"{driver}:\n{r.stderr[-2000:]}"
-
-
 def test_runner_argv_contract_without_a_device(tmp_path):
     """tests/runner.cpp:13-65 — everything the CLI decides before it encodes: argument count, the 50 MB floor of
     memory_limit_mb, external mode without a limit, unknown and out-of-scope modes; errors are uncaught
