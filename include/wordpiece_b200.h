@@ -216,6 +216,12 @@ size_t wp_debug_displaced_singles(const wp_vocab *v, uint32_t min_displacement, 
 size_t wp_debug_word_slots(const wp_vocab *v);
 size_t wp_debug_static_words(const wp_vocab *v);
 uint32_t wp_debug_word_lookup(const wp_vocab *v, const char *text, size_t len, int32_t *ids_out, uint32_t *displacement);
+/* the limits the kernels were compiled with, in this order: tile bytes, LONG segment bytes, K1 segments per tile,
+ * K3 segments per block, K3 staged ids per block, ids of a segment K3 copies warp-wise (more than this), K3 mixed-path
+ * limit of such segments per block, K2L bytes per round, word-key bytes, ids of a word slot, the 5-bit id count
+ * of a slow segment (at this value the count is in the slow entry), ids a slow entry holds inline.  Writes at most
+ * `cap` of them to `out`; returns their number (no device needed) */
+size_t wp_debug_kernel_geometry(uint32_t *out, size_t cap);
 
 #ifdef __cplusplus
 }

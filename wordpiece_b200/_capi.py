@@ -95,6 +95,7 @@ EXPORTED_SYMBOLS = [
     "wp_debug_word_slots",
     "wp_debug_static_words",
     "wp_debug_word_lookup",
+    "wp_debug_kernel_geometry",
     "wp_debug_plan_chunks",
     "wp_debug_stage",
 ]
@@ -181,6 +182,8 @@ def load_library() -> C.CDLL:
     L.wp_debug_displaced_singles.restype = sz
     L.wp_debug_word_lookup.argtypes = [vp, C.c_char_p, sz, C.POINTER(C.c_int32), C.POINTER(C.c_uint32)]
     L.wp_debug_word_lookup.restype = C.c_uint32
+    L.wp_debug_kernel_geometry.argtypes = [C.POINTER(C.c_uint32), sz]
+    L.wp_debug_kernel_geometry.restype = sz
     _lib = L
     return L
 
@@ -197,6 +200,22 @@ def kernel_launch_count() -> int:
 
 def tile_bytes() -> int:
     return int(load_library().wp_tile_bytes())
+
+
+KERNEL_GEOMETRY_FIELDS = ("tile", "long_segment_bytes", "seg_cap", "scatter_segs", "scatter_stage", "scatter_big",
+                          "mixed_max_big", "long_block", "word_key_bytes", "word_max_ids", "seg_slow_count_max",
+                          "inline_ids")
+
+
+def kernel_geometry() -> dict:
+    """The limits the kernels were compiled with (``wp_debug_kernel_geometry``, test hook, no device):
+    ``KERNEL_GEOMETRY_FIELDS`` -> value."""
+    L = load_library()
+    n = int(L.wp_debug_kernel_geometry(None, 0))
+    buf = (C.c_uint32 * n)()
+    L.wp_debug_kernel_geometry(buf, n)
+    assert n == len(KERNEL_GEOMETRY_FIELDS), n
+    return {k: int(buf[i]) for i, k in enumerate(KERNEL_GEOMETRY_FIELDS)}
 
 
 def _as_bytes(x) -> bytes:

@@ -1863,6 +1863,8 @@ uint32_t wp_debug_word_lookup(const wp_vocab *v, const char *text, size_t len, i
   return cnt;
 }
 
+size_t wp_debug_kernel_geometry(uint32_t *out, size_t cap) { return wp::kernel_geometry(out, out ? cap : 0); }
+
 /* The chunk plan of the host-buffer pipeline for a text (no device needed): writes up to `cap` cut offsets
  * (first 0, last n) to `cuts`, returns their number, or 0 if some stretch has no ASCII space to cut at. */
 size_t wp_debug_plan_chunks(const char *text, size_t n, size_t chunk, size_t *cuts, size_t cap) {

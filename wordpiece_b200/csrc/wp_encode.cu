@@ -2306,6 +2306,14 @@ cudaError_t launch_publish_count(const CallCounters *call, uint32_t parity, unsi
 
 uint32_t encode_tile_bytes() { return TILE; }
 uint32_t scatter_block_segments() { return SCATTER_SEGS; }
+size_t kernel_geometry(uint32_t *out, size_t cap) {
+  const uint32_t g[] = {TILE, LONG_SEGMENT_BYTES, WP_K1_SEG_CAP, SCATTER_SEGS, SCATTER_STAGE, SCATTER_BIG, MIXED_MAX_BIG,
+                        LONG_BLOCK, WORD_KEY_BYTES, WORD_MAX_IDS, SEG_SLOW_COUNT_MAX,
+                        3u /* ids K2's result form of a slow entry holds inline (wp_match_kernel) */};
+  const size_t n = sizeof(g) / sizeof(g[0]);
+  for (size_t i = 0; i < n && i < cap; i++) out[i] = g[i];
+  return n;
+}
 
 cudaError_t launch_encode_range(const EncodeParams &P, int sm_count, cudaStream_t stream, uint64_t *launches,
                                 cudaEvent_t *timing, unsigned phases) {

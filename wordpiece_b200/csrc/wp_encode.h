@@ -153,6 +153,9 @@ cudaError_t launch_text_offsets(const EncodeParams &P, uint32_t i0, uint32_t i1,
 
 uint32_t encode_tile_bytes();
 uint32_t scatter_block_segments();
+// The compiled limits of the kernels, in the order of wp_debug_kernel_geometry (wordpiece_b200.h); returns their
+// number and writes at most `cap` of them.
+size_t kernel_geometry(uint32_t *out, size_t cap);
 // Enqueue the kernels of one range: PHASE_SPLIT = K1, PHASE_MATCH = K2 + K2L, PHASE_SCATTER = K3 (the host
 // may put the phases of a range on different streams to overlap consecutive ranges).  *launches is
 // incremented per kernel launched.  `timing` (optional, all phases only): 4 events recorded around the
