@@ -124,3 +124,19 @@ def test_batch_pipeline_of_parts(gpu_device, monkeypatch, part):
     _check_batch(v, o, texts, f"parts of {part}")
     _check_batch(v, o, texts[:5], "then a small batch on the same handle")
     v.close()
+
+
+def test_batch_repeat_after_void_part_switches_k1_mode(gpu_device, monkeypatch):
+    """A pipelined batch whose part 0 overflows the default id spill of its first range (a space-free word of
+    40 000 ids) while part 1, never finished before the whole batch is repeated as one part, holds a tile of
+    4 096 segments: the repeat trips the dense-tile flag of the regular K1 and must itself be repeated with the
+    full-capacity K1, as a single call would be."""
+    from wordpiece_b200 import Vocab
+
+    monkeypatch.setenv("WORDPIECE_B200_RANGE_BYTES", "4096")
+    monkeypatch.setenv("WORDPIECE_B200_MEMO", "0")
+    monkeypatch.setenv("WORDPIECE_B200_BATCH_PART", "4096")
+    vocab = ["[UNK]", "a", "##a", "!"]
+    v = Vocab(vocab, device=gpu_device)
+    _check_batch(v, Oracle(vocab), [b"a" * 40000, b"!" * 8192], "void part, then a dense tile")
+    v.close()

@@ -1,8 +1,8 @@
 #!/usr/bin/env python3
 """word_piece::fast::encode(std::string, vector<string>) on 1 GiB through the C++ helper (lib/dropin_bench) under
 combinations of the host-copy switches: WORDPIECE_B200_COPY_THREADS, WORDPIECE_B200_STREAM_STORES (staging
-copies in), WORDPIECE_B200_STREAM_OUT (ids out into the caller's vector); `--set hugepages`: the transparent-huge-page
-advice on the result vector on / off (WORDPIECE_B200_HUGEPAGES).   python tools/dropin_sweep.py [--mib 1024] [--set ...]"""
+copies in); `--set hugepages`: the transparent-huge-page advice on the result vector on / off
+(WORDPIECE_B200_HUGEPAGES).   python tools/dropin_sweep.py [--mib 1024] [--set ...]"""
 import argparse
 import json
 import os

@@ -147,11 +147,6 @@ struct wp_vocab {
   cudaEvent_t last_done = nullptr;
   bool use_ticket = false;  // K1 hands its tiles out by ticket (set for good once a look-back has stalled, see wp_encode.cu)
   bool dense_tiles = false; // K1 with full-capacity segment lists (set for good once a tile overflowed the regular ones)
-  // overlap of consecutive ranges (see enqueue_encode): K2/K2L/K3 run on a second, high-priority stream
-  cudaStream_t s_aux = nullptr;
-  cudaEvent_t ev_split[2] = {nullptr, nullptr};    // K1 of the range in scratch half b is done
-  cudaEvent_t ev_scatter[2] = {nullptr, nullptr};  // K3 of the range in scratch half b is done (the half is free)
-  cudaEvent_t ev_match = nullptr;                  // K2 of a warm-up range is done (its words are all recorded)
   // optional per-kernel timing (wp_set_kernel_timing): events around K1/K2/K3 of every range
   bool timing = false;
   std::vector<cudaEvent_t> timing_events;  // 4 per range of the last call
@@ -307,7 +302,6 @@ wp_status enqueue_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_
   }
   const size_t range_bytes = n_bytes < range_max ? n_bytes : range_max;
   const Workspace w = plan_workspace(range_bytes, spill_ids ? spill_ids : range_bytes + tile);
-  wp_status st = WP_OK;
   if (!v->last_done) WP_CUDA(cudaEventCreateWithFlags(&v->last_done, cudaEventDisableTiming));
   WP_CUDA(cudaStreamWaitEvent(stream, v->last_done, 0));  // (a never-recorded event does not block)
   WP_CUDA(cudaMemsetAsync(v->d_call, 0, sizeof(wp::CallCounters), stream));
@@ -370,14 +364,14 @@ wp_status enqueue_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_
     P.id_offsets = batch->d_offsets;
   }
   // batch calls: the texts [i0, i1) that start in the range whose K3 was just enqueued get their id offsets
-  auto text_offsets = [&](cudaStream_t s) -> cudaError_t {
+  auto text_offsets = [&]() -> cudaError_t {
     if (!batch) return cudaSuccess;
     const unsigned long long lo = static_cast<unsigned long long>(P.first_tile) * tile;
     const unsigned long long hi = lo + static_cast<unsigned long long>(P.n_tiles) * tile;
     const unsigned long long *b = batch->h_bounds, *e = b + batch->n_texts;
     const uint32_t i0 = static_cast<uint32_t>(std::lower_bound(b, e, lo) - b);
     const uint32_t i1 = static_cast<uint32_t>(std::lower_bound(b, e, hi) - b);
-    return wp::launch_text_offsets(P, i0, i1, s, &launches);
+    return wp::launch_text_offsets(P, i0, i1, stream, &launches);
   };
   // Two small ranges first (2 MiB, 8 MiB): the first fills the word memo — its own unsettled words all go
   // through K2 — the second shows whether the text repeats its words (memo_worthwhile), so that the bulk of
@@ -400,130 +394,84 @@ wp_status enqueue_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_
   }
   const uint32_t n_ranges = static_cast<uint32_t>(ranges.size());
 
-  // OVERLAP of consecutive ranges — an EXPERIMENT, off unless WORDPIECE_B200_OVERLAP=1: every K1 goes to the
-  // caller's stream, K2/K2L/K3 to a second, higher-priority stream, and the scratch is doubled (range r uses
-  // half r & 1).  Order kept by events: K2(r) after K1(r); K1(r+2) after K3(r) (the scratch half is free);
-  // K3(r) after K3(r-1) (stream order: the id offset chain).  The words K2 records while the next K1 is
-  // already running are tagged with their epoch and that K1 does not use them (wp_table.h), so no slot is
-  // read while it is written; during the warm-up ranges K1 waits for the K2 before it instead.  Ids do not
-  // depend on any of this.  MEASURED (1 GiB English, B200): 9.97 ms against 7.48 ms serial.  K1's seven
-  // resident tiles hold 62 720 of an SM's 65 536 registers, so K2's and K3's persistent blocks (sized to fill
-  // the GPU on their own) only get in by pushing K1 tiles out, and all three are bound by latency at their
-  // resident warp count, not by issue slots someone else could use: sharing an SM slows each by what it gives.
-  bool overlap = false;
-  if (const char *e = std::getenv("WORDPIECE_B200_OVERLAP")) overlap = std::atoi(e) != 0 && n_ranges >= 3 && !v->timing;
-  const size_t half = align_up(w.total, 256);
-  st = ensure_work(v, overlap ? 2 * half : w.total);
+  const wp_status st = ensure_work(v, w.total);
   if (st != WP_OK) return st;
-  if (overlap && !v->s_aux) {
-    int lo = 0, hi = 0;
-    WP_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));  // hi = greatest priority (numerically lowest)
-    WP_CUDA(cudaStreamCreateWithPriority(&v->s_aux, cudaStreamNonBlocking, hi));
-    for (int b = 0; b < 2; b++) {
-      WP_CUDA(cudaEventCreateWithFlags(&v->ev_split[b], cudaEventDisableTiming));
-      WP_CUDA(cudaEventCreateWithFlags(&v->ev_scatter[b], cudaEventDisableTiming));
-    }
-    WP_CUDA(cudaEventCreateWithFlags(&v->ev_match, cudaEventDisableTiming));
-  }
-  auto bind_scratch = [&](uint8_t *base) {
-    P.counters = reinterpret_cast<wp::RangeCounters *>(base);
-    P.tile_state = reinterpret_cast<unsigned long long *>(base + w.off_tile_state);
-    P.block_state = reinterpret_cast<unsigned long long *>(base + w.off_block_state);
-    P.seg_result = reinterpret_cast<uint32_t *>(base + w.off_seg);
-    P.slow = reinterpret_cast<wp::SlowEntry *>(base + w.off_slow);
-    P.long_list = reinterpret_cast<uint32_t *>(base + w.off_long);
-    P.arena = reinterpret_cast<uint32_t *>(base + w.off_arena);
-  };
-  const uint32_t n_warmup = (use_memo && !warm) ? 2u : 0u;  // ranges 0 and 1 warm the memo up
+  uint8_t *const scratch = v->d_work;
+  P.counters = reinterpret_cast<wp::RangeCounters *>(scratch);
+  P.tile_state = reinterpret_cast<unsigned long long *>(scratch + w.off_tile_state);
+  P.block_state = reinterpret_cast<unsigned long long *>(scratch + w.off_block_state);
+  P.seg_result = reinterpret_cast<uint32_t *>(scratch + w.off_seg);
+  P.slow = reinterpret_cast<wp::SlowEntry *>(scratch + w.off_slow);
+  P.long_list = reinterpret_cast<uint32_t *>(scratch + w.off_long);
+  P.arena = reinterpret_cast<uint32_t *>(scratch + w.off_arena);
   for (uint32_t range = 0; range < n_ranges; range++) {
-    const uint32_t b = overlap ? (range & 1u) : 0u;
-    uint8_t *scratch = v->d_work + (overlap ? b * half : 0);
-    bind_scratch(scratch);
     P.first_tile = static_cast<uint32_t>(ranges[range].first);
     P.n_tiles = static_cast<uint32_t>(ranges[range].second);
     P.range_parity = range & 1u;
     P.range_index = warm ? range + 2 : range;
-    P.record_epoch = P.range_index + 1u < wp::WORD_EPOCH_MAX ? P.range_index + 1u : wp::WORD_EPOCH_MAX;
-    P.accept_epoch = wp::WORD_EPOCH_MAX;
-    if (!overlap) {
-      static const bool poison_scratch = std::getenv("WORDPIECE_B200_POISON_SCRATCH") != nullptr;
-      if (poison_scratch)  // (tests) everything a range must write before it reads, filled with 0xCD on the launching stream
-        WP_CUDA(cudaMemsetAsync(scratch + w.off_seg, 0xCD, w.total - w.off_seg, stream));
-      WP_CUDA(cudaMemsetAsync(scratch, 0, w.zero_bytes, stream));
-      cudaEvent_t *tev = nullptr;
-      if (v->timing) {
-        while (v->timing_events.size() < v->timing_used + 4) {
-          cudaEvent_t e;
-          WP_CUDA(cudaEventCreate(&e));
-          v->timing_events.push_back(e);
-        }
-        tev = v->timing_events.data() + v->timing_used;
-        v->timing_used += 4;
-      }
-      WP_CUDA(wp::launch_encode_range(P, v->sm_count, stream, &launches, tev));
-      WP_CUDA(text_offsets(stream));
-      continue;
-    }
-    // the K2 that ran (or runs) right before this K1: finished for the ranges after the warm-up ones (K1
-    // waits for it), possibly still recording otherwise — then its epoch (range index) is not accepted
-    const bool wait_match = range >= 1 && range <= n_warmup;
-    P.accept_epoch = wait_match || range == 0 ? wp::WORD_EPOCH_MAX : (P.range_index >= 1 ? P.range_index - 1u : 0u);
-    if (P.accept_epoch >= wp::WORD_EPOCH_MAX && !(wait_match || range == 0)) P.accept_epoch = wp::WORD_EPOCH_MAX - 1u;
-    if (range >= 2) WP_CUDA(cudaStreamWaitEvent(stream, v->ev_scatter[b], 0));
-    if (wait_match) WP_CUDA(cudaStreamWaitEvent(stream, v->ev_match, 0));
+    static const bool poison_scratch = std::getenv("WORDPIECE_B200_POISON_SCRATCH") != nullptr;
+    if (poison_scratch)  // (tests) everything a range must write before it reads, filled with 0xCD on the launching stream
+      WP_CUDA(cudaMemsetAsync(scratch + w.off_seg, 0xCD, w.total - w.off_seg, stream));
     WP_CUDA(cudaMemsetAsync(scratch, 0, w.zero_bytes, stream));
-    WP_CUDA(wp::launch_encode_range(P, v->sm_count, stream, &launches, nullptr, wp::PHASE_SPLIT));
-    WP_CUDA(cudaEventRecord(v->ev_split[b], stream));
-    WP_CUDA(cudaStreamWaitEvent(v->s_aux, v->ev_split[b], 0));
-    WP_CUDA(wp::launch_encode_range(P, v->sm_count, v->s_aux, &launches, nullptr, wp::PHASE_MATCH));
-    if (range < n_warmup) WP_CUDA(cudaEventRecord(v->ev_match, v->s_aux));
-    WP_CUDA(wp::launch_encode_range(P, v->sm_count, v->s_aux, &launches, nullptr, wp::PHASE_SCATTER));
-    WP_CUDA(text_offsets(v->s_aux));
-    WP_CUDA(cudaEventRecord(v->ev_scatter[b], v->s_aux));
+    cudaEvent_t *tev = nullptr;
+    if (v->timing) {
+      while (v->timing_events.size() < v->timing_used + 4) {
+        cudaEvent_t e;
+        WP_CUDA(cudaEventCreate(&e));
+        v->timing_events.push_back(e);
+      }
+      tev = v->timing_events.data() + v->timing_used;
+      v->timing_used += 4;
+    }
+    WP_CUDA(wp::launch_encode_range(P, v->sm_count, stream, &launches, tev));
+    WP_CUDA(text_offsets());
   }
-  if (overlap) {
-    // the caller's stream continues only when the last K3 (which is after every other kernel of the call) is done
-    WP_CUDA(cudaStreamWaitEvent(stream, v->ev_scatter[(n_ranges - 1) & 1u], 0));
-  }
-  const uint32_t range = n_ranges;
   WP_CUDA(cudaEventRecord(v->last_done, stream));
   g_launches.fetch_add(launches, std::memory_order_relaxed);
   info->n_tiles = static_cast<uint32_t>(n_tiles);
-  info->n_ranges = range;
+  info->n_ranges = n_ranges;
   info->launches = launches;
   return WP_OK;
 }
 
-// Wait for the enqueued call and collect its counters.  *overflow tells the caller to retry with a larger spill.
-wp_status finish_stats(wp_vocab *v, size_t n_bytes, const EnqueueInfo &info, cudaStream_t stream, bool *overflow) {
-  WP_CUDA(cudaMemcpyAsync(v->h_call, v->d_call, sizeof(wp::CallCounters), cudaMemcpyDeviceToHost, stream));
-  WP_CUDA(cudaStreamSynchronize(stream));
-  v->stats.n_bytes = n_bytes;
-  v->stats.n_ids = v->h_call->ids_total[info.n_ranges & 1u];
-  v->stats.n_tiles = info.n_tiles;
-  v->stats.dirty_tiles = v->h_call->dirty_tiles;
-  v->stats.long_segments = v->h_call->long_segments;
-  v->stats.memo_hits = v->h_call->memo_hits;
-  v->stats.kernel_launches = info.launches;
-  *overflow = v->h_call->overflow != 0;
-  if (v->h_call->stalled) v->use_ticket = true;  // a K1 look-back gave up: from now on tiles go by ticket
-  if (v->h_call->dense) v->dense_tiles = true;   // a tile with more segments than the regular K1's lists hold
-  return WP_OK;
+// The outcome of a finished call of n_bytes text bytes, from its counters (as copied to the host) and its
+// EnqueueInfo.  The K1 modes the call asked for are switched on for the handle for good, and its statistics are
+// added to *acc.  Returns true if the call's ids are void (a scratch capacity was exceeded): the call is then
+// repeated with the id spill left in *spill — unchanged if the overflow switched a K1 mode on, which is cure
+// enough, else one as large as the text.  Every repeat so turns on one of three one-way switches (ticket, dense
+// tiles, large spill), and kMaxAttempts bounds the repeats of every entry point.
+constexpr int kMaxAttempts = 1 + 3;
+bool absorb_call(wp_vocab *v, const wp::CallCounters &c, const EnqueueInfo &info, size_t n_bytes, wp_stats *acc,
+                 size_t *spill) {
+  const bool switched = (c.stalled && !v->use_ticket) || (c.dense && !v->dense_tiles);
+  if (c.stalled) v->use_ticket = true;  // a K1 look-back gave up: from now on tiles go by ticket
+  if (c.dense) v->dense_tiles = true;   // a tile with more segments than the regular K1's lists hold
+  acc->n_tiles += info.n_tiles;
+  acc->dirty_tiles += c.dirty_tiles;
+  acc->long_segments += c.long_segments;
+  acc->memo_hits += c.memo_hits;
+  acc->kernel_launches += info.launches;
+  if (!c.overflow) return false;
+  if (!switched) *spill = n_bytes + 4096;
+  return true;
 }
 
-// enqueue + wait, retrying once with a spill as large as the text if a walked segment outgrew the default
+// enqueue + wait, repeated while the ids are void (absorb_call)
 wp_status run_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_t *d_ids, size_t capacity,
                      cudaStream_t stream) {
   size_t spill = 0;
-  for (int attempt = 0; attempt < 3; attempt++) {
+  for (int attempt = 0; attempt < kMaxAttempts; attempt++) {
     EnqueueInfo info;
-    wp_status st = enqueue_encode(v, d_text, n_bytes, d_ids, capacity, stream, spill, &info);
+    const wp_status st = enqueue_encode(v, d_text, n_bytes, d_ids, capacity, stream, spill, &info);
     if (st != WP_OK) return st;
-    bool overflow = false;
-    st = finish_stats(v, n_bytes, info, stream, &overflow);
-    if (st != WP_OK) return st;
-    if (!overflow) return WP_OK;
-    if (!v->h_call->stalled && !v->h_call->dense) spill = n_bytes + 4096;  // (else: the same call again, other K1 mode)
+    WP_CUDA(cudaMemcpyAsync(v->h_call, v->d_call, sizeof(wp::CallCounters), cudaMemcpyDeviceToHost, stream));
+    WP_CUDA(cudaStreamSynchronize(stream));
+    wp_stats acc{};
+    if (absorb_call(v, *v->h_call, info, n_bytes, &acc, &spill)) continue;
+    v->stats = acc;
+    v->stats.n_bytes = n_bytes;
+    v->stats.n_ids = v->h_call->ids_total[info.n_ranges & 1u];
+    return WP_OK;
   }
   return fail(WP_ERR_CUDA, "internal scratch overflow");
 }
@@ -868,14 +816,8 @@ wp_status encode_pipelined(wp_vocab *v, const char *text, size_t n_bytes, int32_
     wp_vocab::PipeSlot &sl = v->slot[j % kPipeSlots];
     WP_CUDA(cudaEventSynchronize(sl.cmp_done));
     const size_t cnt = static_cast<size_t>(sl.h_call->ids_total[infos[j].n_ranges & 1u]);
-    overflow = overflow || sl.h_call->overflow != 0;
-    if (sl.h_call->stalled) v->use_ticket = true;
-    if (sl.h_call->dense) v->dense_tiles = true;
-    acc.n_tiles += infos[j].n_tiles;
-    acc.dirty_tiles += sl.h_call->dirty_tiles;
-    acc.long_segments += sl.h_call->long_segments;
-    acc.memo_hits += sl.h_call->memo_hits;
-    acc.kernel_launches += infos[j].launches;
+    size_t spill = 0;  // (a void chunk is not repeated: the caller encodes the whole text in one call instead)
+    if (absorb_call(v, *sl.h_call, infos[j], cuts[j + 1] - cuts[j], &acc, &spill)) overflow = true;
     counts[j] = cnt;
     offsets[j] = total;
     if (!overflow && cnt > 0 && total + cnt <= capacity) {
@@ -904,9 +846,7 @@ wp_status encode_pipelined(wp_vocab *v, const char *text, size_t n_bytes, int32_
     if (!stage_out || counts[j] == 0 || overflow || offsets[j] + counts[j] > capacity) return WP_OK;
     wp_vocab::PipeSlot &sl = v->slot[j % kPipeSlots];
     WP_CUDA(cudaEventSynchronize(sl.d2h_done));
-    // (streamed: the caller's fresh pages are written without being read into the caches first)
-    static const bool stream_out = std::getenv("WORDPIECE_B200_STREAM_OUT") != nullptr && std::atoi(std::getenv("WORDPIECE_B200_STREAM_OUT")) != 0;
-    pool.copy(ids + offsets[j], sl.h_ids, counts[j] * sizeof(int32_t), stream_out);
+    pool.copy(ids + offsets[j], sl.h_ids, counts[j] * sizeof(int32_t));
     return WP_OK;
   };
 
@@ -1081,12 +1021,6 @@ void wp_vocab_destroy(wp_vocab *v) {
     }
     for (cudaEvent_t e : v->timing_events) cudaEventDestroy(e);
     if (v->last_done) cudaEventDestroy(v->last_done);
-    for (int b = 0; b < 2; b++) {
-      if (v->ev_split[b]) cudaEventDestroy(v->ev_split[b]);
-      if (v->ev_scatter[b]) cudaEventDestroy(v->ev_scatter[b]);
-    }
-    if (v->ev_match) cudaEventDestroy(v->ev_match);
-    if (v->s_aux) cudaStreamDestroy(v->s_aux);
     if (v->s_h2d) cudaStreamDestroy(v->s_h2d);
     if (v->s_d2h) cudaStreamDestroy(v->s_d2h);
     cudaFree(v->d_call);
@@ -1494,17 +1428,11 @@ wp_status wp_encode_batch(wp_vocab *v, const char *const *texts, const size_t *l
     const PartPlan &p = parts[j];
     const size_t n = p.last - p.first;
     WP_CUDA(cudaEventSynchronize(b.cmp_done));
-    *overflow = b.h_call->overflow != 0;
-    if (b.h_call->stalled) v->use_ticket = true;
-    if (b.h_call->dense) v->dense_tiles = true;
+    size_t spill = 0;  // (a void part is not repeated: the whole batch is, as one part, see below)
+    *overflow = absorb_call(v, *b.h_call, infos[j], p.packed, &acc, &spill);
     if (*overflow) return WP_OK;
     const size_t cnt = static_cast<size_t>(b.h_offsets[n]);
     for (size_t i = 0; i < n; i++) offsets[p.first + i] = total + static_cast<size_t>(b.h_offsets[i]);
-    acc.n_tiles += infos[j].n_tiles;
-    acc.dirty_tiles += b.h_call->dirty_tiles;
-    acc.long_segments += b.h_call->long_segments;
-    acc.memo_hits += b.h_call->memo_hits;
-    acc.kernel_launches += infos[j].launches;
     cudaStream_t out_stream = n_parts > 1 ? v->s_d2h : v->stream;
     if (cnt > 0 && total + cnt <= capacity) {
       if (n_parts > 1) WP_CUDA(cudaStreamWaitEvent(out_stream, b.cmp_done, 0));
@@ -1544,29 +1472,28 @@ wp_status wp_encode_batch(wp_vocab *v, const char *const *texts, const size_t *l
     if (st != WP_OK) return st;
   }
   if (overflow) {
-    // a long segment outgrew the default id spill of some part (rare): the whole batch again as ONE part with a
-    // spill as large as the text, nothing pipelined
+    // the ids of some part are void (rare: a long segment outgrew the default id spill, or K1 has to change its
+    // mode): the whole batch again as ONE part with a spill as large as the text, nothing pipelined, repeated
+    // while its ids are void as in run_encode
     WP_CUDA(cudaStreamSynchronize(v->stream));
     if (n_parts > 1) WP_CUDA(cudaStreamSynchronize(v->s_d2h));
     parts.assign(1, plan_part(lens, 0, n_texts));
-    infos.assign(1, EnqueueInfo{});
-    acc = wp_stats{};
-    total = 0;
     wp_vocab::BatchSlot &b = v->bslot[0];
     wp_status st = ensure_batch_slot(b, parts[0], packed);
     if (st != WP_OK) return st;
     pack_part(b, parts[0], texts, lens);
-    st = enqueue_part(v, b, parts[0], v->stream, packed + 4096, false, packed, &infos[0]);
-    if (st != WP_OK) return st;
-    WP_CUDA(cudaEventSynchronize(b.cmp_done));
-    if (b.h_call->overflow) return fail(WP_ERR_CUDA, "internal scratch overflow");
+    size_t spill = packed + 4096;
+    for (int attempt = 0; overflow; attempt++) {
+      if (attempt == kMaxAttempts) return fail(WP_ERR_CUDA, "internal scratch overflow");
+      EnqueueInfo info;
+      st = enqueue_part(v, b, parts[0], v->stream, spill, false, packed, &info);
+      if (st != WP_OK) return st;
+      WP_CUDA(cudaEventSynchronize(b.cmp_done));
+      acc = wp_stats{};
+      overflow = absorb_call(v, *b.h_call, info, packed, &acc, &spill);
+    }
     const size_t cnt = static_cast<size_t>(b.h_offsets[n_texts]);
     for (size_t i = 0; i < n_texts; i++) offsets[i] = static_cast<size_t>(b.h_offsets[i]);
-    acc.n_tiles = infos[0].n_tiles;
-    acc.dirty_tiles = b.h_call->dirty_tiles;
-    acc.long_segments = b.h_call->long_segments;
-    acc.memo_hits = b.h_call->memo_hits;
-    acc.kernel_launches = infos[0].launches;
     if (cnt > 0 && cnt <= capacity) WP_CUDA(cudaMemcpyAsync(ids, b.d_ids, cnt * sizeof(int32_t), cudaMemcpyDeviceToHost, v->stream));
     total = cnt;
   }

@@ -45,10 +45,8 @@
 // Debug build (make variant NAME=bounds DEFS=-DWP_DEBUG_BOUNDS): every index into the scratch arrays, the lists in
 // shared memory and the output is checked where it is used; a violation prints its place and traps.  The
 // parity suites and the fuzz sweep are run under this build once per round (tools/gpu_bounds.sh).
-#if defined(WP_DEBUG_BOUNDS) || defined(WP_K2L_TRACE)
-#include <cstdio>
-#endif
 #ifdef WP_DEBUG_BOUNDS
+#include <cstdio>
 #define WP_CHECK(cond)                                                                                              \
   do {                                                                                                              \
     if (!(cond)) {                                                                                                  \
@@ -924,7 +922,6 @@ __global__ void __launch_bounds__(THREADS) wp_split_kernel(EncodeParams P) {
   // applied with predicates; only the further probes behind an occupied slot are a loop.
   constexpr int PER_TURN = WP_K1_PER_TURN;
   uint32_t my_dyn = 0, my_elig = 0;
-  const uint32_t accept_epoch = P.accept_epoch;
   const uint32_t word_mask = P.word_mask;
 #pragma unroll 1
   for (uint32_t base = 0; base < n_segs; base += PER_TURN * THREADS) {
@@ -966,7 +963,7 @@ __global__ void __launch_bounds__(THREADS) wp_split_kernel(EncodeParams P) {
       const bool look = state[u] == 1u;
       auto slot_hit = [&](const uint4 &a, const uint4 &m) {
         return (m.x & WORD_READY) && word_meta_len(m.x) == wlen[u] && a.x == key[u][0] && a.y == key[u][1] &&
-               a.z == key[u][2] && a.w == key[u][3] && word_meta_epoch(m.x) <= accept_epoch;
+               a.z == key[u][2] && a.w == key[u][3];
       };
       bool hit = slot_hit(sa[u], sb[u]);
       bool absent = sb[u].x == 0u;         // an empty slot ends the probe sequence: no such word
@@ -1151,10 +1148,6 @@ __global__ void __launch_bounds__(THREADS) wp_split_kernel(EncodeParams P) {
         out.off = 0;
         out.meta = ((sv >> 14) << 16) | SLOW_META_LONG | (static_cast<uint32_t>((pos >> 32) & 0xFFu) << 24);
         out.pos_lo = static_cast<uint32_t>(pos);
-#ifdef WP_K2L_TRACE
-        printf("K1 tile %u LONG k %u wpos %d pos %llu slot %u long_at %u seg %u (thread %d, lo %u hi %u)\n", rel_tile, k, wpos,
-               static_cast<unsigned long long>(pos), slow_base + i, long_at, out.seg, tid, lo, hi);
-#endif
         if (long_at < P.long_capacity) P.long_list[long_at] = slow_base + i;  // K2L's work list
         long_at++;
       } else {
@@ -1215,7 +1208,7 @@ __global__ void __launch_bounds__(MATCH_THREADS, WP_K2_BLOCKS) wp_match_kernel(E
   // K1 of this range is done, so the counters are final: every lane reads the same verdict
   const bool worth = memo_worthwhile(P.call->memo_lookups, P.call->memo_hits, P.range_index <= 1);
   if (blockIdx.x == 0 && tid == 0 && !worth) P.call->memo_off = 1u;
-  bool record = P.record_words != 0 && (P.range_index < 2 || worth) && P.record_epoch < WORD_EPOCH_MAX;
+  bool record = P.record_words != 0 && (P.range_index < 2 || worth);
 
   bool have = false;       // this lane holds an unfinished segment
   bool ext = false;        // the current node has children
@@ -1361,9 +1354,6 @@ __global__ void __launch_bounds__(MATCH_THREADS, WP_K2_BLOCKS) wp_match_kernel(E
       out[2] = t2;
       res = make_uint4(nid, area, 0u, 0u);
     }
-#ifdef WP_K2L_TRACE
-    if (seg_len > 300u) printf("K2 writes a result to slot %u: seg_len %u seg %u nid %u\n", ent_index, seg_len, seg, nid);
-#endif
     *reinterpret_cast<uint4 *>(&P.slow[ent_index]) = res;
     P.seg_result[seg] = SEG_RESULT_SLOW | (min(nid, SEG_SLOW_COUNT_MAX) << SEG_SLOW_INDEX_BITS) | ent_index;
     have = false;
@@ -1387,7 +1377,7 @@ __global__ void __launch_bounds__(MATCH_THREADS, WP_K2_BLOCKS) wp_match_kernel(E
           slot->ids[2] = t2;
           for (uint32_t q = 3; q < nid; q++) slot->ids[q] = __ldcg(out + q);
           __threadfence();
-          *reinterpret_cast<volatile unsigned int *>(&slot->meta) = word_meta(seg_len, nid, true, P.record_epoch);
+          *reinterpret_cast<volatile unsigned int *>(&slot->meta) = word_meta(seg_len, nid, true);
           placed = true;
         } else if (old == WORD_CLAIMED) {
           placed = true;  // another lane is writing this slot right now (most likely the same word)
@@ -1427,11 +1417,7 @@ static_assert((1 << LONG_LEVELS) >= LONG_BLOCK, "the strides must reach across a
 
 struct LongSmem {
   uint16_t jump[LONG_LEVELS][LONG_BLOCK];
-#ifdef WP_K2L_RANK32
-  uint32_t rank[LONG_BLOCK];
-#else
   uint16_t rank[LONG_BLOCK];
-#endif
   uint32_t delta[LONG_BLOCK];  // raw bytes from a piece start to the position behind its longest match (0 = none)
   int32_t id[LONG_BLOCK];
   uint8_t code[LONG_BLOCK];    // 0 = dropped / continuation byte, 1 = lead of an ordinary char
@@ -1457,10 +1443,6 @@ __global__ void __launch_bounds__(LONG_THREADS) wp_long_kernel(EncodeParams P) {
     if (sm.entry >= n_long) break;
     const uint32_t si = P.long_list[sm.entry];
     const SlowEntry ent = P.slow[si];
-#ifdef WP_K2L_TRACE
-    if (tid == 0)
-      printf("K2L entry %u takes slot %u: off %u meta 0x%x pos_lo %u seg %u\n", sm.entry, si, ent.off, ent.meta, ent.pos_lo, ent.seg);
-#endif
     const size_t start = static_cast<size_t>(ent.pos_lo) | (static_cast<size_t>(ent.meta >> 24) << 32);
     uint32_t len0, cls0;
     gnext(tv, start, &len0, &cls0);  // the start is a valid lead of a non-space class
@@ -1577,34 +1559,13 @@ __global__ void __launch_bounds__(LONG_THREADS) wp_long_kernel(EncodeParams P) {
         sm.code[i] = static_cast<uint8_t>(code);
         sm.delta[i] = delta;
         sm.id[i] = id;
-        sm.rank[i] = static_cast<decltype(sm.rank[0] + 0)>(LONG_END) & 0xFFFFu;
+        sm.rank[i] = static_cast<uint16_t>(LONG_END);
       }
       if (tid == 0) {
         sm.n_round = 0;
         sm.cur_next = b0 + n;  // (a block without a piece start: only dropped bytes)
       }
       __syncthreads();
-#ifdef WP_K2L_SERIAL
-      // (hunt build: the chain followed by one thread, as a cross-check of the ranking below)
-      if (tid == 0) {
-        uint32_t i = 0, cnt = 0;
-        while (i < n) {
-          if (sm.code[i] == 0) {
-            i++;
-            continue;
-          }
-          const uint32_t dl = sm.delta[i];
-          if (dl == 0) {
-            sm.failed = 1;
-            break;
-          }
-          out[n_out + cnt++] = sm.id[i];
-          i += dl;
-        }
-        sm.n_round = cnt;
-        sm.cur_next = b0 + i;
-      }
-#else
       // B: successors (the first valid lead at or behind the end of the match), doubled LONG_LEVELS - 1 times
 #pragma unroll 1
       for (uint32_t i = tid; i < n; i += LONG_THREADS) {
@@ -1640,25 +1601,7 @@ __global__ void __launch_bounds__(LONG_THREADS) wp_long_kernel(EncodeParams P) {
           if (r == LONG_END) continue;
           const uint32_t j = sm.jump[k][i];
           WP_CHECK(j == LONG_END || (j < n && j > i && r + (1u << k) < LONG_BLOCK));
-#ifdef WP_K2L_SNAP
-          (void)j;
-        }
-        // (hunt build: every thread first reads, then — behind a barrier — writes)
-        uint32_t tj[LONG_BLOCK / LONG_THREADS], tv2[LONG_BLOCK / LONG_THREADS];
-        int q = 0;
-        for (uint32_t i = tid; i < n; i += LONG_THREADS, q++) {
-          const uint32_t r = sm.rank[i];
-          const uint32_t j = r == LONG_END ? LONG_END : sm.jump[k][i];
-          tj[q] = j;
-          tv2[q] = r + (1u << k);
-        }
-        __syncthreads();
-        q = 0;
-        for (uint32_t i = tid; i < n; i += LONG_THREADS, q++) {
-          if (tj[q] != LONG_END) sm.rank[tj[q]] = static_cast<uint16_t>(tv2[q]);
-#else
           if (j != LONG_END) sm.rank[j] = static_cast<uint16_t>(r + (1u << k));
-#endif
         }
         __syncthreads();
       }
@@ -1679,14 +1622,8 @@ __global__ void __launch_bounds__(LONG_THREADS) wp_long_kernel(EncodeParams P) {
           }
         }
       }
-#endif
       __syncthreads();
       if (tid == 0) {
-#ifdef WP_K2L_TRACE
-        printf("K2L entry %u round b0 %llu n %u n_out %u n_round %u cur_next %llu failed %u seg_end %llu\n", sm.entry,
-               static_cast<unsigned long long>(b0), n, n_out, sm.n_round, sm.cur_next, sm.failed,
-               static_cast<unsigned long long>(seg_end));
-#endif
         sm.n_out = n_out + sm.n_round;
         sm.cur = sm.cur_next;
         if (sm.failed || sm.cur_next >= seg_end) sm.finished = 1;
@@ -1695,11 +1632,6 @@ __global__ void __launch_bounds__(LONG_THREADS) wp_long_kernel(EncodeParams P) {
     }
     if (tid == 0) {
       uint32_t cnt = sm.n_out;
-#ifdef WP_K2L_TRACE
-      printf("K2L entry %u done: start %llu seg_end %llu n_out %u failed %u word_first %u off %u\n", sm.entry,
-             static_cast<unsigned long long>(start), static_cast<unsigned long long>(seg_end), sm.n_out, sm.failed,
-             sm.word_first, sm.off);
-#endif
       if (sm.failed) {  // fast.cpp:79-88: the word's pieces are rolled back, one UNK stands for it
         cnt = sm.word_first + 1;
         P.arena[sm.off + sm.word_first] = static_cast<uint32_t>(V.unk_id);
@@ -2062,14 +1994,12 @@ __global__ void __launch_bounds__(SCATTER_THREADS, WP_K3_BLOCKS) wp_scatter_kern
     } else {
       // a block with unusually many ids (long words cut into many pieces).  Usually a few long segments among
       // ordinary ones: those are kept out of the staging buffer (scatter_mixed)
-#ifndef WP_K3_NO_MIXED
       const ScatterView view{P.seg_result, P.slow, P.arena, P.words, P.block_state, P.call, P.ids,
                              static_cast<unsigned long long>(P.capacity), P.slow_capacity, P.arena_capacity, P.range_parity};
       if (scatter_mixed(view, sm, first, n_segs, b, n_blocks, ids_in, total, at)) {  // uniform
         if (tid == 0) sm.block_index[(it + 1u) & 1u] = atomicAdd(&P.counters->scatter_ticket, 1u);
         continue;
       }
-#endif
       // otherwise: write directly
       if (warp == 0) {
         const unsigned long long base = lookback_walk(P.block_state, b, total, lane);
@@ -2316,7 +2246,7 @@ size_t kernel_geometry(uint32_t *out, size_t cap) {
 }
 
 cudaError_t launch_encode_range(const EncodeParams &P, int sm_count, cudaStream_t stream, uint64_t *launches,
-                                cudaEvent_t *timing, unsigned phases) {
+                                cudaEvent_t *timing) {
   // the opt-in to > 48 KB of dynamic shared memory is per device (K1 stays below it, but keep it explicit)
   static bool configured[64] = {false};
   int dev = 0;
@@ -2349,61 +2279,44 @@ cudaError_t launch_encode_range(const EncodeParams &P, int sm_count, cudaStream_
   cfg.stream = stream;
   cfg.attrs = attr;
 
-  if (phases != PHASE_ALL) timing = nullptr;
   if (timing) cudaEventRecord(timing[0], stream);
-  if (phases & PHASE_SPLIT) {
-    cfg.gridDim = dim3(P.n_tiles);
-    cfg.blockDim = dim3(THREADS);
-    cfg.numAttrs = window(P.words, P.persist_words_bytes, P.persist_words_ratio);
-    if (P.dense_tiles) {
-      cfg.dynamicSmemBytes = sizeof(TileSmemT<TILE>);
-      e = cudaLaunchKernelEx(&cfg, wp_split_kernel<TILE>, P);
-    } else {
-      cfg.dynamicSmemBytes = sizeof(TileSmemT<WP_K1_SEG_CAP>);
-      e = cudaLaunchKernelEx(&cfg, wp_split_kernel<WP_K1_SEG_CAP>, P);
-    }
-    if (e != cudaSuccess) return e;
-    if (launches) *launches += 1;
+  cfg.gridDim = dim3(P.n_tiles);
+  cfg.blockDim = dim3(THREADS);
+  cfg.numAttrs = window(P.words, P.persist_words_bytes, P.persist_words_ratio);
+  if (P.dense_tiles) {
+    cfg.dynamicSmemBytes = sizeof(TileSmemT<TILE>);
+    e = cudaLaunchKernelEx(&cfg, wp_split_kernel<TILE>, P);
+  } else {
+    cfg.dynamicSmemBytes = sizeof(TileSmemT<WP_K1_SEG_CAP>);
+    e = cudaLaunchKernelEx(&cfg, wp_split_kernel<WP_K1_SEG_CAP>, P);
   }
+  if (e != cudaSuccess) return e;
+  if (launches) *launches += 1;
   if (timing) cudaEventRecord(timing[1], stream);
-  if (phases & PHASE_MATCH) {
-    // = resident capacity (see the launch bound): one wave, large shares; a small range (a 4 KiB call is ONE tile)
-    // gets a grid to match — a tile has at most MAX_TILE_SLOW unsettled segments, 8 warps x 32 lanes take 256 at a time
-#ifdef WP_NO_GRID_TRIM
-    cfg.gridDim = dim3(sm_count * WP_K2_BLOCKS);
-#else
-    cfg.gridDim = dim3(min(static_cast<unsigned>(sm_count * WP_K2_BLOCKS), P.n_tiles * 4u));
-#endif
-    cfg.blockDim = dim3(MATCH_THREADS);
-    cfg.dynamicSmemBytes = 0;
-    cfg.numAttrs = window(P.vocab.edges, P.persist_edges_bytes, P.persist_edges_ratio);
-    e = cudaLaunchKernelEx(&cfg, wp_match_kernel, P);
-    if (e != cudaSuccess) return e;
 
-#ifdef WP_NO_GRID_TRIM
-    cfg.gridDim = dim3(sm_count * 8);
-#else
-    cfg.gridDim = dim3(min(static_cast<unsigned>(sm_count * 8), P.n_tiles * 2u + 2u));  // (one CTA per long segment, by ticket)
-#endif
-    cfg.blockDim = dim3(LONG_THREADS);
-    e = cudaLaunchKernelEx(&cfg, wp_long_kernel, P);
-    if (e != cudaSuccess) return e;
-    if (launches) *launches += 2;
-  }
+  // = resident capacity (see the launch bound): one wave, large shares; a small range (a 4 KiB call is ONE tile)
+  // gets a grid to match — a tile has at most MAX_TILE_SLOW unsettled segments, 8 warps x 32 lanes take 256 at a time
+  cfg.gridDim = dim3(min(static_cast<unsigned>(sm_count * WP_K2_BLOCKS), P.n_tiles * 4u));
+  cfg.blockDim = dim3(MATCH_THREADS);
+  cfg.dynamicSmemBytes = 0;
+  cfg.numAttrs = window(P.vocab.edges, P.persist_edges_bytes, P.persist_edges_ratio);
+  e = cudaLaunchKernelEx(&cfg, wp_match_kernel, P);
+  if (e != cudaSuccess) return e;
+
+  cfg.gridDim = dim3(min(static_cast<unsigned>(sm_count * 8), P.n_tiles * 2u + 2u));  // (one CTA per long segment, by ticket)
+  cfg.blockDim = dim3(LONG_THREADS);
+  e = cudaLaunchKernelEx(&cfg, wp_long_kernel, P);
+  if (e != cudaSuccess) return e;
+  if (launches) *launches += 2;
   if (timing) cudaEventRecord(timing[2], stream);
-  if (phases & PHASE_SCATTER) {
-#ifdef WP_NO_GRID_TRIM
-    cfg.gridDim = dim3(sm_count * WP_K3_BLOCKS);
-#else
-    cfg.gridDim = dim3(min(static_cast<unsigned>(sm_count * WP_K3_BLOCKS), P.n_tiles * 2u));  // a tile has at most two blocks of segments
-#endif
-    cfg.blockDim = dim3(SCATTER_THREADS);
-    cfg.dynamicSmemBytes = 0;
-    cfg.numAttrs = window(P.words, P.persist_words_bytes, P.persist_words_ratio);
-    e = cudaLaunchKernelEx(&cfg, wp_scatter_kernel, P);
-    if (e != cudaSuccess) return e;
-    if (launches) *launches += 1;
-  }
+
+  cfg.gridDim = dim3(min(static_cast<unsigned>(sm_count * WP_K3_BLOCKS), P.n_tiles * 2u));  // a tile has at most two blocks of segments
+  cfg.blockDim = dim3(SCATTER_THREADS);
+  cfg.dynamicSmemBytes = 0;
+  cfg.numAttrs = window(P.words, P.persist_words_bytes, P.persist_words_ratio);
+  e = cudaLaunchKernelEx(&cfg, wp_scatter_kernel, P);
+  if (e != cudaSuccess) return e;
+  if (launches) *launches += 1;
   if (timing) cudaEventRecord(timing[3], stream);
   return cudaSuccess;
 }

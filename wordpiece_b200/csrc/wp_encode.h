@@ -124,8 +124,6 @@ struct EncodeParams {
   uint32_t range_index;             // 0, 1, 2, ... within the call
   uint32_t use_ticket;              // K1 takes its tiles from RangeCounters::split_ticket instead of blockIdx.x
   uint32_t dense_tiles;             // K1 with full-capacity segment lists (seven tiles per SM instead of eight)
-  uint32_t accept_epoch;            // K1 uses word slots of an epoch <= this (wp_table.h); WORD_EPOCH_MAX = all
-  uint32_t record_epoch;            // epoch K2 tags its recordings with (range index + 1)
   // batch of texts in one buffer (wp_encode_batch), else bounds = nullptr: bounds[i] = byte offset at which
   // text i starts (ascending, each preceded by a space); tile_bound[t] = index of the first text that starts in
   // absolute tile t or later (n_tiles_total + 1 entries); K1 writes bound_seg[i] = the number, within the
@@ -156,13 +154,10 @@ uint32_t scatter_block_segments();
 // The compiled limits of the kernels, in the order of wp_debug_kernel_geometry (wordpiece_b200.h); returns their
 // number and writes at most `cap` of them.
 size_t kernel_geometry(uint32_t *out, size_t cap);
-// Enqueue the kernels of one range: PHASE_SPLIT = K1, PHASE_MATCH = K2 + K2L, PHASE_SCATTER = K3 (the host
-// may put the phases of a range on different streams to overlap consecutive ranges).  *launches is
-// incremented per kernel launched.  `timing` (optional, all phases only): 4 events recorded around the
-// launches (before K1, K1|K2, K2+K2L|K3, after K3).
-constexpr unsigned PHASE_SPLIT = 1u, PHASE_MATCH = 2u, PHASE_SCATTER = 4u, PHASE_ALL = 7u;
+// Enqueue the kernels of one range (K1, K2 + K2L, K3).  *launches is incremented per kernel launched.
+// `timing` (optional): 4 events recorded around the launches (before K1, K1|K2, K2+K2L|K3, after K3).
 cudaError_t launch_encode_range(const EncodeParams &P, int sm_count, cudaStream_t stream, uint64_t *launches,
-                                cudaEvent_t *timing = nullptr, unsigned phases = PHASE_ALL);
+                                cudaEvent_t *timing = nullptr);
 
 // ids -> "id id id " (decimal, one space after every id).  launch_format_total adds the text length to *total
 // (zeroed by the caller); launch_format writes it to `out` (block_state: one zeroed word per

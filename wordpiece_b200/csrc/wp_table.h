@@ -75,17 +75,10 @@ static_assert(sizeof(WordSlot) == 64, "a word slot is two 32-byte sectors; K1 re
 constexpr uint32_t WORD_CLAIMED = 1u;
 constexpr uint32_t WORD_READY = 0x80000000u;
 constexpr uint32_t WORD_DYNAMIC = 0x40000000u;   // recorded by K2 during this call (statistics only)
-// Epoch of a slot, bits 12..27: 0 for the static words, range index + 1 for a word K2 recorded.  When the
-// kernels of consecutive ranges overlap (K1 of range r+1 runs next to K2 of range r, which is filling the
-// table), K1 only accepts slots of an epoch whose K2 had finished before it started: a slot that may still
-// be in the middle of being written is never read for its ids.
-constexpr uint32_t WORD_EPOCH_SHIFT = 12;
-constexpr uint32_t WORD_EPOCH_MAX = 0xFFFFu;     // a K2 whose epoch would reach this stops recording
 WP_HD uint32_t word_meta_len(uint32_t meta) { return meta & 0x1Fu; }
 WP_HD uint32_t word_meta_count(uint32_t meta) { return (meta >> 8) & 0xFu; }
-WP_HD uint32_t word_meta_epoch(uint32_t meta) { return (meta >> WORD_EPOCH_SHIFT) & WORD_EPOCH_MAX; }
-WP_HD uint32_t word_meta(uint32_t len, uint32_t count, bool dynamic, uint32_t epoch = 0) {
-  return WORD_READY | (dynamic ? WORD_DYNAMIC : 0u) | (epoch << WORD_EPOCH_SHIFT) | (count << 8) | len;
+WP_HD uint32_t word_meta(uint32_t len, uint32_t count, bool dynamic) {
+  return WORD_READY | (dynamic ? WORD_DYNAMIC : 0u) | (count << 8) | len;
 }
 // Multiply-add over the four key words and the length (five IMADs), one fold, index from the high bits.
 WP_HD uint32_t word_hash(uint32_t k0, uint32_t k1, uint32_t k2, uint32_t k3, uint32_t len, uint32_t shift) {
