@@ -168,12 +168,14 @@ wp_status wp_encode_sharded_gather(wp_vocab *const *handles, size_t n_handles, c
 /* Many texts in ONE call (SURVEY 8(f): the batch entry the reference lacks — it rebuilds its maps per call,
  * fast.cpp:154-157, :21-35).  Text i (texts[i], lens[i] bytes; may be empty) is encoded exactly as
  * fast::encode(texts[i], vocab) would encode it; its ids are ids[offsets[i] .. offsets[i + 1]), offsets has
- * n_texts + 1 entries and *n_ids = offsets[n_texts].  One packed host->device copy, one pass of the kernels
- * over the whole batch, one copy back.  WP_ERR_CAPACITY (with *n_ids and offsets set) if capacity is short. */
+ * n_texts + 1 entries and *n_ids = offsets[n_texts].  The texts are packed into one buffer and encoded by one
+ * pass of the kernels; a large batch is cut into parts of whole texts that are packed, copied in, encoded and
+ * copied back in a pipeline.  WP_ERR_CAPACITY (with *n_ids and offsets set) if capacity is short. */
 wp_status wp_encode_batch(wp_vocab *v, const char *const *texts, const size_t *lens, size_t n_texts, int32_t *ids,
                           size_t capacity, size_t *offsets, size_t *n_ids);
 
-/* Counters of the last completed wp_encode / wp_encode_into / wp_encode_device call. */
+/* Counters of the last completed encode call on the handle (every encode entry point sets them; for a pipelined
+ * call they are summed over its parts). */
 wp_status wp_last_stats(wp_vocab *v, wp_stats *out);
 
 /* Per-kernel device time (diagnostics for bench.py's roofline): when enabled, every following encode call

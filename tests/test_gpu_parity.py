@@ -669,9 +669,12 @@ def test_two_handles_in_two_host_threads(gpu_device):
     calls, host-buffer calls large enough for the chunk pipeline (shared copy pool), and batches."""
     import threading
 
+    import torch
+
     from wordpiece_b200 import Vocab
 
     os.environ["WORDPIECE_B200_PIPE_CHUNK"] = "150000"
+    os.environ["WORDPIECE_B200_BATCH_PART"] = "65536"
     try:
         jobs = []
         for seed in (4101, 4102):
@@ -686,8 +689,13 @@ def test_two_handles_in_two_host_threads(gpu_device):
             try:
                 text, vocab, exp, pieces, exp_pieces = jobs[i]
                 v = Vocab(vocab, device=gpu_device)
+                out = np.zeros(exp.size + 1, np.int32)
+                pinned = torch.zeros(exp.size + 1, dtype=torch.int32).pin_memory()
                 for rep in range(6):
                     assert np.array_equal(v.encode(text), exp), (i, rep, "encode")
+                    for tag, buf in (("into", out), ("into pinned", pinned.numpy())):
+                        n = v.encode_into(text, buf)
+                        assert n == exp.size and np.array_equal(buf[:n], exp), (i, rep, tag)
                     ids, offs = v.encode_batch(pieces)
                     for k, e in enumerate(exp_pieces):
                         assert np.array_equal(ids[int(offs[k]):int(offs[k + 1])], e), (i, rep, "batch", k)
@@ -703,3 +711,4 @@ def test_two_handles_in_two_host_threads(gpu_device):
         assert not errors, errors[0]
     finally:
         os.environ.pop("WORDPIECE_B200_PIPE_CHUNK", None)
+        os.environ.pop("WORDPIECE_B200_BATCH_PART", None)

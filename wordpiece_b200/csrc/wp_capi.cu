@@ -16,8 +16,10 @@
 #include <functional>
 #include <mutex>
 #include <new>
+#include <optional>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "../../include/wordpiece_b200.h"
@@ -31,18 +33,21 @@ const char *const kHostOnly = "host-only vocabulary handle (device -1): encoding
 std::atomic<uint64_t> g_launches{0};
 
 // WORDPIECE_B200_TRACE=1: wall-clock milestones of a process on stderr (where does a short job's time go?)
-// WORDPIECE_B200_TRACE=2 additionally waits for the stream at every stage of a batch part, so that the
-// differences between milestones are the stages' own durations (a diagnosis mode: it serialises the pipeline)
-bool trace_stage_sync() {
-  static const bool on = std::getenv("WORDPIECE_B200_TRACE") != nullptr && std::atoi(std::getenv("WORDPIECE_B200_TRACE")) >= 2;
-  return on;
-}
 void trace(const char *what) {
   static const bool on = std::getenv("WORDPIECE_B200_TRACE") != nullptr;
   if (!on) return;
   static const auto t0 = std::chrono::steady_clock::now();
   std::fprintf(stderr, "[wordpiece_b200 %8.2f ms] %s\n",
                std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(), what);
+}
+// WORDPIECE_B200_TRACE=2 additionally waits for the stream at every stage of a pipeline part, so that the
+// differences between milestones are the stages' own durations (a diagnosis mode: it serialises the pipeline)
+cudaError_t trace_stage(cudaStream_t stream, const char *what) {
+  static const bool on = std::getenv("WORDPIECE_B200_TRACE") != nullptr && std::atoi(std::getenv("WORDPIECE_B200_TRACE")) >= 2;
+  if (!on) return cudaSuccess;
+  const cudaError_t e = cudaStreamSynchronize(stream);
+  trace(what);
+  return e;
 }
 
 wp_status fail(wp_status st, const std::string &msg) {
@@ -59,8 +64,8 @@ wp_status fail(wp_status st, const std::string &msg) {
 
 // WORDPIECE_B200_POISON=1 (tests): every device allocation of the library is filled with 0xCD bytes, so that a
 // kernel that reads scratch it has not written shows up in a fresh process as it would on recycled memory.
-// (value = bit mask of allocation classes: 1 scratch, 2 ids / text staging, 4 batch input, 8 batch output, 16 tables,
-// 32 call counters, 64 pipeline slots; "1" alone therefore poisons the scratch only, 127 everything)
+// (value = bit mask of allocation classes: 1 scratch, 2 ids / text staging, 4 pipeline slot input, 8 batch output,
+// 16 tables, 32 call counters, 64 pipeline slot ids; "1" alone therefore poisons the scratch only, 127 everything)
 template <class T>
 cudaError_t dev_alloc(T **p, size_t bytes, int cls = 127) {
   cudaError_t e = cudaMalloc(reinterpret_cast<void **>(p), bytes);
@@ -84,6 +89,58 @@ struct DeviceGuard {
   }
 };
 
+// An array that frees itself: device memory (dev_alloc, poison class `cls`) or pinned host memory.  grow(n) makes
+// room for at least n elements and reallocates only when n exceeds the capacity: exactly n the first time, an
+// eighth and 256 bytes more when it has to grow again, so that a handle's memory follows its largest call and is
+// never reallocated per call.  An empty array makes no CUDA call (host-only handles run on machines without one).
+template <class T, bool kPinned>
+class Buffer {
+ public:
+  T *p = nullptr;
+  size_t cap = 0;  // elements
+  explicit Buffer(int cls = 127) : cls_(cls) {}
+  Buffer(Buffer &&o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)), cls_(o.cls_) {}
+  Buffer &operator=(Buffer &&) = delete;
+  ~Buffer() { release(); }
+  cudaError_t grow(size_t n) {
+    if (n <= cap) return cudaSuccess;
+    const size_t want = cap ? n + n / 8 + 256 / sizeof(T) : n;
+    release();
+    const cudaError_t e = kPinned ? cudaMallocHost(reinterpret_cast<void **>(&p), want * sizeof(T))
+                                  : dev_alloc(&p, want * sizeof(T), cls_);
+    if (e == cudaSuccess) cap = want;
+    return e;
+  }
+
+ private:
+  void release() {
+    if (p) kPinned ? cudaFreeHost(p) : cudaFree(p);
+    p = nullptr;
+    cap = 0;
+  }
+  int cls_;
+};
+template <class T>
+using DeviceBuffer = Buffer<T, false>;
+template <class T>
+using PinnedBuffer = Buffer<T, true>;
+
+// A CUDA event or stream that destroys itself
+template <class H, cudaError_t (*Destroy)(H)>
+struct Owned {
+  H h = nullptr;
+  Owned() = default;
+  Owned(Owned &&o) noexcept : h(std::exchange(o.h, nullptr)) {}
+  Owned &operator=(Owned &&) = delete;
+  ~Owned() {
+    if (h) Destroy(h);
+  }
+  operator H() const { return h; }
+};
+using Event = Owned<cudaEvent_t, cudaEventDestroy>;
+using Stream = Owned<cudaStream_t, cudaStreamDestroy>;
+
+
 constexpr size_t kRangeBytesMax = size_t(64) << 20;  // text bytes encoded per K1/K2/K3 round (bounds the scratch)
 constexpr uint32_t kWorkWordSlotsLog2 = 20;          // working word table of a large call: 2^20 slots of 64 bytes = 64 MiB
 constexpr size_t kMemoMinBytes = size_t(4) << 20;    // texts below this use the static word table as it is: recording
@@ -95,61 +152,44 @@ static_assert(kRangeBytesMax / 2 + 1024 <= (size_t(1) << wp::SEG_SLOW_INDEX_BITS
 struct wp_vocab {
   wp::HostVocab host;
   int device = 0;
-  cudaStream_t stream = nullptr;
+  Stream stream;
   // device tables
-  wp::Edge *d_edges = nullptr;
-  wp::WordSlot *d_words_static = nullptr;  // image built from the vocabulary, never written by a kernel
-  wp::WordSlot *d_words_work = nullptr;    // per-call working table K2 records into (allocated on the first large call)
+  DeviceBuffer<wp::Edge> d_edges{16};
+  DeviceBuffer<wp::WordSlot> d_words_static{16};  // image built from the vocabulary, never written by a kernel
+  DeviceBuffer<wp::WordSlot> d_words_work{16};    // per-call working table K2 records into (allocated on the first large call)
   uint32_t work_words_log2 = 0;
   size_t device_bytes = 0;
-  // scratch, grown on demand (layout: see Workspace below)
-  uint8_t *d_work = nullptr;
-  size_t work_bytes = 0;
-  wp::CallCounters *d_call = nullptr;
+  DeviceBuffer<uint8_t> d_work{1};  // scratch (layout: see Workspace below)
+  DeviceBuffer<wp::CallCounters> d_call{32};
   int sm_count = 0;
   size_t persist_words_bytes = 0, persist_edges_bytes = 0, persist_work_bytes = 0;  // L2 access-policy windows
   float persist_words_ratio = 0.f, persist_edges_ratio = 0.f, persist_work_ratio = 0.f;
   size_t set_aside = 0, max_window = 0;
-  uint8_t *d_text = nullptr;  // staging for the host-buffer entry points
-  size_t text_cap = 0;
-  int32_t *d_ids = nullptr;
-  size_t ids_cap = 0;
-  char *d_fmt = nullptr;  // wp_encode_text: the ids as decimal text
-  size_t fmt_cap = 0;
-  wp::CallCounters *h_call = nullptr;  // pinned
-  // wp_encode_batch: packed input (tile index, text starts, texts) in pinned host memory and its device
-  // mirror; per-text outputs (first segment, first id) on the device; the id offsets in pinned host memory
-  // (three sets: a large batch is cut into parts that are packed, copied and encoded in a pipeline)
-  struct BatchSlot {
-    uint8_t *h_in = nullptr, *d_in = nullptr, *d_out = nullptr;
-    size_t in_cap = 0, out_cap = 0;
-    unsigned long long *h_offsets = nullptr;
-    size_t offsets_cap = 0;
-    int32_t *d_ids = nullptr;
-    size_t ids_cap = 0;
-    wp::CallCounters *h_call = nullptr;  // pinned
-    cudaEvent_t h2d_done = nullptr, cmp_done = nullptr, d2h_done = nullptr;
-  } bslot[3];
-  // host-buffer pipeline (wp_encode_into on large texts): three chunks in flight
-  struct PipeSlot {
-    uint8_t *d_text = nullptr;
-    int32_t *d_ids = nullptr;
-    wp::CallCounters *h_call = nullptr;  // pinned
-    // staging for callers whose buffers are pageable (a std::string, a std::vector): pinned, allocated on demand
-    uint8_t *h_text = nullptr;
-    int32_t *h_ids = nullptr;
-    cudaEvent_t h2d_done = nullptr, cmp_done = nullptr, d2h_done = nullptr;
+  DeviceBuffer<uint8_t> d_text{2};  // staging of the single-shot host-buffer path
+  DeviceBuffer<int32_t> d_ids{2};
+  DeviceBuffer<char> d_fmt;  // wp_encode_text: the ids as decimal text
+  PinnedBuffer<wp::CallCounters> h_call;
+  // The host pipeline (run_pipeline): input block in pinned host memory and on the device, ids, a batch part's
+  // per-text outputs (first segment, first id) and id offsets, counters, pinned id staging for pageable callers
+  struct Slot {
+    PinnedBuffer<uint8_t> h_in;
+    DeviceBuffer<uint8_t> d_in{4};
+    DeviceBuffer<int32_t> d_ids{64};
+    DeviceBuffer<uint8_t> d_out{8};
+    PinnedBuffer<unsigned long long> h_offsets;
+    PinnedBuffer<wp::CallCounters> h_call;
+    PinnedBuffer<int32_t> h_ids;
+    Event h2d_done, cmp_done, d2h_done;
   } slot[3];
-  cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
-  bool pipe_ready = false;
+  Stream s_h2d, s_d2h;
   // every call on a handle shares its scratch, counters and word table: the kernels of one call must have
   // finished before those of the next begin, on whatever streams the caller enqueues them
-  cudaEvent_t last_done = nullptr;
+  Event last_done;
   bool use_ticket = false;  // K1 hands its tiles out by ticket (set for good once a look-back has stalled, see wp_encode.cu)
   bool dense_tiles = false; // K1 with full-capacity segment lists (set for good once a tile overflowed the regular ones)
   // optional per-kernel timing (wp_set_kernel_timing): events around K1/K2/K3 of every range
   bool timing = false;
-  std::vector<cudaEvent_t> timing_events;  // 4 per range of the last call
+  std::vector<Event> timing_events;  // 4 per range of the last call
   size_t timing_used = 0;
   wp_stats stats{};
 };
@@ -164,7 +204,7 @@ uint32_t log2_of(size_t pow2) {
 
 wp::DeviceVocab device_view(const wp_vocab *v) {
   wp::DeviceVocab d{};
-  d.edges = v->d_edges;
+  d.edges = v->d_edges.p;
   d.edge_mask = static_cast<uint32_t>(v->host.edges.size() - 1);
   d.edge_shift = 32 - log2_of(v->host.edges.size());
   d.unk_id = v->host.unk_id;
@@ -176,14 +216,14 @@ wp_status upload(wp_vocab *v) {
   const wp::HostVocab &h = v->host;
   const size_t b_edges = h.edges.size() * sizeof(wp::Edge);
   const size_t b_words = h.words.size() * sizeof(wp::WordSlot);
-  WP_CUDA(dev_alloc(&v->d_edges, b_edges, 16));
-  WP_CUDA(dev_alloc(&v->d_words_static, b_words, 16));
-  WP_CUDA(cudaMemcpy(v->d_edges, h.edges.data(), b_edges, cudaMemcpyHostToDevice));
-  WP_CUDA(cudaMemcpy(v->d_words_static, h.words.data(), b_words, cudaMemcpyHostToDevice));
+  WP_CUDA(v->d_edges.grow(h.edges.size()));
+  WP_CUDA(v->d_words_static.grow(h.words.size()));
+  WP_CUDA(cudaMemcpy(v->d_edges.p, h.edges.data(), b_edges, cudaMemcpyHostToDevice));
+  WP_CUDA(cudaMemcpy(v->d_words_static.p, h.words.data(), b_words, cudaMemcpyHostToDevice));
   v->device_bytes = b_edges + b_words;
-  WP_CUDA(cudaStreamCreateWithFlags(&v->stream, cudaStreamNonBlocking));
-  WP_CUDA(cudaMallocHost(&v->h_call, sizeof(wp::CallCounters)));
-  WP_CUDA(dev_alloc(&v->d_call, sizeof(wp::CallCounters), 32));
+  for (Stream *s : {&v->stream, &v->s_h2d, &v->s_d2h}) WP_CUDA(cudaStreamCreateWithFlags(&s->h, cudaStreamNonBlocking));
+  WP_CUDA(v->h_call.grow(1));
+  WP_CUDA(v->d_call.grow(1));
   WP_CUDA(cudaDeviceGetAttribute(&v->sm_count, cudaDevAttrMultiProcessorCount, v->device));
   {
     // keep the table a kernel reads at random resident in L2 (best effort: an unsupported attribute only
@@ -259,17 +299,6 @@ Workspace plan_workspace(size_t range_bytes, size_t spill_ids) {
   return w;
 }
 
-wp_status ensure_work(wp_vocab *v, size_t need) {
-  if (need > v->work_bytes) {
-    if (v->d_work) cudaFree(v->d_work);
-    v->d_work = nullptr;
-    v->work_bytes = 0;
-    WP_CUDA(dev_alloc(&v->d_work, need, 1));
-    v->work_bytes = need;
-  }
-  return WP_OK;
-}
-
 // A batch of texts packed into one buffer (wp_encode_batch): see EncodeParams::bounds.
 struct BatchArgs {
   const unsigned long long *h_bounds = nullptr;  // host copy of the text starts (ascending), n_texts entries
@@ -302,15 +331,15 @@ wp_status enqueue_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_
   }
   const size_t range_bytes = n_bytes < range_max ? n_bytes : range_max;
   const Workspace w = plan_workspace(range_bytes, spill_ids ? spill_ids : range_bytes + tile);
-  if (!v->last_done) WP_CUDA(cudaEventCreateWithFlags(&v->last_done, cudaEventDisableTiming));
+  if (!v->last_done) WP_CUDA(cudaEventCreateWithFlags(&v->last_done.h, cudaEventDisableTiming));
   WP_CUDA(cudaStreamWaitEvent(stream, v->last_done, 0));  // (a never-recorded event does not block)
-  WP_CUDA(cudaMemsetAsync(v->d_call, 0, sizeof(wp::CallCounters), stream));
+  WP_CUDA(cudaMemsetAsync(v->d_call.p, 0, sizeof(wp::CallCounters), stream));
   v->timing_used = 0;
   bool use_memo = (call_bytes ? call_bytes : n_bytes) >= kMemoMinBytes;  // judged on the whole user call
   if (const char *e = std::getenv("WORDPIECE_B200_MEMO")) use_memo = std::atoi(e) != 0;  // 0 = off, 1 = on (tests)
   uint64_t launches = 0;
   if (use_memo) {
-    if (!v->d_words_work) {
+    if (!v->d_words_work.p) {
       uint32_t lg = kWorkWordSlotsLog2;
       if (const char *e = std::getenv("WORDPIECE_B200_WORD_SLOTS_LOG2")) {  // test hook: a small, crowded table
         const int x = std::atoi(e);
@@ -318,7 +347,7 @@ wp_status enqueue_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_
       }
       const uint32_t static_lg = log2_of(v->host.words.size());
       if (lg < static_lg) lg = static_lg;  // the static words must fit with room to spare
-      WP_CUDA(dev_alloc(&v->d_words_work, (size_t(1) << lg) * sizeof(wp::WordSlot), 16));
+      WP_CUDA(v->d_words_work.grow(size_t(1) << lg));
       v->work_words_log2 = lg;
       if (v->persist_words_bytes) {
         const size_t b = (size_t(1) << lg) * sizeof(wp::WordSlot);
@@ -330,7 +359,7 @@ wp_status enqueue_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_
     // every user call starts from the static words only: what K2 records never outlives the call (the chunks
     // of one pipelined host-buffer call share it), so neither ids nor timing depend on earlier calls
     if (!warm)
-      WP_CUDA(wp::launch_seed_words(v->d_words_static, static_cast<uint32_t>(v->host.words.size()), v->d_words_work,
+      WP_CUDA(wp::launch_seed_words(v->d_words_static.p, static_cast<uint32_t>(v->host.words.size()), v->d_words_work.p,
                                     v->work_words_log2, stream, &launches));
   }
   wp::EncodeParams P{};
@@ -339,13 +368,13 @@ wp_status enqueue_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_
   P.n_bytes = n_bytes;
   P.ids = d_ids;
   P.capacity = capacity;
-  P.call = v->d_call;
+  P.call = v->d_call.p;
   P.seg_capacity = w.seg_cap;
   P.slow_capacity = w.slow_cap;
   P.long_capacity = w.long_cap;
   P.arena_capacity = w.arena_cap;
   P.n_scatter_blocks = w.n_scatter_blocks;
-  P.words = use_memo ? v->d_words_work : v->d_words_static;
+  P.words = use_memo ? v->d_words_work.p : v->d_words_static.p;
   const uint32_t words_log2 = use_memo ? v->work_words_log2 : log2_of(v->host.words.size());
   P.word_mask = (1u << words_log2) - 1u;
   P.word_shift = 32 - words_log2;
@@ -394,9 +423,8 @@ wp_status enqueue_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_
   }
   const uint32_t n_ranges = static_cast<uint32_t>(ranges.size());
 
-  const wp_status st = ensure_work(v, w.total);
-  if (st != WP_OK) return st;
-  uint8_t *const scratch = v->d_work;
+  WP_CUDA(v->d_work.grow(w.total));
+  uint8_t *const scratch = v->d_work.p;
   P.counters = reinterpret_cast<wp::RangeCounters *>(scratch);
   P.tile_state = reinterpret_cast<unsigned long long *>(scratch + w.off_tile_state);
   P.block_state = reinterpret_cast<unsigned long long *>(scratch + w.off_block_state);
@@ -413,17 +441,17 @@ wp_status enqueue_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_
     if (poison_scratch)  // (tests) everything a range must write before it reads, filled with 0xCD on the launching stream
       WP_CUDA(cudaMemsetAsync(scratch + w.off_seg, 0xCD, w.total - w.off_seg, stream));
     WP_CUDA(cudaMemsetAsync(scratch, 0, w.zero_bytes, stream));
-    cudaEvent_t *tev = nullptr;
+    cudaEvent_t tev[4];
     if (v->timing) {
       while (v->timing_events.size() < v->timing_used + 4) {
-        cudaEvent_t e;
-        WP_CUDA(cudaEventCreate(&e));
-        v->timing_events.push_back(e);
+        Event e;
+        WP_CUDA(cudaEventCreate(&e.h));
+        v->timing_events.push_back(std::move(e));
       }
-      tev = v->timing_events.data() + v->timing_used;
+      for (int k = 0; k < 4; k++) tev[k] = v->timing_events[v->timing_used + k];
       v->timing_used += 4;
     }
-    WP_CUDA(wp::launch_encode_range(P, v->sm_count, stream, &launches, tev));
+    WP_CUDA(wp::launch_encode_range(P, v->sm_count, stream, &launches, v->timing ? tev : nullptr));
     WP_CUDA(text_offsets());
   }
   WP_CUDA(cudaEventRecord(v->last_done, stream));
@@ -456,24 +484,53 @@ bool absorb_call(wp_vocab *v, const wp::CallCounters &c, const EnqueueInfo &info
   return true;
 }
 
-// enqueue + wait, repeated while the ids are void (absorb_call)
-wp_status run_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_t *d_ids, size_t capacity,
-                     cudaStream_t stream) {
-  size_t spill = 0;
-  for (int attempt = 0; attempt < kMaxAttempts; attempt++) {
+// One call of n_bytes text bytes, repeated while its ids are void (absorb_call), the first time with id spill
+// `spill`.  attempt(spill, &info) enqueues the call on `stream` and a copy of its counters to `counters` (pinned).
+template <class Attempt>
+wp_status repeat_call(wp_vocab *v, cudaStream_t stream, size_t n_bytes, size_t spill,
+                      const wp::CallCounters &counters, Attempt &&attempt) {
+  for (int i = 0; i < kMaxAttempts; i++) {
     EnqueueInfo info;
-    const wp_status st = enqueue_encode(v, d_text, n_bytes, d_ids, capacity, stream, spill, &info);
+    const wp_status st = attempt(spill, &info);
     if (st != WP_OK) return st;
-    WP_CUDA(cudaMemcpyAsync(v->h_call, v->d_call, sizeof(wp::CallCounters), cudaMemcpyDeviceToHost, stream));
     WP_CUDA(cudaStreamSynchronize(stream));
     wp_stats acc{};
-    if (absorb_call(v, *v->h_call, info, n_bytes, &acc, &spill)) continue;
+    if (absorb_call(v, counters, info, n_bytes, &acc, &spill)) continue;
     v->stats = acc;
     v->stats.n_bytes = n_bytes;
-    v->stats.n_ids = v->h_call->ids_total[info.n_ranges & 1u];
+    v->stats.n_ids = counters.ids_total[info.n_ranges & 1u];
     return WP_OK;
   }
   return fail(WP_ERR_CUDA, "internal scratch overflow");
+}
+
+// A device-resident text, encoded and waited for
+wp_status run_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_t *d_ids, size_t capacity,
+                     cudaStream_t stream, size_t spill = 0) {
+  return repeat_call(v, stream, n_bytes, spill, *v->h_call.p, [&](size_t sp, EnqueueInfo *info) -> wp_status {
+    const wp_status st = enqueue_encode(v, d_text, n_bytes, d_ids, capacity, stream, sp, info);
+    if (st != WP_OK) return st;
+    WP_CUDA(cudaMemcpyAsync(v->h_call.p, v->d_call.p, sizeof(wp::CallCounters), cudaMemcpyDeviceToHost, stream));
+    return WP_OK;
+  });
+}
+
+// Host text -> ids in the handle's device buffer v->d_ids (count in v->stats.n_ids), through the staging buffer
+// v->d_text.  The id buffer holds at least ids_want ids; `retry_short`: if that was too few, once more with the
+// exact count (the launches of both attempts are counted).
+wp_status encode_staged(wp_vocab *v, const char *text, size_t n_bytes, size_t ids_want, bool retry_short,
+                        size_t spill = 0) {
+  WP_CUDA(v->d_text.grow(n_bytes));
+  WP_CUDA(cudaMemcpyAsync(v->d_text.p, text, n_bytes, cudaMemcpyHostToDevice, v->stream));
+  for (int attempt = 0;; attempt++) {
+    WP_CUDA(v->d_ids.grow(ids_want));
+    const uint64_t before = v->stats.kernel_launches;
+    const wp_status st = run_encode(v, v->d_text.p, n_bytes, v->d_ids.p, v->d_ids.cap, v->stream, spill);
+    if (st != WP_OK) return st;
+    if (attempt) v->stats.kernel_launches += before;
+    if (!retry_short || attempt || v->stats.n_ids <= v->d_ids.cap) return WP_OK;
+    ids_want = static_cast<size_t>(v->stats.n_ids);
+  }
 }
 
 // ---- copies into pinned staging memory with STREAMING (non-temporal) stores
@@ -685,24 +742,6 @@ bool is_pageable(const void *p) {
 }
 
 constexpr size_t kPipeChunk = size_t(16) << 20;  // host-buffer pipeline: text bytes per chunk (16 MiB measured best: 8/16/32 MiB -> 41.6/43.6/40.5 GB/s e2e on one box)
-constexpr int kPipeSlots = 3;
-
-wp_status ensure_pipeline(wp_vocab *v) {
-  if (v->pipe_ready) return WP_OK;
-  WP_CUDA(cudaStreamCreateWithFlags(&v->s_h2d, cudaStreamNonBlocking));
-  WP_CUDA(cudaStreamCreateWithFlags(&v->s_d2h, cudaStreamNonBlocking));
-  for (auto &sl : v->slot) {
-    WP_CUDA(dev_alloc(&sl.d_text, kPipeChunk + 256, 64));
-    WP_CUDA(dev_alloc(&sl.d_ids, kPipeChunk * sizeof(int32_t), 64));  // ids <= bytes
-    WP_CUDA(cudaMallocHost(&sl.h_call, sizeof(wp::CallCounters)));
-    WP_CUDA(cudaEventCreateWithFlags(&sl.h2d_done, cudaEventDisableTiming));
-    WP_CUDA(cudaEventCreateWithFlags(&sl.cmp_done, cudaEventDisableTiming));
-    WP_CUDA(cudaEventCreateWithFlags(&sl.d2h_done, cudaEventDisableTiming));
-  }
-  v->pipe_ready = true;
-  return WP_OK;
-}
-
 inline bool is_ascii_space(unsigned char c) { return (c >= 0x09 && c <= 0x0D) || c == 0x20; }
 inline bool is_ascii_punct(unsigned char c) {
   return (c >= 0x21 && c <= 0x2F) || (c >= 0x3A && c <= 0x40) || (c >= 0x5B && c <= 0x60) || (c >= 0x7B && c <= 0x7E);
@@ -780,123 +819,253 @@ bool plan_chunks(const char *text, size_t n, size_t chunk, std::vector<size_t> *
   return true;
 }
 
-constexpr size_t kStageIds = kPipeChunk / 2;  // ids per pinned staging slot (32 MiB; a chunk of ordinary text has a quarter of that)
+/* ------------------------------------------------------------------ the host pipeline (run_pipeline)
+ * A batch is packed into one buffer, each text followed by one space: a space ends every word and resets the
+ * matcher's state (fast.cpp:89-91), a byte sequence cut short at the end of a text stays invalid in front of
+ * it, so the ids of the packed buffer are the ids of the texts one after the other.  K1 numbers the first
+ * segment of every text, K5 turns the numbers into id offsets (wp_encode.h). */
 
-// Host text -> host ids through a three-stage pipeline: while chunk i is encoded, chunk i+1 is copied in
-// and the ids of chunk i-1 are copied out (the PCIe copies, not the kernels, bound this entry point).
-// Pageable caller memory (the reference's own signature hands over a std::string and expects a std::vector)
-// is staged through pinned slots by the CopyPool: chunk i+1 -> pinned before its H2D, and the ids of chunk
-// i-2 pinned -> caller after their D2H.  *fell_back is set if the text could not be chunked or a chunk
-// outgrew the scratch; nothing is lost then, the caller runs the single-shot path.
-wp_status encode_pipelined(wp_vocab *v, const char *text, size_t n_bytes, int32_t *ids, size_t capacity,
-                           size_t *n_ids, bool *fell_back) {
-  *fell_back = false;
-  std::vector<size_t> cuts;
-  if (!plan_chunks(text, n_bytes, pipe_chunk_bytes(), &cuts)) {
-    *fell_back = true;
-    return WP_OK;
+constexpr size_t kBatchPart = size_t(8) << 20;  // packed bytes per part of a large batch
+
+size_t batch_part_bytes() {
+  if (const char *e = std::getenv("WORDPIECE_B200_BATCH_PART")) {  // test hook: pipeline small batches
+    const long long x = std::atoll(e);
+    if (x >= 256 && static_cast<size_t>(x) <= kBatchPart) return static_cast<size_t>(x);
   }
-  wp_status st = ensure_pipeline(v);
+  return kBatchPart;
+}
+
+// One part of a pipelined call: a chunk of one text (wp_encode_into: no texts; only `packed` and `in_bytes`, the
+// chunk's length, are set), or whole texts of a batch, whose input block is laid out as
+// tile index | text starts | packed texts (16-byte aligned for K1's vector loads)
+struct PartPlan {
+  size_t first = 0, last = 0;  // texts [first, last)
+  size_t packed = 0;           // bytes incl. one separator per text
+  size_t n_tiles = 0, off_bounds = 0, off_text = 0, in_bytes = 0, off_offsets = 0, out_bytes = 0;
+};
+
+PartPlan plan_part(const size_t *lens, size_t first, size_t last) {
+  PartPlan p;
+  p.first = first;
+  p.last = last;
+  const size_t n = last - first;
+  p.packed = n;
+  for (size_t i = first; i < last; i++) p.packed += lens[i];
+  const size_t tile = wp::encode_tile_bytes();
+  p.n_tiles = (p.packed + tile - 1) / tile;
+  p.off_bounds = align_up((p.n_tiles + 1) * sizeof(uint32_t), 256);
+  p.off_text = align_up(p.off_bounds + n * sizeof(unsigned long long), 256);
+  p.in_bytes = p.off_text + p.packed;
+  p.off_offsets = align_up(n * sizeof(uint32_t), 256);
+  p.out_bytes = p.off_offsets + (n + 1) * sizeof(unsigned long long);
+  return p;
+}
+
+// texts -> the part's input block (text starts, tile index, the texts with their separators)
+void pack_part(uint8_t *block, const PartPlan &p, const char *const *texts, const size_t *lens,
+               bool streamed = stream_stores()) {
+  const size_t n = p.last - p.first;
+  uint32_t *tile_bound = reinterpret_cast<uint32_t *>(block);
+  unsigned long long *bounds = reinterpret_cast<unsigned long long *>(block + p.off_bounds);
+  char *text = reinterpret_cast<char *>(block + p.off_text);
+  unsigned long long at = 0;
+  for (size_t i = 0; i < n; i++) {
+    bounds[i] = at;
+    at += lens[p.first + i] + 1;
+  }
+  auto pack = [&](size_t part, size_t parts) {  // equal byte shares, whole texts
+    const unsigned long long lo = static_cast<unsigned long long>(p.packed) * part / parts;
+    const unsigned long long hi = static_cast<unsigned long long>(p.packed) * (part + 1) / parts;
+    size_t i = static_cast<size_t>(std::lower_bound(bounds, bounds + n, lo) - bounds);
+    const size_t end = part + 1 == parts ? n : static_cast<size_t>(std::lower_bound(bounds, bounds + n, hi) - bounds);
+    if (streamed) {  // (the texts of a share are contiguous in the packed buffer)
+      if (i >= end) return;
+      StreamWriter w(text + bounds[i]);
+      for (; i < end; i++) {
+        w.put(texts[p.first + i], lens[p.first + i]);
+        w.put(' ');
+      }
+      w.finish();
+      return;
+    }
+    for (; i < end; i++) {
+      char *dst = text + bounds[i];
+      const size_t len = lens[p.first + i];
+      if (len) std::memcpy(dst, texts[p.first + i], len);
+      dst[len] = ' ';
+    }
+  };
+  if (p.packed >= (size_t(1) << 20)) {
+    CopyPool::get().run(pack);
+  } else {
+    pack(0, 1);
+  }
+  const size_t tile = wp::encode_tile_bytes();
+  size_t i = 0;
+  for (size_t t = 0; t <= p.n_tiles; t++) {  // tile_bound[t] = first text that starts at or after byte t * tile
+    const unsigned long long lo = static_cast<unsigned long long>(t) * tile;
+    while (i < n && bounds[i] < lo) i++;
+    tile_bound[t] = static_cast<uint32_t>(i);
+  }
+}
+
+constexpr int kSlots = 3;
+
+// Room in slot sl for part p (`fill_pinned`: its input is staged in the slot's pinned memory; `stage_ids`: pinned
+// id staging).  Before a buffer of a slot in use grows, the host waits until the slot's previous part has left it.
+wp_status fit_slot(wp_vocab::Slot &sl, const PartPlan &p, bool fill_pinned, size_t stage_ids, bool in_use) {
+  bool waited = !in_use;
+  auto grow = [&](auto &buf, size_t want) -> cudaError_t {
+    if (want > buf.cap && !waited) {
+      waited = true;
+      const cudaError_t e = cudaEventSynchronize(sl.d2h_done);
+      if (e != cudaSuccess) return e;
+    }
+    return buf.grow(want);
+  };
+  WP_CUDA(grow(sl.h_in, fill_pinned ? p.in_bytes : 0));
+  WP_CUDA(grow(sl.d_in, p.in_bytes));
+  WP_CUDA(grow(sl.d_ids, p.packed));  // one id per byte is the worst case
+  WP_CUDA(grow(sl.d_out, p.out_bytes));
+  WP_CUDA(grow(sl.h_offsets, p.last > p.first ? p.last - p.first + 1 : 0));  // (a batch part's texts + 1)
+  WP_CUDA(grow(sl.h_ids, stage_ids));
+  WP_CUDA(grow(sl.h_call, 1));
+  for (Event *e : {&sl.h2d_done, &sl.cmp_done, &sl.d2h_done})
+    if (!e->h) WP_CUDA(cudaEventCreateWithFlags(&e->h, cudaEventDisableTiming));
+  trace("part: buffers ready");
+  return WP_OK;
+}
+
+// Enqueue part p in slot sl: the H2D copy of its input block from host memory `src` on `copy_stream`, then on
+// v->stream the kernels, for a batch part its id offsets and their copy to sl.h_offsets, and the copy of the
+// counters to sl.h_call.
+wp_status enqueue_part(wp_vocab *v, wp_vocab::Slot &sl, const PartPlan &p, const void *src, cudaStream_t copy_stream,
+                       size_t spill, bool warm, size_t call_bytes, EnqueueInfo *info) {
+  const size_t n = p.last - p.first;  // texts (none: a chunk of one text)
+  WP_CUDA(cudaMemcpyAsync(sl.d_in.p, src, p.in_bytes, cudaMemcpyHostToDevice, copy_stream));
+  WP_CUDA(trace_stage(copy_stream, "part:   [stage] input block on the device"));
+  WP_CUDA(cudaEventRecord(sl.h2d_done, copy_stream));
+  WP_CUDA(cudaStreamWaitEvent(v->stream, sl.h2d_done, 0));
+  BatchArgs batch;
+  batch.h_bounds = reinterpret_cast<const unsigned long long *>(static_cast<const uint8_t *>(src) + p.off_bounds);
+  batch.n_texts = n;
+  batch.d_tile_bound = reinterpret_cast<const uint32_t *>(sl.d_in.p);
+  batch.d_bounds = reinterpret_cast<const unsigned long long *>(sl.d_in.p + p.off_bounds);
+  batch.d_bound_seg = reinterpret_cast<uint32_t *>(sl.d_out.p);
+  batch.d_offsets = reinterpret_cast<unsigned long long *>(sl.d_out.p + p.off_offsets);
+  const wp_status st = enqueue_encode(v, sl.d_in.p + p.off_text, p.packed, sl.d_ids.p, sl.d_ids.cap, v->stream, spill,
+                                      info, warm, call_bytes, n ? &batch : nullptr);
   if (st != WP_OK) return st;
-  const bool stage_in = is_pageable(text), stage_out = capacity > 0 && is_pageable(ids);
-  for (auto &sl : v->slot) {
-    if (stage_in && !sl.h_text) WP_CUDA(cudaMallocHost(&sl.h_text, kPipeChunk));
-    if (stage_out && !sl.h_ids) WP_CUDA(cudaMallocHost(&sl.h_ids, kStageIds * sizeof(int32_t)));
+  WP_CUDA(trace_stage(v->stream, "part:   [stage] kernels done"));
+  if (n) {
+    uint64_t launches = 0;
+    WP_CUDA(wp::launch_publish_count(v->d_call.p, info->n_ranges & 1u, batch.d_offsets + n, v->stream, &launches));
+    WP_CUDA(cudaEventRecord(v->last_done, v->stream));
+    g_launches.fetch_add(launches, std::memory_order_relaxed);
+    info->launches += launches;
+    WP_CUDA(cudaMemcpyAsync(sl.h_offsets.p, batch.d_offsets, (n + 1) * sizeof(unsigned long long),
+                            cudaMemcpyDeviceToHost, v->stream));
   }
-  CopyPool &pool = CopyPool::get();
-  const size_t n_chunks = cuts.size() - 1;
-  std::vector<EnqueueInfo> infos(n_chunks);
-  std::vector<size_t> counts(n_chunks, 0), offsets(n_chunks, 0);
-  size_t total = 0;
-  bool overflow = false;
-  wp_stats acc{};
+  WP_CUDA(cudaMemcpyAsync(sl.h_call.p, v->d_call.p, sizeof(wp::CallCounters), cudaMemcpyDeviceToHost, v->stream));
+  WP_CUDA(cudaEventRecord(sl.cmp_done, v->stream));
+  trace("part: enqueued");
+  return WP_OK;
+}
 
-  // chunk j's kernels are done: read its count, start the copy of its ids device -> host
-  auto start_d2h = [&](size_t j) -> wp_status {
-    wp_vocab::PipeSlot &sl = v->slot[j % kPipeSlots];
+// The parts of one call (wp_encode_into: text chunks, wp_encode_batch: whole texts) into ids[0, capacity) through
+// three slots: while part k is encoded, part k+1 is filled and copied in and the ids of part k-1 are copied out
+// (the PCIe copies, not the kernels, bound these calls).  fill(k, slot) returns the host address of part k's input
+// block (`fill_pinned`: it writes it to the slot's pinned input); done(k, slot, first_id) takes what a finished
+// part adds besides its ids.  `stage_out`: ids go to the pageable caller through pinned staging and the CopyPool.
+// A void part ends the call with *repeat set: the caller repeats the whole call, the first time with *spill.
+template <class Fill, class Done>
+wp_status run_pipeline(wp_vocab *v, const std::vector<PartPlan> &parts, size_t call_bytes, bool fill_pinned,
+                       bool stage_out, int32_t *ids, size_t capacity, Fill &&fill, Done &&done,
+                       size_t *n_ids, bool *repeat, size_t *spill) {
+  CopyPool &pool = CopyPool::get();
+  const size_t n_parts = parts.size();
+  // ids per pinned staging slot (32 MiB at the default chunk size; a chunk of ordinary text has a quarter of that)
+  const size_t stage_ids = stage_out ? pipe_chunk_bytes() / 2 : 0;
+  std::vector<EnqueueInfo> infos(n_parts);
+  std::vector<size_t> first_id(n_parts, 0), staged(n_parts, 0);
+  size_t total = 0;
+  wp_stats acc{};
+  *repeat = false;
+
+  // part j's kernels are done: absorb its counters, start the copy of its ids device -> host
+  auto finish = [&](size_t j) -> wp_status {
+    wp_vocab::Slot &sl = v->slot[j % kSlots];
     WP_CUDA(cudaEventSynchronize(sl.cmp_done));
-    const size_t cnt = static_cast<size_t>(sl.h_call->ids_total[infos[j].n_ranges & 1u]);
-    size_t spill = 0;  // (a void chunk is not repeated: the caller encodes the whole text in one call instead)
-    if (absorb_call(v, *sl.h_call, infos[j], cuts[j + 1] - cuts[j], &acc, &spill)) overflow = true;
-    counts[j] = cnt;
-    offsets[j] = total;
-    if (!overflow && cnt > 0 && total + cnt <= capacity) {
+    *repeat = absorb_call(v, *sl.h_call.p, infos[j], call_bytes, &acc, spill);
+    if (*repeat) return WP_OK;
+    const size_t cnt = static_cast<size_t>(sl.h_call.p->ids_total[infos[j].n_ranges & 1u]);
+    done(j, sl, total);
+    first_id[j] = total;
+    if (cnt > 0 && total + cnt <= capacity) {
       WP_CUDA(cudaStreamWaitEvent(v->s_d2h, sl.cmp_done, 0));
       if (!stage_out) {
-        WP_CUDA(cudaMemcpyAsync(ids + total, sl.d_ids, cnt * sizeof(int32_t), cudaMemcpyDeviceToHost, v->s_d2h));
-      } else if (cnt <= kStageIds) {
-        WP_CUDA(cudaMemcpyAsync(sl.h_ids, sl.d_ids, cnt * sizeof(int32_t), cudaMemcpyDeviceToHost, v->s_d2h));
+        WP_CUDA(cudaMemcpyAsync(ids + total, sl.d_ids.p, cnt * sizeof(int32_t), cudaMemcpyDeviceToHost, v->s_d2h));
+      } else if (cnt <= sl.h_ids.cap) {
+        WP_CUDA(cudaMemcpyAsync(sl.h_ids.p, sl.d_ids.p, cnt * sizeof(int32_t), cudaMemcpyDeviceToHost, v->s_d2h));
+        staged[j] = cnt;
       } else {
         // more ids than the staging slot holds (text of one- and two-byte tokens): piece by piece, synchronously
-        for (size_t done = 0; done < cnt; done += kStageIds) {
-          const size_t part = cnt - done < kStageIds ? cnt - done : kStageIds;
-          WP_CUDA(cudaMemcpyAsync(sl.h_ids, sl.d_ids + done, part * sizeof(int32_t), cudaMemcpyDeviceToHost, v->s_d2h));
+        for (size_t at = 0; at < cnt; at += sl.h_ids.cap) {
+          const size_t piece = std::min(cnt - at, sl.h_ids.cap);
+          WP_CUDA(cudaMemcpyAsync(sl.h_ids.p, sl.d_ids.p + at, piece * sizeof(int32_t), cudaMemcpyDeviceToHost,
+                                  v->s_d2h));
           WP_CUDA(cudaStreamSynchronize(v->s_d2h));
-          pool.copy(ids + total + done, sl.h_ids, part * sizeof(int32_t));
+          pool.copy(ids + total + at, sl.h_ids.p, piece * sizeof(int32_t));
         }
-        counts[j] = 0;  // already delivered
       }
     }
     WP_CUDA(cudaEventRecord(sl.d2h_done, v->s_d2h));
+    WP_CUDA(trace_stage(v->s_d2h, "part:   [stage] ids on the host"));
     total += cnt;
     return WP_OK;
   };
-  // chunk j's ids have arrived in its pinned slot: hand them to the caller
+  // part j's staged ids have arrived in its slot: hand them to the caller
   auto deliver = [&](size_t j) -> wp_status {
-    if (!stage_out || counts[j] == 0 || overflow || offsets[j] + counts[j] > capacity) return WP_OK;
-    wp_vocab::PipeSlot &sl = v->slot[j % kPipeSlots];
+    if (staged[j] == 0) return WP_OK;
+    wp_vocab::Slot &sl = v->slot[j % kSlots];
     WP_CUDA(cudaEventSynchronize(sl.d2h_done));
-    pool.copy(ids + offsets[j], sl.h_ids, counts[j] * sizeof(int32_t));
+    pool.copy(ids + first_id[j], sl.h_ids.p, staged[j] * sizeof(int32_t));
     return WP_OK;
   };
 
-  for (size_t i = 0; i < n_chunks; i++) {
-    wp_vocab::PipeSlot &sl = v->slot[i % kPipeSlots];
-    const size_t begin = cuts[i], len = cuts[i + 1] - cuts[i];
-    if (i >= kPipeSlots) {  // the slot's previous ids must have left before its buffers are reused
-      WP_CUDA(cudaStreamWaitEvent(v->s_h2d, sl.d2h_done, 0));
-      WP_CUDA(cudaStreamWaitEvent(v->stream, sl.d2h_done, 0));
-    }
-    const char *src = text + begin;
-    if (stage_in) {
-      if (i >= kPipeSlots) WP_CUDA(cudaEventSynchronize(sl.h2d_done));  // the slot's previous text has left
-      pool.copy(sl.h_text, src, len, /*streamed=*/true);
-      src = reinterpret_cast<const char *>(sl.h_text);
-    }
-    WP_CUDA(cudaMemcpyAsync(sl.d_text, src, len, cudaMemcpyHostToDevice, v->s_h2d));
-    WP_CUDA(cudaEventRecord(sl.h2d_done, v->s_h2d));
-    WP_CUDA(cudaStreamWaitEvent(v->stream, sl.h2d_done, 0));
-    st = enqueue_encode(v, sl.d_text, len, sl.d_ids, kPipeChunk, v->stream, 0, &infos[i], /*warm=*/i != 0, n_bytes);
-    if (st != WP_OK) return st;
-    WP_CUDA(cudaMemcpyAsync(sl.h_call, v->d_call, sizeof(wp::CallCounters), cudaMemcpyDeviceToHost, v->stream));
-    WP_CUDA(cudaEventRecord(sl.cmp_done, v->stream));
-    if (i >= 2) {  // (before the slot of chunk i-2 is reused by chunk i+1; its D2H was started an iteration ago)
-      st = deliver(i - 2);
+  // (two more rounds than parts drain the pipeline: the last part is finished, then its staged ids delivered)
+  for (size_t k = 0; k < n_parts + 2 && !*repeat; k++) {
+    wp_status st;
+    if (k < n_parts) {
+      wp_vocab::Slot &sl = v->slot[k % kSlots];
+      const bool reused = k >= kSlots;  // the slot holds part k-3
+      if (reused) {  // its ids must have left before the device reuses its buffers, its input before the host does
+        WP_CUDA(cudaStreamWaitEvent(v->s_h2d, sl.d2h_done, 0));
+        WP_CUDA(cudaStreamWaitEvent(v->stream, sl.d2h_done, 0));
+        if (fill_pinned) WP_CUDA(cudaEventSynchronize(sl.h2d_done));
+      }
+      st = fit_slot(sl, parts[k], fill_pinned, stage_ids, reused);
+      if (st != WP_OK) return st;
+      st = enqueue_part(v, sl, parts[k], fill(k, sl), v->s_h2d, 0, /*warm=*/k != 0, call_bytes, &infos[k]);
       if (st != WP_OK) return st;
     }
-    if (i >= 1) {
-      st = start_d2h(i - 1);
+    if (k >= 2) {  // (before the slot of part k-2 is reused by part k+1; its D2H was started a round ago)
+      st = deliver(k - 2);
       if (st != WP_OK) return st;
     }
+    if (k >= 1 && k <= n_parts) {
+      st = finish(k - 1);
+      if (st != WP_OK) return st;
+      trace("part: previous part finished (ids on their way out)");
+    }
   }
-  if (n_chunks >= 2) {
-    st = deliver(n_chunks - 2);
-    if (st != WP_OK) return st;
-  }
-  st = start_d2h(n_chunks - 1);
-  if (st != WP_OK) return st;
-  st = deliver(n_chunks - 1);
-  if (st != WP_OK) return st;
   WP_CUDA(cudaStreamSynchronize(v->s_d2h));
-  if (overflow) {
-    *fell_back = true;
-    return WP_OK;
-  }
+  WP_CUDA(cudaStreamSynchronize(v->stream));  // (idle unless a void part left later parts in flight)
+  if (*repeat) return WP_OK;
   v->stats = acc;
-  v->stats.n_bytes = n_bytes;
+  v->stats.n_bytes = call_bytes;
   v->stats.n_ids = total;
   *n_ids = total;
-  if (total > capacity) return fail(WP_ERR_CAPACITY, "id buffer too small");
   return WP_OK;
 }
 
@@ -987,47 +1156,12 @@ wp_status wp_vocab_create_from_file(const char *vocab_file, int device, wp_vocab
 }
 
 void wp_vocab_destroy(wp_vocab *v) {
-  if (!v) return;
-  if (v->device >= 0) {
-    DeviceGuard g(v->device);
+  std::optional<DeviceGuard> g;  // (a host-only handle owns no CUDA resource: its teardown makes no CUDA call)
+  if (v && v->device >= 0) {
+    g.emplace(v->device);
     if (v->stream) cudaStreamSynchronize(v->stream);
-    cudaFree(v->d_edges);
-    cudaFree(v->d_words_static);
-    cudaFree(v->d_words_work);
-    cudaFree(v->d_work);
-    cudaFree(v->d_text);
-    cudaFree(v->d_ids);
-    if (v->h_call) cudaFreeHost(v->h_call);
-    for (auto &b : v->bslot) {
-      if (b.h_in) cudaFreeHost(b.h_in);
-      if (b.h_offsets) cudaFreeHost(b.h_offsets);
-      if (b.h_call) cudaFreeHost(b.h_call);
-      cudaFree(b.d_in);
-      cudaFree(b.d_out);
-      cudaFree(b.d_ids);
-      if (b.h2d_done) cudaEventDestroy(b.h2d_done);
-      if (b.cmp_done) cudaEventDestroy(b.cmp_done);
-      if (b.d2h_done) cudaEventDestroy(b.d2h_done);
-    }
-    for (auto &sl : v->slot) {
-      cudaFree(sl.d_text);
-      cudaFree(sl.d_ids);
-      if (sl.h_call) cudaFreeHost(sl.h_call);
-      if (sl.h_text) cudaFreeHost(sl.h_text);
-      if (sl.h_ids) cudaFreeHost(sl.h_ids);
-      if (sl.h2d_done) cudaEventDestroy(sl.h2d_done);
-      if (sl.cmp_done) cudaEventDestroy(sl.cmp_done);
-      if (sl.d2h_done) cudaEventDestroy(sl.d2h_done);
-    }
-    for (cudaEvent_t e : v->timing_events) cudaEventDestroy(e);
-    if (v->last_done) cudaEventDestroy(v->last_done);
-    if (v->s_h2d) cudaStreamDestroy(v->s_h2d);
-    if (v->s_d2h) cudaStreamDestroy(v->s_d2h);
-    cudaFree(v->d_call);
-    cudaFree(v->d_fmt);
-    if (v->stream) cudaStreamDestroy(v->stream);
   }
-  delete v;
+  delete v;  // (the owners free their memory, events and streams on the handle's device)
 }
 
 size_t wp_vocab_size(const wp_vocab *v) { return v ? v->host.tokens.size() : 0; }
@@ -1058,7 +1192,7 @@ wp_status wp_encode_device_async(wp_vocab *v, const void *d_text, size_t n_bytes
   if (st != WP_OK) return st;
   if (d_n_ids) {
     uint64_t launches = 0;
-    WP_CUDA(wp::launch_publish_count(v->d_call, info.n_ranges & 1u, reinterpret_cast<unsigned long long *>(d_n_ids), s,
+    WP_CUDA(wp::launch_publish_count(v->d_call.p, info.n_ranges & 1u, reinterpret_cast<unsigned long long *>(d_n_ids), s,
                                      &launches));
     WP_CUDA(cudaEventRecord(v->last_done, s));  // the count reads the counters the next call clears
     g_launches.fetch_add(launches, std::memory_order_relaxed);
@@ -1096,73 +1230,62 @@ wp_status wp_encode_into(wp_vocab *v, const char *text, size_t n_bytes, int32_t 
   }
   DeviceGuard g(v->device);
   trace("wp_encode_into: begin");
-  if (n_bytes > 2 * pipe_chunk_bytes()) {
-    bool fell_back = false;
-    const wp_status pst = encode_pipelined(v, text, n_bytes, ids, capacity, n_ids, &fell_back);
-    if (pst != WP_OK || !fell_back) return pst;
+  size_t spill = 0;
+  bool repeat = true;
+  std::vector<size_t> cuts;
+  if (n_bytes > 2 * pipe_chunk_bytes() && plan_chunks(text, n_bytes, pipe_chunk_bytes(), &cuts)) {
+    // Pageable caller memory (the reference's own signature hands over a std::string and expects a std::vector)
+    // is staged through the slots' pinned memory by the CopyPool
+    std::vector<PartPlan> chunks(cuts.size() - 1);
+    for (size_t k = 0; k < chunks.size(); k++) chunks[k].packed = chunks[k].in_bytes = cuts[k + 1] - cuts[k];
+    const bool stage_in = is_pageable(text);
+    const wp_status st = run_pipeline(
+        v, chunks, n_bytes, stage_in, capacity > 0 && is_pageable(ids), ids, capacity,
+        [&](size_t k, wp_vocab::Slot &sl) -> const void * {
+          if (!stage_in) return text + cuts[k];
+          CopyPool::get().copy(sl.h_in.p, text + cuts[k], chunks[k].packed, /*streamed=*/true);
+          return sl.h_in.p;
+        },
+        [](size_t, wp_vocab::Slot &, size_t) {}, n_ids, &repeat, &spill);
+    if (st != WP_OK) return st;
   }
-  if (n_bytes > v->text_cap) {
-    cudaFree(v->d_text);
-    v->d_text = nullptr;
-    v->text_cap = 0;
-    const size_t cap = n_bytes + n_bytes / 8 + 256;
-    WP_CUDA(dev_alloc(&v->d_text, cap, 2));
-    v->text_cap = cap;
+  // Void pipelined ids: the whole text once more in one call (through the pipeline, a single part would need
+  // pinned id staging as large as the text).  One id per byte is the worst case (a run of single-byte tokens):
+  // the id buffer holds what the caller can take, bounded by that.
+  if (repeat) {
+    const size_t want = capacity < n_bytes ? capacity : n_bytes;
+    const wp_status st = encode_staged(v, text, n_bytes, want ? want : 1, /*retry_short=*/false, spill);
+    if (st != WP_OK) return st;
+    *n_ids = static_cast<size_t>(v->stats.n_ids);
+    trace("wp_encode_into: ids on the device");
+    if (*n_ids > 0 && *n_ids <= capacity) {
+      WP_CUDA(cudaMemcpyAsync(ids, v->d_ids.p, *n_ids * sizeof(int32_t), cudaMemcpyDeviceToHost, v->stream));
+      WP_CUDA(cudaStreamSynchronize(v->stream));
+      trace("wp_encode_into: ids on the host");
+    }
   }
-  // One id per byte is the worst case (a run of single-byte tokens); allocate what the caller can take,
-  // bounded by that, and retry once with the exact count if the guess was short.
-  size_t want = capacity < n_bytes ? capacity : n_bytes;
-  if (want == 0) want = 1;
-  if (want > v->ids_cap) {
-    cudaFree(v->d_ids);
-    v->d_ids = nullptr;
-    v->ids_cap = 0;
-    WP_CUDA(dev_alloc(&v->d_ids, want * sizeof(int32_t), 2));
-    v->ids_cap = want;
-  }
-  WP_CUDA(cudaMemcpyAsync(v->d_text, text, n_bytes, cudaMemcpyHostToDevice, v->stream));
-  wp_status st = run_encode(v, v->d_text, n_bytes, v->d_ids, v->ids_cap, v->stream);
-  if (st != WP_OK) return st;
-  *n_ids = static_cast<size_t>(v->stats.n_ids);
-  if (v->stats.n_ids > capacity) return fail(WP_ERR_CAPACITY, "id buffer too small");
-  trace("wp_encode_into: ids on the device");
-  if (*n_ids > 0) {
-    WP_CUDA(cudaMemcpyAsync(ids, v->d_ids, *n_ids * sizeof(int32_t), cudaMemcpyDeviceToHost, v->stream));
-    WP_CUDA(cudaStreamSynchronize(v->stream));
-  }
-  trace("wp_encode_into: ids on the host");
-  return WP_OK;
+  return *n_ids > capacity ? fail(WP_ERR_CAPACITY, "id buffer too small") : WP_OK;
 }
 
-// Host text -> ids in the handle's device buffer v->d_ids (count in v->stats.n_ids).
+// Host text -> ids in the handle's device buffer v->d_ids (count in v->stats.n_ids).  First guess: half an id per
+// byte (English-like text needs ~0.25); exact retry if short.
 static wp_status encode_to_device_buffer(wp_vocab *v, const char *text, size_t n_bytes) {
-  if (n_bytes > v->text_cap) {
-    cudaFree(v->d_text);
-    v->d_text = nullptr;
-    v->text_cap = 0;
-    const size_t cap = n_bytes + n_bytes / 8 + 256;
-    WP_CUDA(dev_alloc(&v->d_text, cap, 2));
-    v->text_cap = cap;
-  }
-  // first guess: half an id per byte (English-like text needs ~0.25); exact retry if short
-  size_t guess = n_bytes / 2 + 1024;
-  if (guess > n_bytes) guess = n_bytes;
-  WP_CUDA(cudaMemcpyAsync(v->d_text, text, n_bytes, cudaMemcpyHostToDevice, v->stream));
-  for (int attempt = 0; attempt < 2; attempt++) {
-    if (guess > v->ids_cap) {
-      cudaFree(v->d_ids);
-      v->d_ids = nullptr;
-      v->ids_cap = 0;
-      WP_CUDA(dev_alloc(&v->d_ids, guess * sizeof(int32_t), 2));
-      v->ids_cap = guess;
+  return encode_staged(v, text, n_bytes, std::min(n_bytes, n_bytes / 2 + 1024), /*retry_short=*/true);
+}
+
+// n bytes of device memory -> a new malloc block of n + extra bytes (at least one), for the caller to free
+static wp_status download(wp_vocab *v, const void *d_src, size_t n, size_t extra, const char *what, void **out) {
+  void *host = std::malloc(n + extra ? n + extra : 1);
+  if (!host) return fail(WP_ERR_NOMEM, "out of memory");
+  if (n > 0) {
+    cudaError_t e = cudaMemcpyAsync(host, d_src, n, cudaMemcpyDeviceToHost, v->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(v->stream);
+    if (e != cudaSuccess) {
+      std::free(host);
+      return fail(WP_ERR_CUDA, std::string(what) + cudaGetErrorString(e));
     }
-    const uint64_t before = v->stats.kernel_launches;
-    wp_status st = run_encode(v, v->d_text, n_bytes, v->d_ids, v->ids_cap, v->stream);
-    if (st != WP_OK) return st;
-    if (attempt) v->stats.kernel_launches += before;
-    if (v->stats.n_ids <= v->ids_cap) break;
-    guess = static_cast<size_t>(v->stats.n_ids);
   }
+  *out = host;
   return WP_OK;
 }
 
@@ -1182,199 +1305,13 @@ wp_status wp_encode(wp_vocab *v, const char *text, size_t n_bytes, int32_t **ids
   if (st != WP_OK) return st;
   trace("wp_encode: ids on the device");
   const size_t cnt = static_cast<size_t>(v->stats.n_ids);
-  int32_t *host = static_cast<int32_t *>(std::malloc(cnt ? cnt * sizeof(int32_t) : 1));
-  if (!host) return fail(WP_ERR_NOMEM, "out of memory");
-  if (cnt > 0) {
-    cudaError_t e = cudaMemcpyAsync(host, v->d_ids, cnt * sizeof(int32_t), cudaMemcpyDeviceToHost, v->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(v->stream);
-    if (e != cudaSuccess) {
-      std::free(host);
-      return fail(WP_ERR_CUDA, std::string("copy ids: ") + cudaGetErrorString(e));
-    }
-  }
-  *ids_out = host;
+  void *host = nullptr;
+  const wp_status dst = download(v, v->d_ids.p, cnt * sizeof(int32_t), 0, "copy ids: ", &host);
+  if (dst != WP_OK) return dst;
+  *ids_out = static_cast<int32_t *>(host);
   *n_ids = cnt;
   return WP_OK;
 }
-
-/* ------------------------------------------------------------------ batch of texts
- * The texts are packed into one buffer, each followed by one space: a space ends every word and resets the
- * matcher's state (fast.cpp:89-91), a byte sequence cut short at the end of a text stays invalid in front of
- * it, so the ids of the packed buffer are the ids of the texts one after the other.  K1 numbers the first
- * segment of every text, K5 turns the numbers into id offsets (wp_encode.h).  A large batch is cut into parts
- * of whole texts that go through a pipeline like the one of wp_encode_into: part k+1 is packed (all threads
- * of the CopyPool) and copied in while part k is encoded and the ids of part k-1 are copied out. */
-}  // extern "C"
-
-namespace {
-
-constexpr size_t kBatchPart = size_t(8) << 20;  // packed bytes per part of a large batch
-
-size_t batch_part_bytes() {
-  if (const char *e = std::getenv("WORDPIECE_B200_BATCH_PART")) {  // test hook: pipeline small batches
-    const long long x = std::atoll(e);
-    if (x >= 256 && static_cast<size_t>(x) <= kBatchPart) return static_cast<size_t>(x);
-  }
-  return kBatchPart;
-}
-
-// Layout of a part's input block: tile index | text starts | packed texts (16-byte aligned for K1's vector loads)
-struct PartPlan {
-  size_t first = 0, last = 0;  // texts [first, last)
-  size_t packed = 0;           // bytes incl. one separator per text
-  size_t n_tiles = 0, off_bounds = 0, off_text = 0, in_bytes = 0, off_offsets = 0, out_bytes = 0;
-};
-
-PartPlan plan_part(const size_t *lens, size_t first, size_t last) {
-  PartPlan p;
-  p.first = first;
-  p.last = last;
-  const size_t n = last - first;
-  p.packed = n;
-  for (size_t i = first; i < last; i++) p.packed += lens[i];
-  const size_t tile = wp::encode_tile_bytes();
-  p.n_tiles = (p.packed + tile - 1) / tile;
-  p.off_bounds = align_up((p.n_tiles + 1) * sizeof(uint32_t), 256);
-  p.off_text = align_up(p.off_bounds + n * sizeof(unsigned long long), 256);
-  p.in_bytes = p.off_text + p.packed;
-  p.off_offsets = align_up(n * sizeof(uint32_t), 256);
-  p.out_bytes = p.off_offsets + (n + 1) * sizeof(unsigned long long);
-  return p;
-}
-
-wp_status ensure_batch_slot(wp_vocab::BatchSlot &b, const PartPlan &p, size_t ids_want) {
-  const size_t n = p.last - p.first;
-  if (p.in_bytes > b.in_cap) {
-    if (b.h_in) cudaFreeHost(b.h_in);
-    cudaFree(b.d_in);
-    b.h_in = b.d_in = nullptr;
-    b.in_cap = 0;
-    const size_t cap = p.in_bytes + p.in_bytes / 4 + 4096;
-    WP_CUDA(cudaMallocHost(&b.h_in, cap));
-    WP_CUDA(dev_alloc(&b.d_in, cap, 4));
-    b.in_cap = cap;
-  }
-  if (p.out_bytes > b.out_cap) {
-    cudaFree(b.d_out);
-    b.d_out = nullptr;
-    b.out_cap = 0;
-    const size_t cap = p.out_bytes + p.out_bytes / 4 + 256;
-    WP_CUDA(dev_alloc(&b.d_out, cap, 8));
-    b.out_cap = cap;
-  }
-  if (n + 1 > b.offsets_cap) {
-    if (b.h_offsets) cudaFreeHost(b.h_offsets);
-    b.h_offsets = nullptr;
-    b.offsets_cap = 0;
-    const size_t cap = n + 1 + n / 4 + 64;
-    WP_CUDA(cudaMallocHost(&b.h_offsets, cap * sizeof(unsigned long long)));
-    b.offsets_cap = cap;
-  }
-  if (ids_want > b.ids_cap) {
-    cudaFree(b.d_ids);
-    b.d_ids = nullptr;
-    b.ids_cap = 0;
-    const size_t cap = ids_want + ids_want / 8 + 256;
-    WP_CUDA(dev_alloc(&b.d_ids, cap * sizeof(int32_t), 2));
-    b.ids_cap = cap;
-  }
-  if (!b.h_call) {
-    WP_CUDA(cudaMallocHost(&b.h_call, sizeof(wp::CallCounters)));
-    WP_CUDA(cudaEventCreateWithFlags(&b.h2d_done, cudaEventDisableTiming));
-    WP_CUDA(cudaEventCreateWithFlags(&b.cmp_done, cudaEventDisableTiming));
-    WP_CUDA(cudaEventCreateWithFlags(&b.d2h_done, cudaEventDisableTiming));
-  }
-  return WP_OK;
-}
-
-// texts -> the part's pinned input block (text starts, tile index, the texts with their separators)
-void pack_part(wp_vocab::BatchSlot &b, const PartPlan &p, const char *const *texts, const size_t *lens,
-               bool streamed = stream_stores()) {
-  const size_t n = p.last - p.first;
-  uint32_t *tile_bound = reinterpret_cast<uint32_t *>(b.h_in);
-  unsigned long long *bounds = reinterpret_cast<unsigned long long *>(b.h_in + p.off_bounds);
-  char *text = reinterpret_cast<char *>(b.h_in + p.off_text);
-  unsigned long long at = 0;
-  for (size_t i = 0; i < n; i++) {
-    bounds[i] = at;
-    at += lens[p.first + i] + 1;
-  }
-  auto pack = [&](size_t part, size_t parts) {  // equal byte shares, whole texts
-    const unsigned long long lo = static_cast<unsigned long long>(p.packed) * part / parts;
-    const unsigned long long hi = static_cast<unsigned long long>(p.packed) * (part + 1) / parts;
-    size_t i = static_cast<size_t>(std::lower_bound(bounds, bounds + n, lo) - bounds);
-    const size_t end = part + 1 == parts ? n : static_cast<size_t>(std::lower_bound(bounds, bounds + n, hi) - bounds);
-    if (streamed) {  // (the texts of a share are contiguous in the packed buffer)
-      if (i >= end) return;
-      StreamWriter w(text + bounds[i]);
-      for (; i < end; i++) {
-        w.put(texts[p.first + i], lens[p.first + i]);
-        w.put(' ');
-      }
-      w.finish();
-      return;
-    }
-    for (; i < end; i++) {
-      char *dst = text + bounds[i];
-      const size_t len = lens[p.first + i];
-      if (len) std::memcpy(dst, texts[p.first + i], len);
-      dst[len] = ' ';
-    }
-  };
-  if (p.packed >= (size_t(1) << 20)) {
-    CopyPool::get().run(pack);
-  } else {
-    pack(0, 1);
-  }
-  const size_t tile = wp::encode_tile_bytes();
-  size_t i = 0;
-  for (size_t t = 0; t <= p.n_tiles; t++) {  // tile_bound[t] = first text that starts at or after byte t * tile
-    const unsigned long long lo = static_cast<unsigned long long>(t) * tile;
-    while (i < n && bounds[i] < lo) i++;
-    tile_bound[t] = static_cast<uint32_t>(i);
-  }
-}
-
-// Enqueue one part: H2D of its input block on `copy_stream`, kernels + id offsets + counters on v->stream.
-wp_status enqueue_part(wp_vocab *v, wp_vocab::BatchSlot &b, const PartPlan &p, cudaStream_t copy_stream, size_t spill,
-                       bool warm, size_t call_bytes, EnqueueInfo *info) {
-  const size_t n = p.last - p.first;
-  BatchArgs batch;
-  batch.h_bounds = reinterpret_cast<const unsigned long long *>(b.h_in + p.off_bounds);
-  batch.n_texts = n;
-  batch.d_tile_bound = reinterpret_cast<const uint32_t *>(b.d_in);
-  batch.d_bounds = reinterpret_cast<const unsigned long long *>(b.d_in + p.off_bounds);
-  batch.d_bound_seg = reinterpret_cast<uint32_t *>(b.d_out);
-  batch.d_offsets = reinterpret_cast<unsigned long long *>(b.d_out + p.off_offsets);
-  WP_CUDA(cudaMemcpyAsync(b.d_in, b.h_in, p.in_bytes, cudaMemcpyHostToDevice, copy_stream));
-  if (trace_stage_sync()) {
-    WP_CUDA(cudaStreamSynchronize(copy_stream));
-    trace("wp_encode_batch:   [stage] input block on the device");
-  }
-  if (copy_stream != v->stream) {
-    WP_CUDA(cudaEventRecord(b.h2d_done, copy_stream));
-    WP_CUDA(cudaStreamWaitEvent(v->stream, b.h2d_done, 0));
-  }
-  wp_status st = enqueue_encode(v, b.d_in + p.off_text, p.packed, b.d_ids, b.ids_cap, v->stream, spill, info, warm, call_bytes, &batch);
-  if (st != WP_OK) return st;
-  if (trace_stage_sync()) {
-    WP_CUDA(cudaStreamSynchronize(v->stream));
-    trace("wp_encode_batch:   [stage] kernels done");
-  }
-  uint64_t launches = 0;
-  WP_CUDA(wp::launch_publish_count(v->d_call, info->n_ranges & 1u, batch.d_offsets + n, v->stream, &launches));
-  WP_CUDA(cudaEventRecord(v->last_done, v->stream));
-  g_launches.fetch_add(launches, std::memory_order_relaxed);
-  info->launches += launches;
-  WP_CUDA(cudaMemcpyAsync(b.h_offsets, batch.d_offsets, (n + 1) * sizeof(unsigned long long), cudaMemcpyDeviceToHost, v->stream));
-  WP_CUDA(cudaMemcpyAsync(b.h_call, v->d_call, sizeof(wp::CallCounters), cudaMemcpyDeviceToHost, v->stream));
-  WP_CUDA(cudaEventRecord(b.cmp_done, v->stream));
-  return WP_OK;
-}
-
-}  // namespace
-
-extern "C" {
 
 wp_status wp_encode_batch(wp_vocab *v, const char *const *texts, const size_t *lens, size_t n_texts, int32_t *ids,
                           size_t capacity, size_t *offsets, size_t *n_ids) {
@@ -1396,117 +1333,54 @@ wp_status wp_encode_batch(wp_vocab *v, const char *const *texts, const size_t *l
   }
   DeviceGuard g(v->device);
   trace("wp_encode_batch: begin");
-  // parts of whole texts, about kBatchPart packed bytes each (one part: the whole batch in one go)
+  // a large batch: parts of whole texts, about kBatchPart packed bytes each
   std::vector<PartPlan> parts;
   const size_t part_bytes = batch_part_bytes();
-  if (packed <= 3 * part_bytes / 2) {
-    parts.push_back(plan_part(lens, 0, n_texts));
-  } else {
-    size_t first = 0, bytes = 0;
-    for (size_t i = 0; i < n_texts; i++) {
-      bytes += lens[i] + 1;
-      if (bytes >= part_bytes || i + 1 == n_texts) {
-        parts.push_back(plan_part(lens, first, i + 1));
-        first = i + 1;
-        bytes = 0;
-      }
+  for (size_t i = 0, first = 0, bytes = 0; packed > 3 * part_bytes / 2 && i < n_texts; i++) {
+    bytes += lens[i] + 1;
+    if (bytes >= part_bytes || i + 1 == n_texts) {
+      parts.push_back(plan_part(lens, first, i + 1));
+      first = i + 1;
+      bytes = 0;
     }
   }
-  const size_t n_parts = parts.size();
-  if (n_parts > 1) {
-    const wp_status st = ensure_pipeline(v);  // (its copy streams)
-    if (st != WP_OK) return st;
-  }
-  std::vector<EnqueueInfo> infos(n_parts);
-  wp_stats acc{};
-  size_t total = 0;
   static_assert(sizeof(size_t) == sizeof(unsigned long long), "offsets are copied as they are");
-
-  // part j's kernels are done: its offsets go to the caller (rebased), its ids start their way device -> host
-  auto finish_part = [&](size_t j, bool *overflow) -> wp_status {
-    wp_vocab::BatchSlot &b = v->bslot[j % 3];
-    const PartPlan &p = parts[j];
-    const size_t n = p.last - p.first;
-    WP_CUDA(cudaEventSynchronize(b.cmp_done));
-    size_t spill = 0;  // (a void part is not repeated: the whole batch is, as one part, see below)
-    *overflow = absorb_call(v, *b.h_call, infos[j], p.packed, &acc, &spill);
-    if (*overflow) return WP_OK;
-    const size_t cnt = static_cast<size_t>(b.h_offsets[n]);
-    for (size_t i = 0; i < n; i++) offsets[p.first + i] = total + static_cast<size_t>(b.h_offsets[i]);
-    cudaStream_t out_stream = n_parts > 1 ? v->s_d2h : v->stream;
-    if (cnt > 0 && total + cnt <= capacity) {
-      if (n_parts > 1) WP_CUDA(cudaStreamWaitEvent(out_stream, b.cmp_done, 0));
-      WP_CUDA(cudaMemcpyAsync(ids + total, b.d_ids, cnt * sizeof(int32_t), cudaMemcpyDeviceToHost, out_stream));
-    }
-    WP_CUDA(cudaEventRecord(b.d2h_done, out_stream));
-    if (trace_stage_sync()) {
-      WP_CUDA(cudaStreamSynchronize(out_stream));
-      trace("wp_encode_batch:   [stage] ids on the host");
-    }
-    total += cnt;
-    return WP_OK;
-  };
-
-  bool overflow = false;
-  for (size_t k = 0; k < n_parts && !overflow; k++) {
-    wp_vocab::BatchSlot &b = v->bslot[k % 3];
-    const PartPlan &p = parts[k];
-    const size_t want = p.packed;  // one id per byte is the worst case
-    if (k >= 3) WP_CUDA(cudaEventSynchronize(b.d2h_done));  // the slot's previous part has left (host and device buffers)
-    wp_status st = ensure_batch_slot(b, p, want);
-    if (st != WP_OK) return st;
-    trace("wp_encode_batch: part: buffers ready");
-    pack_part(b, p, texts, lens);
+  auto fill = [&](size_t k, wp_vocab::Slot &sl) -> const void * {
+    pack_part(sl.h_in.p, parts[k], texts, lens);
     trace("wp_encode_batch: part packed");
-    st = enqueue_part(v, b, p, n_parts > 1 ? v->s_h2d : v->stream, 0, /*warm=*/k != 0, packed, &infos[k]);
+    return sl.h_in.p;
+  };
+  auto rebase = [&](size_t k, const wp_vocab::Slot &sl, size_t first_id) {  // part k's offsets
+    const PartPlan &p = parts[k];
+    for (size_t i = p.first; i < p.last; i++) offsets[i] = first_id + static_cast<size_t>(sl.h_offsets.p[i - p.first]);
+  };
+  size_t spill = 0;
+  bool repeat = true;  // (a small batch goes as one part)
+  if (parts.size() > 1) {
+    const wp_status st = run_pipeline(v, parts, packed, /*fill_pinned=*/true, /*stage_out=*/false, ids, capacity,
+                                      fill, rebase, n_ids, &repeat, &spill);
     if (st != WP_OK) return st;
-    trace("wp_encode_batch: part enqueued");
-    if (k >= 1) {
-      st = finish_part(k - 1, &overflow);
-      if (st != WP_OK) return st;
-      trace("wp_encode_batch: previous part finished (ids on their way out)");
-    }
   }
-  if (!overflow) {
-    const wp_status st = finish_part(n_parts - 1, &overflow);
-    if (st != WP_OK) return st;
-  }
-  if (overflow) {
-    // the ids of some part are void (rare: a long segment outgrew the default id spill, or K1 has to change its
-    // mode): the whole batch again as ONE part with a spill as large as the text, nothing pipelined, repeated
-    // while its ids are void as in run_encode
-    WP_CUDA(cudaStreamSynchronize(v->stream));
-    if (n_parts > 1) WP_CUDA(cudaStreamSynchronize(v->s_d2h));
+  if (repeat) {  // the whole batch as one part: a small batch, or a pipelined one whose ids are void
     parts.assign(1, plan_part(lens, 0, n_texts));
-    wp_vocab::BatchSlot &b = v->bslot[0];
-    wp_status st = ensure_batch_slot(b, parts[0], packed);
+    const PartPlan &whole = parts[0];
+    wp_vocab::Slot &sl = v->slot[0];
+    wp_status st = fit_slot(sl, whole, /*fill_pinned=*/true, 0, /*in_use=*/false);
     if (st != WP_OK) return st;
-    pack_part(b, parts[0], texts, lens);
-    size_t spill = packed + 4096;
-    for (int attempt = 0; overflow; attempt++) {
-      if (attempt == kMaxAttempts) return fail(WP_ERR_CUDA, "internal scratch overflow");
-      EnqueueInfo info;
-      st = enqueue_part(v, b, parts[0], v->stream, spill, false, packed, &info);
-      if (st != WP_OK) return st;
-      WP_CUDA(cudaEventSynchronize(b.cmp_done));
-      acc = wp_stats{};
-      overflow = absorb_call(v, *b.h_call, info, packed, &acc, &spill);
-    }
-    const size_t cnt = static_cast<size_t>(b.h_offsets[n_texts]);
-    for (size_t i = 0; i < n_texts; i++) offsets[i] = static_cast<size_t>(b.h_offsets[i]);
-    if (cnt > 0 && cnt <= capacity) WP_CUDA(cudaMemcpyAsync(ids, b.d_ids, cnt * sizeof(int32_t), cudaMemcpyDeviceToHost, v->stream));
-    total = cnt;
+    const void *src = fill(0, sl);
+    st = repeat_call(v, v->stream, packed, spill, *sl.h_call.p, [&](size_t sp, EnqueueInfo *info) {
+      return enqueue_part(v, sl, whole, src, v->stream, sp, /*warm=*/false, packed, info);
+    });
+    if (st != WP_OK) return st;
+    *n_ids = static_cast<size_t>(v->stats.n_ids);
+    rebase(0, sl, 0);
+    if (*n_ids > 0 && *n_ids <= capacity)
+      WP_CUDA(cudaMemcpyAsync(ids, sl.d_ids.p, *n_ids * sizeof(int32_t), cudaMemcpyDeviceToHost, v->stream));
+    WP_CUDA(cudaStreamSynchronize(v->stream));
   }
-  WP_CUDA(cudaStreamSynchronize(v->stream));
-  if (n_parts > 1) WP_CUDA(cudaStreamSynchronize(v->s_d2h));
   trace("wp_encode_batch: ids on the host");
-  offsets[n_texts] = total;
-  v->stats = acc;
-  v->stats.n_bytes = packed;
-  v->stats.n_ids = total;
-  *n_ids = total;
-  if (total > capacity) return fail(WP_ERR_CAPACITY, "id buffer too small");
-  return WP_OK;
+  offsets[n_texts] = *n_ids;
+  return *n_ids > capacity ? fail(WP_ERR_CAPACITY, "id buffer too small") : WP_OK;
 }
 
 size_t wp_next_safe_cut(const char *text, size_t n_bytes, size_t pos) {
@@ -1592,14 +1466,14 @@ static wp_status encode_sharded(wp_vocab *const *handles, size_t n, const char *
       if (v->device != gather_device) {
         cudaDeviceEnablePeerAccess(gather_device, 0);  // best effort: without it the copy is staged through the host
         cudaGetLastError();
-        WP_CUDA(cudaMemcpyPeerAsync(d_gather + info[i].id_offset, gather_device, v->d_ids, v->device,
+        WP_CUDA(cudaMemcpyPeerAsync(d_gather + info[i].id_offset, gather_device, v->d_ids.p, v->device,
                                     cnt * sizeof(int32_t), v->stream));
       } else {
-        WP_CUDA(cudaMemcpyAsync(d_gather + info[i].id_offset, v->d_ids, cnt * sizeof(int32_t), cudaMemcpyDeviceToDevice,
+        WP_CUDA(cudaMemcpyAsync(d_gather + info[i].id_offset, v->d_ids.p, cnt * sizeof(int32_t), cudaMemcpyDeviceToDevice,
                                 v->stream));
       }
     } else {
-      WP_CUDA(cudaMemcpyAsync(h_ids + info[i].id_offset, v->d_ids, cnt * sizeof(int32_t), cudaMemcpyDeviceToHost,
+      WP_CUDA(cudaMemcpyAsync(h_ids + info[i].id_offset, v->d_ids.p, cnt * sizeof(int32_t), cudaMemcpyDeviceToHost,
                               v->stream));
     }
     WP_CUDA(cudaStreamSynchronize(v->stream));
@@ -1631,56 +1505,34 @@ wp_status wp_encode_text(wp_vocab *v, const char *text, size_t n_bytes, char **o
   *out_len = 0;
   *n_ids = 0;
   if (v->device < 0) return fail(WP_ERR_NO_DEVICE, kHostOnly);
-  if (n_bytes == 0) {
-    v->stats = wp_stats{};
-    *out = static_cast<char *>(std::malloc(1));
-    if (!*out) return fail(WP_ERR_NOMEM, "out of memory");
-    (*out)[0] = 0;
-    return WP_OK;
-  }
   DeviceGuard g(v->device);
-  wp_status st = encode_to_device_buffer(v, text, n_bytes);
+  v->stats = wp_stats{};
+  wp_status st = n_bytes ? encode_to_device_buffer(v, text, n_bytes) : WP_OK;  // (no text: "", as fast.cpp:145)
   if (st != WP_OK) return st;
   const size_t cnt = static_cast<size_t>(v->stats.n_ids);
   unsigned long long total = 0;
-  char *host = nullptr;
   if (cnt > 0) {
     // the encode scratch is idle now: [0] total length, [1] ticket, then one look-back word per block
     const size_t n_blocks = (cnt + wp::format_block_ids() - 1) / wp::format_block_ids();
     const size_t need = (2 + n_blocks) * sizeof(unsigned long long);
-    st = ensure_work(v, need);
-    if (st != WP_OK) return st;
-    unsigned long long *w = reinterpret_cast<unsigned long long *>(v->d_work);
+    WP_CUDA(v->d_work.grow(need));
+    unsigned long long *w = reinterpret_cast<unsigned long long *>(v->d_work.p);
     WP_CUDA(cudaMemsetAsync(w, 0, need, v->stream));
     uint64_t launches = 0;
-    WP_CUDA(wp::launch_format_total(v->d_ids, cnt, w, v->sm_count, v->stream, &launches));
+    WP_CUDA(wp::launch_format_total(v->d_ids.p, cnt, w, v->sm_count, v->stream, &launches));
     WP_CUDA(cudaMemcpyAsync(&total, w, sizeof(total), cudaMemcpyDeviceToHost, v->stream));
     WP_CUDA(cudaStreamSynchronize(v->stream));
-    if (total > v->fmt_cap) {
-      cudaFree(v->d_fmt);
-      v->d_fmt = nullptr;
-      v->fmt_cap = 0;
-      const size_t cap = static_cast<size_t>(total) + static_cast<size_t>(total) / 8 + 256;
-      WP_CUDA(dev_alloc(&v->d_fmt, cap));
-      v->fmt_cap = cap;
-    }
-    WP_CUDA(wp::launch_format(v->d_ids, cnt, v->d_fmt, w + 2, reinterpret_cast<unsigned int *>(w + 1), v->sm_count,
+    WP_CUDA(v->d_fmt.grow(static_cast<size_t>(total)));
+    WP_CUDA(wp::launch_format(v->d_ids.p, cnt, v->d_fmt.p, w + 2, reinterpret_cast<unsigned int *>(w + 1), v->sm_count,
                               v->stream, &launches));
     g_launches.fetch_add(launches, std::memory_order_relaxed);
     v->stats.kernel_launches += launches;
   }
-  host = static_cast<char *>(std::malloc(static_cast<size_t>(total) + 1));
-  if (!host) return fail(WP_ERR_NOMEM, "out of memory");
-  if (total > 0) {
-    cudaError_t e = cudaMemcpyAsync(host, v->d_fmt, static_cast<size_t>(total), cudaMemcpyDeviceToHost, v->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(v->stream);
-    if (e != cudaSuccess) {
-      std::free(host);
-      return fail(WP_ERR_CUDA, std::string("copy id text: ") + cudaGetErrorString(e));
-    }
-  }
-  host[total] = 0;
-  *out = host;
+  void *block = nullptr;
+  st = download(v, v->d_fmt.p, static_cast<size_t>(total), 1, "copy id text: ", &block);
+  if (st != WP_OK) return st;
+  *out = static_cast<char *>(block);
+  (*out)[total] = 0;
   *out_len = static_cast<size_t>(total);
   *n_ids = cnt;
   return WP_OK;
@@ -1813,12 +1665,10 @@ size_t wp_debug_stage(const char *const *texts, const size_t *lens, size_t n, ch
   }
   const PartPlan p = plan_part(lens, 0, n);
   if (p.packed > out_cap) return 0;
-  wp_vocab::BatchSlot b;
   void *block = nullptr;
   if (posix_memalign(&block, 256, p.in_bytes + 64) != 0) return 0;
-  b.h_in = static_cast<uint8_t *>(block);
-  pack_part(b, p, texts, lens, mode == 1);
-  std::memcpy(out, b.h_in + p.off_text, p.packed);
+  pack_part(static_cast<uint8_t *>(block), p, texts, lens, mode == 1);
+  std::memcpy(out, static_cast<uint8_t *>(block) + p.off_text, p.packed);
   std::free(block);
   return p.packed;
 }
