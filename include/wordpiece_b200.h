@@ -174,6 +174,25 @@ wp_status wp_encode_sharded_gather(wp_vocab *const *handles, size_t n_handles, c
 wp_status wp_encode_batch(wp_vocab *v, const char *const *texts, const size_t *lens, size_t n_texts, int32_t *ids,
                           size_t capacity, size_t *offsets, size_t *n_ids);
 
+/* Device string column -> device ids.  Text i is d_chars[d_offsets[i] .. d_offsets[i + 1]) (Arrow layout: n_texts + 1
+ * uint64 offsets into a buffer of n_chars bytes; d_offsets[0] need not be 0).  Every text is encoded exactly as
+ * fast::encode(text_i, vocab) would encode it.  Its ids are d_ids[d_id_offsets[i] .. d_id_offsets[i + 1]), and
+ * d_id_offsets[n_texts] is the total.  Both offset arrays are in device memory of the handle's device.  The column
+ * is packed on the device as wp_encode_batch packs host texts (n_chars + n_texts bytes) and encoded by one call of
+ * the kernels on `stream` (NULL = the CUDA default stream), which is then synchronised.  WP_ERR_CAPACITY (with
+ * *n_ids and d_id_offsets set) if capacity is short (n_chars ids always suffice); WP_ERR_INVALID_ARG if the offsets
+ * do not ascend or end past n_chars.  n_texts == 0: d_id_offsets[0] = 0 and no kernel runs. */
+wp_status wp_encode_batch_device(wp_vocab *v, const void *d_chars, size_t n_chars, const uint64_t *d_offsets,
+                                 size_t n_texts, int32_t *d_ids, size_t capacity, uint64_t *d_id_offsets, size_t *n_ids,
+                                 void *stream);
+
+/* As above but fully asynchronous, with the contract of wp_encode_device_async: if the call outgrows its scratch,
+ * or the column is malformed, d_id_offsets[n_texts] is UINT64_MAX and the ids are incomplete — repeat the call
+ * through wp_encode_batch_device.  Host-side argument errors are reported at once. */
+wp_status wp_encode_batch_device_async(wp_vocab *v, const void *d_chars, size_t n_chars, const uint64_t *d_offsets,
+                                       size_t n_texts, int32_t *d_ids, size_t capacity, uint64_t *d_id_offsets,
+                                       void *stream);
+
 /* Counters of the last completed encode call on the handle (every encode entry point sets them; for a pipelined
  * call they are summed over its parts). */
 wp_status wp_last_stats(wp_vocab *v, wp_stats *out);

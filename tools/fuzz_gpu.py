@@ -59,13 +59,14 @@ def main():
         else:
             os.environ.pop("WORDPIECE_B200_PIPE_CHUNK", None)
         os.environ["WORDPIECE_B200_TICKET"] = "1" if rng.random() < 0.1 else "0"
-        entry = rng.choice(["encode", "encode_into", "encode_into_pinned", "encode_device", "encode_text", "encode_batch"])
+        entry = rng.choice(["encode", "encode_into", "encode_into_pinned", "encode_device", "encode_text", "encode_batch",
+                            "encode_batch_device"])
         v = wordpiece_b200.Vocab(vocab, device=0)
         if rng.random() < 0.3:  # a handle that has already encoded something else (scratch, memo and shared memory in use)
             other, _ = textgen.case(seed + 77777, min(n, 200000), **kw)
             v.encode(other)
         try:
-            if entry == "encode_batch":
+            if entry in ("encode_batch", "encode_batch_device"):
                 # the text cut at arbitrary BYTE positions (also inside a UTF-8 sequence, inside a word): every piece
                 # must get the ids the oracle gives that piece alone
                 k_cuts = rng.choice([0, 1, 3, 17, 200, 3000])
@@ -78,7 +79,19 @@ def main():
                 o = Oracle(vocab)
                 exp_parts = [o.encode(p) for p in pieces]
                 exp = np.concatenate(exp_parts) if exp_parts else np.zeros(0, np.int32)
-                got, offs = v.encode_batch(pieces)
+                if entry == "encode_batch":
+                    got, offs = v.encode_batch(pieces)
+                else:
+                    # the pieces as a slice of a larger column: unused bytes before and after, d_offsets[0] > 0, and
+                    # d_chars at any alignment
+                    lead, trail, shift = rng.randrange(1, 5000), rng.randrange(0, 5000), rng.randrange(0, 16)
+                    blob = bytes(rng.randrange(256) for _ in range(shift + lead)) + text + b"\xff" * trail
+                    base = torch.frombuffer(bytearray(blob), dtype=torch.uint8).cuda()
+                    d_chars = base[shift:]
+                    d_offsets = torch.tensor([lead] + [lead + c for c in cuts] + [lead + len(text)], dtype=torch.int64,
+                                             device="cuda")
+                    d_ids, d_offs, k = v.encode_batch_device(d_chars, d_offsets)
+                    got, offs = d_ids[:k].cpu().numpy(), d_offs.cpu().numpy()
                 exp_offs = np.concatenate([[0], np.cumsum([len(e) for e in exp_parts])])
                 assert np.array_equal(np.asarray(offs, dtype=np.int64), exp_offs.astype(np.int64)), "text offsets differ"
             elif entry == "encode":

@@ -82,6 +82,8 @@ EXPORTED_SYMBOLS = [
     "wp_encode_sharded",
     "wp_encode_sharded_gather",
     "wp_encode_batch",
+    "wp_encode_batch_device",
+    "wp_encode_batch_device_async",
     "wp_last_stats",
     "wp_set_kernel_timing",
     "wp_last_kernel_ms",
@@ -148,6 +150,11 @@ def load_library() -> C.CDLL:
         L.wp_encode_batch.restype = C.c_int
     L.wp_encode_device_async.argtypes = [vp, vp, sz, vp, sz, vp, vp]
     L.wp_encode_device_async.restype = C.c_int
+    if hasattr(L, "wp_encode_batch_device"):  # (as wp_encode_batch: an older build may lack it)
+        L.wp_encode_batch_device.argtypes = [vp, vp, sz, vp, sz, vp, sz, vp, C.POINTER(sz), vp]
+        L.wp_encode_batch_device.restype = C.c_int
+        L.wp_encode_batch_device_async.argtypes = [vp, vp, sz, vp, sz, vp, sz, vp, vp]
+        L.wp_encode_batch_device_async.restype = C.c_int
     L.wp_plan_shards.argtypes = [vp, sz, sz, C.POINTER(sz)]
     L.wp_plan_shards.restype = sz
     L.wp_next_safe_cut.argtypes = [vp, sz, sz]
@@ -436,6 +443,56 @@ class Vocab:
             stream = torch.cuda.current_stream(d_text.device).cuda_stream
         _check(self._L.wp_encode_device_async(self._h, d_text.data_ptr(), d_text.numel(), d_ids.data_ptr(),
                                               d_ids.numel(), d_count.data_ptr(), stream))
+
+    @staticmethod
+    def _column(d_chars, d_offsets, d_ids, d_id_offsets):
+        import torch
+
+        assert d_chars.is_cuda and d_chars.dtype == torch.uint8 and d_chars.dim() == 1 and d_chars.is_contiguous()
+        assert d_offsets.is_cuda and d_offsets.dtype == torch.int64 and d_offsets.dim() == 1 and d_offsets.is_contiguous()
+        assert d_offsets.numel() >= 1, "a column of n texts has n + 1 offsets"
+        n_texts = d_offsets.numel() - 1
+        if d_ids is None:
+            d_ids = torch.empty(max(d_chars.numel(), 1), dtype=torch.int32, device=d_chars.device)
+        if d_id_offsets is None:
+            d_id_offsets = torch.empty(n_texts + 1, dtype=torch.int64, device=d_chars.device)
+        assert d_ids.is_cuda and d_ids.dtype == torch.int32 and d_ids.is_contiguous()
+        assert d_id_offsets.is_cuda and d_id_offsets.dtype == torch.int64 and d_id_offsets.is_contiguous()
+        assert d_id_offsets.numel() >= n_texts + 1
+        return n_texts, d_ids, d_id_offsets
+
+    def encode_batch_device(self, d_chars, d_offsets, d_ids=None, d_id_offsets=None, stream=None):
+        """Device string column -> (d_ids, d_id_offsets, n_ids).  ``wp_encode_batch_device``.
+
+        ``d_chars`` is a torch uint8 CUDA tensor, ``d_offsets`` an int64 CUDA tensor of n + 1 entries (Arrow
+        layout: text i is ``d_chars[d_offsets[i]:d_offsets[i + 1]]``, ``d_offsets[0]`` need not be 0).  The ids of
+        text i are ``d_ids[d_id_offsets[i]:d_id_offsets[i + 1]]`` (int64 CUDA tensor of n + 1 entries), each text
+        encoded exactly as ``encode`` would encode it alone.  ``d_ids`` may be a preallocated int32 tensor; otherwise
+        one id per char is allocated (always enough).  Synchronises the stream.
+        """
+        import torch
+
+        n_texts, d_ids, d_id_offsets = self._column(d_chars, d_offsets, d_ids, d_id_offsets)
+        if stream is None:
+            stream = torch.cuda.current_stream(d_chars.device).cuda_stream
+        cnt = C.c_size_t()
+        _check(self._L.wp_encode_batch_device(self._h, d_chars.data_ptr(), d_chars.numel(), d_offsets.data_ptr(), n_texts,
+                                              d_ids.data_ptr(), d_ids.numel(), d_id_offsets.data_ptr(), C.byref(cnt),
+                                              stream))
+        return d_ids, d_id_offsets, int(cnt.value)
+
+    def encode_batch_device_async(self, d_chars, d_offsets, d_ids, d_id_offsets, stream=None) -> None:
+        """Fully asynchronous variant of ``encode_batch_device``: the total lands in ``d_id_offsets[n]``, which
+        reads -1 (UINT64_MAX) if the ids are void or the column is malformed; then repeat the call through
+        ``encode_batch_device``.  ``wp_encode_batch_device_async``."""
+        import torch
+
+        n_texts, d_ids, d_id_offsets = self._column(d_chars, d_offsets, d_ids, d_id_offsets)
+        if stream is None:
+            stream = torch.cuda.current_stream(d_chars.device).cuda_stream
+        _check(self._L.wp_encode_batch_device_async(self._h, d_chars.data_ptr(), d_chars.numel(), d_offsets.data_ptr(),
+                                                    n_texts, d_ids.data_ptr(), d_ids.numel(), d_id_offsets.data_ptr(),
+                                                    stream))
 
     def set_kernel_timing(self, enabled: bool) -> None:
         _check(self._L.wp_set_kernel_timing(self._h, 1 if enabled else 0))

@@ -65,7 +65,8 @@ wp_status fail(wp_status st, const std::string &msg) {
 // WORDPIECE_B200_POISON=1 (tests): every device allocation of the library is filled with 0xCD bytes, so that a
 // kernel that reads scratch it has not written shows up in a fresh process as it would on recycled memory.
 // (value = bit mask of allocation classes: 1 scratch, 2 ids / text staging, 4 pipeline slot input, 8 batch output,
-// 16 tables, 32 call counters, 64 pipeline slot ids; "1" alone therefore poisons the scratch only, 127 everything)
+// 16 tables, 32 call counters, 64 pipeline slot ids, 128 device batch (packed column, its text index, check flag);
+// "1" alone therefore poisons the scratch only, 255 everything)
 template <class T>
 cudaError_t dev_alloc(T **p, size_t bytes, int cls = 127) {
   cudaError_t e = cudaMalloc(reinterpret_cast<void **>(p), bytes);
@@ -182,6 +183,16 @@ struct wp_vocab {
     Event h2d_done, cmp_done, d2h_done;
   } slot[3];
   Stream s_h2d, s_d2h;
+  // The device batch (wp_encode_batch_device): the column packed into whole tiles (16-byte aligned for K1's vector
+  // loads), the text starts, the tile index, K1's first segments, and the column check's flag (a word of its own:
+  // enqueue_encode clears the call counters after the check has run).  Never shared with the pipeline's slots,
+  // whose input the host pipeline writes without waiting for the handle's previous call.
+  DeviceBuffer<uint8_t> d_col_text{128};
+  DeviceBuffer<unsigned long long> d_col_bounds{128};
+  DeviceBuffer<uint32_t> d_col_tile_bound{128};
+  DeviceBuffer<uint32_t> d_col_bound_seg{128};
+  DeviceBuffer<unsigned int> d_col_bad{128};
+  PinnedBuffer<unsigned int> h_col_bad;
   // every call on a handle shares its scratch, counters and word table: the kernels of one call must have
   // finished before those of the next begin, on whatever streams the caller enqueues them
   Event last_done;
@@ -299,9 +310,10 @@ Workspace plan_workspace(size_t range_bytes, size_t spill_ids) {
   return w;
 }
 
-// A batch of texts packed into one buffer (wp_encode_batch): see EncodeParams::bounds.
+// A batch of texts packed into one buffer (wp_encode_batch, wp_encode_batch_device): see EncodeParams::bounds.
 struct BatchArgs {
-  const unsigned long long *h_bounds = nullptr;  // host copy of the text starts (ascending), n_texts entries
+  const unsigned long long *h_bounds = nullptr;  // host copy of the text starts (ascending), n_texts entries; null:
+                                                 // K5 reads the texts of a range from d_tile_bound on the device
   size_t n_texts = 0;
   const unsigned long long *d_bounds = nullptr;
   const uint32_t *d_tile_bound = nullptr;
@@ -395,6 +407,7 @@ wp_status enqueue_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_
   // batch calls: the texts [i0, i1) that start in the range whose K3 was just enqueued get their id offsets
   auto text_offsets = [&]() -> cudaError_t {
     if (!batch) return cudaSuccess;
+    if (!batch->h_bounds) return wp::launch_text_offsets_device(P, v->sm_count, stream, &launches);
     const unsigned long long lo = static_cast<unsigned long long>(P.first_tile) * tile;
     const unsigned long long hi = lo + static_cast<unsigned long long>(P.n_tiles) * tile;
     const unsigned long long *b = batch->h_bounds, *e = b + batch->n_texts;
@@ -513,6 +526,61 @@ wp_status run_encode(wp_vocab *v, const void *d_text, size_t n_bytes, int32_t *d
     WP_CUDA(cudaMemcpyAsync(v->h_call.p, v->d_call.p, sizeof(wp::CallCounters), cudaMemcpyDeviceToHost, stream));
     return WP_OK;
   });
+}
+
+// ---- the device batch (wp_encode_batch_device): a string column in device memory, packed on the device as
+// wp_encode_batch packs host texts (pack_part), encoded in one call of the kernels
+
+// Check and pack the column into the handle's device batch buffers, on `stream` behind the handle's previous call
+// (which may still read them).  `packed` = n_chars + n_texts bytes, whole tiles of which are written.
+wp_status enqueue_column(wp_vocab *v, const void *d_chars, size_t n_chars, const uint64_t *d_offsets, size_t n_texts,
+                         size_t packed, cudaStream_t stream, uint64_t *launches) {
+  const size_t tile = wp::encode_tile_bytes();
+  const size_t n_tiles = (packed + tile - 1) / tile;
+  WP_CUDA(v->d_col_text.grow(n_tiles * tile));
+  WP_CUDA(v->d_col_bounds.grow(n_texts));
+  WP_CUDA(v->d_col_tile_bound.grow(n_tiles + 1));
+  WP_CUDA(v->d_col_bound_seg.grow(n_texts));
+  WP_CUDA(v->d_col_bad.grow(1));
+  if (!v->last_done) WP_CUDA(cudaEventCreateWithFlags(&v->last_done.h, cudaEventDisableTiming));
+  WP_CUDA(cudaStreamWaitEvent(stream, v->last_done, 0));
+  WP_CUDA(cudaMemsetAsync(v->d_col_bad.p, 0, sizeof(unsigned int), stream));
+  wp::ColumnArgs A{};
+  A.chars = static_cast<const uint8_t *>(d_chars);
+  A.n_chars = n_chars;
+  A.offsets = reinterpret_cast<const unsigned long long *>(d_offsets);
+  A.n_texts = static_cast<uint32_t>(n_texts);
+  A.n_tiles = static_cast<uint32_t>(n_tiles);
+  A.bad = v->d_col_bad.p;
+  A.text = v->d_col_text.p;
+  A.bounds = v->d_col_bounds.p;
+  A.tile_bound = v->d_col_tile_bound.p;
+  uint64_t n = 0;
+  WP_CUDA(wp::launch_column_pack(A, stream, &n));
+  g_launches.fetch_add(n, std::memory_order_relaxed);
+  *launches += n;
+  return WP_OK;
+}
+
+// The kernels over the packed column (enqueue_column) into d_ids, K5 writing d_id_offsets[0, n_texts), then
+// d_id_offsets[n_texts] <- the id count, or UINT64_MAX if the call's ids are void or the column is malformed.
+wp_status enqueue_column_encode(wp_vocab *v, size_t packed, size_t n_texts, int32_t *d_ids, size_t capacity,
+                                uint64_t *d_id_offsets, cudaStream_t stream, size_t spill, EnqueueInfo *info) {
+  BatchArgs batch;  // (no h_bounds: K5 takes the texts of every range from the tile index)
+  batch.n_texts = n_texts;
+  batch.d_bounds = v->d_col_bounds.p;
+  batch.d_tile_bound = v->d_col_tile_bound.p;
+  batch.d_bound_seg = v->d_col_bound_seg.p;
+  batch.d_offsets = reinterpret_cast<unsigned long long *>(d_id_offsets);
+  const wp_status st = enqueue_encode(v, v->d_col_text.p, packed, d_ids, capacity, stream, spill, info, false, 0, &batch);
+  if (st != WP_OK) return st;
+  uint64_t launches = 0;
+  WP_CUDA(wp::launch_publish_count(v->d_call.p, info->n_ranges & 1u, batch.d_offsets + n_texts, stream, &launches,
+                                   v->d_col_bad.p));
+  WP_CUDA(cudaEventRecord(v->last_done, stream));  // (the count reads the counters and the flag the next call clears)
+  g_launches.fetch_add(launches, std::memory_order_relaxed);
+  info->launches += launches;
+  return WP_OK;
 }
 
 // Host text -> ids in the handle's device buffer v->d_ids (count in v->stats.n_ids), through the staging buffer
@@ -1380,6 +1448,74 @@ wp_status wp_encode_batch(wp_vocab *v, const char *const *texts, const size_t *l
   }
   trace("wp_encode_batch: ids on the host");
   offsets[n_texts] = *n_ids;
+  return *n_ids > capacity ? fail(WP_ERR_CAPACITY, "id buffer too small") : WP_OK;
+}
+
+// Host-side checks shared by both device batch entry points; *packed <- n_chars + n_texts
+static wp_status check_batch_device(wp_vocab *v, const void *d_chars, size_t n_chars, const uint64_t *d_offsets,
+                                    size_t n_texts, int32_t *d_ids, size_t capacity, uint64_t *d_id_offsets,
+                                    size_t *packed) {
+  if (!v || !d_offsets || !d_id_offsets || (n_chars > 0 && !d_chars) || (capacity > 0 && !d_ids))
+    return fail(WP_ERR_INVALID_ARG, "null argument");
+  if (v->device < 0) return fail(WP_ERR_NO_DEVICE, kHostOnly);
+  if (n_texts >= (size_t(1) << 31)) return fail(WP_ERR_INVALID_ARG, "too many texts in one batch (>= 2^31)");
+  *packed = n_chars + n_texts;
+  if (*packed < n_chars || *packed / wp::encode_tile_bytes() >= 0x7FFFFFFFull)
+    return fail(WP_ERR_INVALID_ARG, "batch too large for one call (> 2^31 tiles)");
+  return WP_OK;
+}
+
+wp_status wp_encode_batch_device_async(wp_vocab *v, const void *d_chars, size_t n_chars, const uint64_t *d_offsets,
+                                       size_t n_texts, int32_t *d_ids, size_t capacity, uint64_t *d_id_offsets,
+                                       void *stream) {
+  size_t packed = 0;
+  wp_status st = check_batch_device(v, d_chars, n_chars, d_offsets, n_texts, d_ids, capacity, d_id_offsets, &packed);
+  if (st != WP_OK) return st;
+  DeviceGuard g(v->device);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);  // NULL = the default stream, as everywhere in CUDA
+  if (n_texts == 0) {
+    WP_CUDA(cudaMemsetAsync(d_id_offsets, 0, sizeof(uint64_t), s));
+    return WP_OK;
+  }
+  uint64_t launches = 0;
+  st = enqueue_column(v, d_chars, n_chars, d_offsets, n_texts, packed, s, &launches);
+  if (st != WP_OK) return st;
+  EnqueueInfo info;
+  return enqueue_column_encode(v, packed, n_texts, d_ids, capacity, d_id_offsets, s, 0, &info);
+}
+
+wp_status wp_encode_batch_device(wp_vocab *v, const void *d_chars, size_t n_chars, const uint64_t *d_offsets,
+                                 size_t n_texts, int32_t *d_ids, size_t capacity, uint64_t *d_id_offsets, size_t *n_ids,
+                                 void *stream) {
+  if (!n_ids) return fail(WP_ERR_INVALID_ARG, "null argument");
+  *n_ids = 0;
+  size_t packed = 0;
+  wp_status st = check_batch_device(v, d_chars, n_chars, d_offsets, n_texts, d_ids, capacity, d_id_offsets, &packed);
+  if (st != WP_OK) return st;
+  DeviceGuard g(v->device);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (n_texts == 0) {
+    v->stats = wp_stats{};
+    WP_CUDA(cudaMemsetAsync(d_id_offsets, 0, sizeof(uint64_t), s));
+    WP_CUDA(cudaStreamSynchronize(s));
+    return WP_OK;
+  }
+  WP_CUDA(v->h_col_bad.grow(1));
+  uint64_t launches = 0;  // (the check and the packer count with the first attempt: a repeat packs nothing again)
+  st = enqueue_column(v, d_chars, n_chars, d_offsets, n_texts, packed, s, &launches);
+  if (st != WP_OK) return st;
+  st = repeat_call(v, s, packed, 0, *v->h_call.p, [&](size_t sp, EnqueueInfo *info) -> wp_status {
+    const wp_status est = enqueue_column_encode(v, packed, n_texts, d_ids, capacity, d_id_offsets, s, sp, info);
+    if (est != WP_OK) return est;
+    info->launches += std::exchange(launches, 0);
+    WP_CUDA(cudaMemcpyAsync(v->h_call.p, v->d_call.p, sizeof(wp::CallCounters), cudaMemcpyDeviceToHost, s));
+    WP_CUDA(cudaMemcpyAsync(v->h_col_bad.p, v->d_col_bad.p, sizeof(unsigned int), cudaMemcpyDeviceToHost, s));
+    return WP_OK;
+  });
+  if (st != WP_OK) return st;
+  if (*v->h_col_bad.p)
+    return fail(WP_ERR_INVALID_ARG, "malformed column: the offsets must ascend and end at most at n_chars");
+  *n_ids = static_cast<size_t>(v->stats.n_ids);
   return *n_ids > capacity ? fail(WP_ERR_CAPACITY, "id buffer too small") : WP_OK;
 }
 

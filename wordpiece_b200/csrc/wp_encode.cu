@@ -2029,9 +2029,11 @@ __global__ void __launch_bounds__(SCATTER_THREADS, WP_K3_BLOCKS) wp_scatter_kern
 
 // ======================================================= K5: text id offsets
 //
-// Batch calls (wp_encode_batch): where do the ids of every text begin?  K1 has numbered the first segment of
-// every text (bound_seg); the ids before segment s are the inclusive prefix K3 left in block_state for the
-// block before s's, plus the id counts of the segments of s's block that lie before s.  One warp per text.
+// Batch calls (wp_encode_batch, wp_encode_batch_device): where do the ids of every text begin?  K1 has numbered
+// the first segment of every text (bound_seg); the ids before segment s are the inclusive prefix K3 left in
+// block_state for the block before s's, plus the id counts of the segments of s's block that lie before s.  One
+// warp per text.  The texts [i0, i1) that start in the range come from the host (a grid that covers them), or,
+// `from_tiles`, from the tile index on the device (a fixed grid that strides over them).
 __device__ __forceinline__ uint32_t seg_id_count(const EncodeParams &P, uint32_t res) {
   if (res < SEG_RESULT_WORD) return 1u;
   uint32_t c = (res >> SEG_SLOW_INDEX_BITS) & ((res & SEG_RESULT_SLOW) ? SEG_SLOW_COUNT_MAX : 0xFu);
@@ -2044,29 +2046,208 @@ __device__ __forceinline__ uint32_t seg_id_count(const EncodeParams &P, uint32_t
 
 constexpr int OFFSET_THREADS = 128;
 
-__global__ void __launch_bounds__(OFFSET_THREADS) wp_text_offsets_kernel(EncodeParams P, uint32_t i0, uint32_t i1) {
+__global__ void __launch_bounds__(OFFSET_THREADS) wp_text_offsets_kernel(EncodeParams P, uint32_t i0, uint32_t i1,
+                                                                         uint32_t from_tiles) {
   const int lane = threadIdx.x & 31;
-  const uint32_t i = i0 + blockIdx.x * (OFFSET_THREADS / 32) + (threadIdx.x >> 5);
-  if (i >= i1 || P.call->overflow) return;
+  if (from_tiles) {
+    i0 = P.tile_bound[P.first_tile];
+    i1 = P.tile_bound[P.first_tile + P.n_tiles];
+  }
+  if (P.call->overflow) return;
   const unsigned long long n_segs = min(P.counters->n_segs, static_cast<unsigned long long>(P.seg_capacity));
-  const unsigned long long s = min(static_cast<unsigned long long>(P.bound_seg[i]), n_segs);
-  const uint32_t blk = static_cast<uint32_t>(s / SCATTER_SEGS);
-  const unsigned long long first = static_cast<unsigned long long>(blk) * SCATTER_SEGS;
-  unsigned long long sum = 0;
-  for (unsigned long long k = first + lane; k < s; k += 32) sum += seg_id_count(P, P.seg_result[k]);
+  const uint32_t warps = gridDim.x * (OFFSET_THREADS / 32);
+#pragma unroll 1
+  for (uint32_t i = i0 + blockIdx.x * (OFFSET_THREADS / 32) + (threadIdx.x >> 5); i < i1; i += warps) {
+    const unsigned long long s = min(static_cast<unsigned long long>(P.bound_seg[i]), n_segs);
+    const uint32_t blk = static_cast<uint32_t>(s / SCATTER_SEGS);
+    const unsigned long long first = static_cast<unsigned long long>(blk) * SCATTER_SEGS;
+    unsigned long long sum = 0;
+    for (unsigned long long k = first + lane; k < s; k += 32) sum += seg_id_count(P, P.seg_result[k]);
 #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(FULL, sum, o);
-  if (lane == 0) {
-    const unsigned long long before = blk ? (P.block_state[blk - 1] & ((1ull << 62) - 1)) : 0ull;
-    P.id_offsets[i] = P.call->ids_total[P.range_parity] + before + sum;  // ([parity] still holds the range's first id)
+    for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(FULL, sum, o);
+    if (lane == 0) {
+      const unsigned long long before = blk ? (P.block_state[blk - 1] & ((1ull << 62) - 1)) : 0ull;
+      P.id_offsets[i] = P.call->ids_total[P.range_parity] + before + sum;  // ([parity] still holds the range's first id)
+    }
   }
 }
 
 cudaError_t launch_text_offsets(const EncodeParams &P, uint32_t i0, uint32_t i1, cudaStream_t stream, uint64_t *launches) {
   if (i1 <= i0) return cudaSuccess;
   const uint32_t per = OFFSET_THREADS / 32;
-  wp_text_offsets_kernel<<<(i1 - i0 + per - 1) / per, OFFSET_THREADS, 0, stream>>>(P, i0, i1);
+  wp_text_offsets_kernel<<<(i1 - i0 + per - 1) / per, OFFSET_THREADS, 0, stream>>>(P, i0, i1, 0u);
   if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_text_offsets_device(const EncodeParams &P, int sm_count, cudaStream_t stream, uint64_t *launches) {
+  if (sm_count <= 0) sm_count = 148;
+  // (the host does not know how many texts start in the range: 16 x 4 warps per SM stride over them)
+  wp_text_offsets_kernel<<<sm_count * 16, OFFSET_THREADS, 0, stream>>>(P, 0u, 0u, 1u);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
+// ================================================= device string column -> packed text (wp_encode_batch_device)
+//
+// A column (Arrow layout: text i = chars[offsets[i] .. offsets[i + 1])) is packed as wp_encode_batch packs host
+// texts: text i at start(i) = offsets[i] - offsets[0] + i, followed by one space; the tail up to the packed length
+// n_chars + n_texts is spaces.  The source byte of a text byte at packed position p is p + offsets[0] - j, j its
+// text: the copy shifts by one at every separator.  Check first, then pack: a column whose offsets do not ascend
+// within [0, n_chars] sets *bad, and the packer then lays out n_texts empty texts (all spaces, start(i) = i) and
+// reads no char, so the kernels that follow index nothing out of range.
+
+constexpr int COLUMN_THREADS = 256;  // packer: 16 bytes of one tile per thread
+
+__global__ void __launch_bounds__(COLUMN_THREADS) wp_column_check_kernel(ColumnArgs A) {
+  const unsigned long long i = static_cast<unsigned long long>(blockIdx.x) * COLUMN_THREADS + threadIdx.x;
+  if (i >= A.n_texts) return;
+  const unsigned long long a = A.offsets[i], b = A.offsets[i + 1];
+  if (a > b || b > A.n_chars) *A.bad = 1u;
+}
+
+struct ColumnSmem {
+  uint4 src[TILE / 16 + 2];   // the tile's source chars, from the 16-byte unit that holds the first one
+  uint32_t sep[TILE / 32];    // bit p: packed position ts + p is a separator
+  uint32_t scan[TILE / 32];   // separators in the words before
+  uint32_t warp_sum[4];
+  uint32_t found[2];          // the first text that starts at or after ts (te)
+};
+
+__global__ void __launch_bounds__(COLUMN_THREADS) wp_column_pack_kernel(ColumnArgs A) {
+  __shared__ ColumnSmem sm;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const uint32_t t = blockIdx.x, n = A.n_texts;
+  const bool bad = *A.bad != 0u;
+  const unsigned long long off0 = bad ? 0ull : A.offsets[0];
+  // start(j) for j in [0, n]; start(n) = the end of the last separator
+  auto start = [&](uint32_t j) -> unsigned long long {
+    WP_CHECK(j <= n);
+    return bad ? static_cast<unsigned long long>(j) : A.offsets[j] - off0 + j;
+  };
+  const unsigned long long ts = static_cast<unsigned long long>(t) * TILE, te = ts + TILE;
+  if (tid < TILE / 32) sm.sep[tid] = 0u;
+  if (warp < 2) {
+    // the first j in [0, n) with start(j) >= x (n if none): a 32-way search, warp 0 for ts, warp 1 for te
+    const unsigned long long x = warp ? te : ts;
+    uint32_t lo = 0, hi = n;
+    while (hi > lo) {
+      const uint32_t span = hi - lo;
+      const uint32_t p = lo + static_cast<uint32_t>(static_cast<unsigned long long>(span) * lane / 32);
+      const uint32_t ge = __ballot_sync(FULL, start(p) >= x);
+      const int k = ge ? __ffs(ge) - 1 : 32;  // lanes probe ascending positions: the first lane at or past x
+      const uint32_t nhi = k < 32 ? lo + static_cast<uint32_t>(static_cast<unsigned long long>(span) * k / 32) : hi;
+      lo = k > 0 ? lo + static_cast<uint32_t>(static_cast<unsigned long long>(span) * (k - 1) / 32) + 1 : lo;
+      hi = nhi;
+    }
+    if (lane == 0) sm.found[warp] = lo;
+  }
+  __syncthreads();
+  const uint32_t a = sm.found[0], b = sm.found[1];
+  WP_CHECK(a <= b && b <= n);
+  const unsigned long long end = start(n);
+  const uint32_t j0 = (a > 0 && start(a) > ts) ? a - 1 : a;  // the text that holds position ts (n: the tail)
+  // text starts and the tile index
+  for (uint32_t i = a + tid; i < b; i += COLUMN_THREADS) {
+    WP_CHECK(i < n);
+    A.bounds[i] = start(i);
+  }
+  if (tid == 0) {
+    WP_CHECK(t < A.n_tiles);
+    A.tile_bound[t] = a;
+    if (t + 1 == A.n_tiles) A.tile_bound[t + 1] = b;  // (= n: every text starts before the packed length)
+  }
+  // separators in the tile: those of the texts [j0, b)
+  const uint32_t j_end = b < n ? b : n;
+  for (uint32_t j = j0 + tid; j < j_end; j += COLUMN_THREADS) {
+    const unsigned long long s = start(j + 1) - 1;
+    if (s >= ts && s < te) atomicOr(&sm.sep[(s - ts) >> 5], 1u << ((s - ts) & 31u));
+  }
+  __syncthreads();
+  if (warp < 4) {  // exclusive scan of the separator counts of the 128 words
+    const uint32_t c = __popc(sm.sep[tid]);
+    uint32_t inc = c;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const uint32_t y = __shfl_up_sync(FULL, inc, o);
+      if (lane >= o) inc += y;
+    }
+    sm.scan[tid] = inc - c;
+    if (lane == 31) sm.warp_sum[warp] = inc;
+  }
+  __syncthreads();
+  if (warp < 4) {
+    for (int w = 0; w < warp; w++) sm.scan[tid] += sm.warp_sum[w];
+  }
+  const uint32_t n_sep = sm.warp_sum[0] + sm.warp_sum[1] + sm.warp_sum[2] + sm.warp_sum[3];
+  // the source chars of the tile: [src_lo, src_lo + count), count = the positions before the tail that are no
+  // separator (every separator of the tile lies before the tail)
+  const unsigned long long tail = end > ts ? end - ts : 0ull;  // local position where the tail begins
+  const unsigned long long lim = tail < static_cast<unsigned long long>(TILE) ? tail : static_cast<unsigned long long>(TILE);
+  unsigned long long src_lo = j0 < n ? ts + off0 - j0 : 0ull;
+  unsigned long long src_hi = j0 < n && lim > n_sep ? src_lo + (lim - n_sep) : src_lo;
+  if (src_hi > A.n_chars) src_hi = A.n_chars;  // (clamps: only a malformed column, which reads nothing, could exceed)
+  if (src_lo > src_hi) src_lo = src_hi;
+  const uintptr_t lo_addr = reinterpret_cast<uintptr_t>(A.chars) + src_lo;
+  const uintptr_t hi_addr = reinterpret_cast<uintptr_t>(A.chars) + src_hi;
+  const uintptr_t base = lo_addr & ~uintptr_t(15);
+  const uint32_t lead = static_cast<uint32_t>(lo_addr - base);
+  __syncthreads();
+  {
+    const uint32_t units = static_cast<uint32_t>((hi_addr - base + 15) / 16);
+    WP_CHECK(units <= TILE / 16 + 2);
+    for (uint32_t u = tid; u < units; u += COLUMN_THREADS) {
+      const uintptr_t at = base + 16u * u;
+      if (at >= lo_addr && at + 16 <= hi_addr) {
+        sm.src[u] = ldg_stream(reinterpret_cast<const uint4 *>(at));
+      } else {  // a unit the column only partly covers: its bytes in [src_lo, src_hi) one by one
+        uint8_t *d = reinterpret_cast<uint8_t *>(&sm.src[u]);
+        for (int k = 0; k < 16; k++)
+          if (at + k >= lo_addr && at + k < hi_addr) d[k] = *reinterpret_cast<const uint8_t *>(at + k);
+      }
+    }
+  }
+  __syncthreads();
+  // 16 packed bytes per thread, one 16-byte store
+  const uint32_t lp0 = 16u * tid;
+  const uint32_t bits = (sm.sep[tid >> 1] >> (16u * (tid & 1))) & 0xFFFFu;
+  uint32_t before = sm.scan[tid >> 1] + ((tid & 1) ? __popc(sm.sep[tid >> 1] & 0xFFFFu) : 0u);
+  const uint8_t *src = reinterpret_cast<const uint8_t *>(sm.src);
+  uint32_t out[4];
+  if (bits == 0 && lp0 + 16u <= lim) {  // text only: 16 consecutive source chars
+    const uint32_t q = lp0 - before + lead;
+    WP_CHECK(q + 16u <= 16u * (TILE / 16 + 2));
+    const uint32_t *w = reinterpret_cast<const uint32_t *>(sm.src) + (q >> 2);
+    const uint32_t sh = 8u * (q & 3u);
+#pragma unroll
+    for (int k = 0; k < 4; k++) out[k] = sh ? __funnelshift_r(w[k], w[k + 1], sh) : w[k];
+  } else {
+#pragma unroll
+    for (int k = 0; k < 4; k++) out[k] = 0u;
+#pragma unroll
+    for (int k = 0; k < 16; k++) {
+      const uint32_t lp = lp0 + k;
+      uint32_t c = 0x20u;
+      if ((bits >> k) & 1u) {
+        before++;
+      } else if (lp < lim) {
+        const uint32_t q = lp - before + lead;
+        WP_CHECK(q < 16u * (TILE / 16 + 2) && base + q < hi_addr);
+        c = src[q];
+      }
+      out[k >> 2] |= c << (8 * (k & 3));
+    }
+  }
+  *reinterpret_cast<uint4 *>(A.text + ts + lp0) = make_uint4(out[0], out[1], out[2], out[3]);
+}
+
+cudaError_t launch_column_pack(const ColumnArgs &A, cudaStream_t stream, uint64_t *launches) {
+  wp_column_check_kernel<<<static_cast<unsigned>((A.n_texts + COLUMN_THREADS - 1) / COLUMN_THREADS), COLUMN_THREADS, 0,
+                           stream>>>(A);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return e;
+  wp_column_pack_kernel<<<A.n_tiles, COLUMN_THREADS, 0, stream>>>(A);
+  if (launches) *launches += 2;
   return cudaGetLastError();
 }
 
@@ -2221,13 +2402,14 @@ cudaError_t launch_seed_words(const WordSlot *image, uint32_t image_slots, WordS
 // The count of an asynchronous call for its caller: UINT64_MAX if a scratch capacity was exceeded (the ids
 // are incomplete then and the caller must repeat the call through a synchronous entry, which retries with
 // more scratch), else the number of ids.
-__global__ void wp_publish_count_kernel(const CallCounters *call, uint32_t parity, unsigned long long *out) {
-  *out = call->overflow ? ~0ull : call->ids_total[parity];
+__global__ void wp_publish_count_kernel(const CallCounters *call, uint32_t parity, unsigned long long *out,
+                                        const unsigned int *invalid) {
+  *out = (call->overflow || (invalid && *invalid)) ? ~0ull : call->ids_total[parity];
 }
 
 cudaError_t launch_publish_count(const CallCounters *call, uint32_t parity, unsigned long long *d_out, cudaStream_t stream,
-                                 uint64_t *launches) {
-  wp_publish_count_kernel<<<1, 1, 0, stream>>>(call, parity, d_out);
+                                 uint64_t *launches, const unsigned int *invalid) {
+  wp_publish_count_kernel<<<1, 1, 0, stream>>>(call, parity, d_out, invalid);
   if (launches) *launches += 1;
   return cudaGetLastError();
 }

@@ -141,13 +141,31 @@ struct EncodeParams {
 cudaError_t launch_seed_words(const WordSlot *image, uint32_t image_slots, WordSlot *work, uint32_t work_slots_log2,
                               cudaStream_t stream, uint64_t *launches);
 
-// *d_out <- the id count of the call whose counters are `call` (UINT64_MAX if its scratch overflowed).
+// *d_out <- the id count of the call whose counters are `call` (UINT64_MAX if its scratch overflowed, or if
+// `invalid` is given and *invalid is set).
 cudaError_t launch_publish_count(const CallCounters *call, uint32_t parity, unsigned long long *d_out, cudaStream_t stream,
-                                 uint64_t *launches);
+                                 uint64_t *launches, const unsigned int *invalid = nullptr);
 
 // K5 (batch calls): id_offsets[i] = index of the first id of text i, for the texts [i0, i1) that start in the
 // range whose K3 has just run on `stream` (same EncodeParams).
 cudaError_t launch_text_offsets(const EncodeParams &P, uint32_t i0, uint32_t i1, cudaStream_t stream, uint64_t *launches);
+// The same for the texts [tile_bound[first_tile], tile_bound[first_tile + n_tiles]), read on the device.
+cudaError_t launch_text_offsets_device(const EncodeParams &P, int sm_count, cudaStream_t stream, uint64_t *launches);
+
+// A string column in device memory (wp_encode_batch_device) and the packed text it becomes.
+struct ColumnArgs {
+  const uint8_t *chars;              // the column's chars, any alignment
+  unsigned long long n_chars;
+  const unsigned long long *offsets; // n_texts + 1 entries: text i = chars[offsets[i] .. offsets[i + 1])
+  uint32_t n_texts;
+  uint32_t n_tiles;                  // tiles of the packed text
+  unsigned int *bad;                 // zeroed; set by the check if the offsets do not ascend within [0, n_chars]
+  uint8_t *text;                     // n_tiles whole tiles, 16-byte aligned: the packed texts, then spaces
+  unsigned long long *bounds;        // n_texts: where text i starts in `text` (EncodeParams::bounds)
+  uint32_t *tile_bound;              // n_tiles + 1 (EncodeParams::tile_bound)
+};
+// The column check (one thread per text) and the packer (one CTA per tile of the packed text).
+cudaError_t launch_column_pack(const ColumnArgs &A, cudaStream_t stream, uint64_t *launches);
 
 uint32_t encode_tile_bytes();
 uint32_t scatter_block_segments();
