@@ -194,7 +194,7 @@ wp_status wp_encode_batch_device_async(wp_vocab *v, const void *d_chars, size_t 
                                        void *stream);
 
 /* Counters of the last completed encode call on the handle (every encode entry point sets them; for a pipelined
- * call they are summed over its parts). */
+ * call they are summed over its parts).  Decode calls (wp_decode, wp_decode_device[_async]) leave them as they are. */
 wp_status wp_last_stats(wp_vocab *v, wp_stats *out);
 
 /* Per-kernel device time (diagnostics for bench.py's roofline): when enabled, every following encode call
@@ -213,6 +213,31 @@ wp_status wp_last_kernel_ms(wp_vocab *v, float ms[3], uint32_t *n_ranges);
  * id == size is WP_ERR_ID_RANGE.  *n_skipped (optional) counts skipped ids. */
 wp_status wp_decode(const wp_vocab *v, const int32_t *ids, size_t n_ids, char **out, size_t **offsets_out,
                     size_t *n_tokens, size_t *n_skipped);
+
+/* Device ids -> device token strings (Arrow layout).  Entry i is the text fast::decode gives ids[i]
+ * ("##" re-added for continuation tokens), or EMPTY where the reference skips the id (id < 0, id > size,
+ * malformed token).  Entry i is d_chars[d_char_offsets[i] .. d_char_offsets[i + 1]); d_char_offsets has
+ * n_ids + 1 uint64 entries, d_char_offsets[0] = 0.  No kept token decodes to zero bytes, so an empty entry means
+ * exactly "skipped".  Because there is one entry per id, the d_id_offsets of wp_encode_batch_device index this
+ * column directly: text t's tokens are entries d_id_offsets[t] .. d_id_offsets[t + 1].
+ * Layout differs from wp_decode on purpose: wp_decode drops the skipped ids, this keeps one (empty) entry for
+ * each, so the column stays aligned with the ids; dropping the empty entries gives wp_decode's output exactly.
+ * The device decode table (every token's decoded bytes) is built and uploaded on a handle's first device decode
+ * call and freed with the handle; it is not counted in wp_vocab_device_bytes.  It uses 32-bit offsets: a
+ * vocabulary whose decoded tokens exceed 4 GiB in all gets WP_ERR_INVALID_ARG.
+ * Synchronises `stream` (NULL = the default stream).  WP_ERR_ID_RANGE if any id == size (as wp_decode).
+ * WP_ERR_CAPACITY if capacity < the bytes needed; then *n_chars holds that number and nothing is written
+ * (d_chars may be NULL with capacity 0: a size query).  *n_skipped (optional) counts the empty entries.
+ * Host-only handle: WP_ERR_NO_DEVICE.  n_ids == 0: d_char_offsets[0] = 0 and no kernel runs.
+ * Calls on one handle are ordered with its encode calls (they share its scratch), on whatever streams. */
+wp_status wp_decode_device(wp_vocab *v, const int32_t *d_ids, size_t n_ids, char *d_chars, size_t capacity,
+                           uint64_t *d_char_offsets, size_t *n_chars, size_t *n_skipped, void *stream);
+
+/* Fully asynchronous form, with the contract of wp_encode_device_async: d_char_offsets[n_ids] is the total byte
+ * count, or UINT64_MAX if an id == size or the capacity is short.  In the UINT64_MAX case nothing is written past
+ * `capacity` and the column is incomplete; repeat the call through wp_decode_device to get the status. */
+wp_status wp_decode_device_async(wp_vocab *v, const int32_t *d_ids, size_t n_ids, char *d_chars, size_t capacity,
+                                 uint64_t *d_char_offsets, void *stream);
 
 void wp_free(void *p);
 

@@ -1,6 +1,7 @@
 #!/usr/bin/env python3
 """Randomised parity sweep on a B200: hostile texts and vocabularies (tests/textgen.py) through randomly
-chosen entry points, range sizes and memo settings, every result compared with the CPU oracle.
+chosen entry points, range sizes and memo settings, every result compared with the CPU oracle (the device decode leg:
+random ids of the vocabulary, compared with the host wp_decode).
     python tools/fuzz_gpu.py [--seconds 120] [--seed0 1000]
 Prints one line per failure (with the seed to reproduce) and a summary; exit code 1 if anything differed."""
 from __future__ import annotations
@@ -60,7 +61,7 @@ def main():
             os.environ.pop("WORDPIECE_B200_PIPE_CHUNK", None)
         os.environ["WORDPIECE_B200_TICKET"] = "1" if rng.random() < 0.1 else "0"
         entry = rng.choice(["encode", "encode_into", "encode_into_pinned", "encode_device", "encode_text", "encode_batch",
-                            "encode_batch_device"])
+                            "encode_batch_device", "decode_device"])
         v = wordpiece_b200.Vocab(vocab, device=0)
         if rng.random() < 0.3:  # a handle that has already encoded something else (scratch, memo and shared memory in use)
             other, _ = textgen.case(seed + 77777, min(n, 200000), **kw)
@@ -94,6 +95,21 @@ def main():
                     got, offs = d_ids[:k].cpu().numpy(), d_offs.cpu().numpy()
                 exp_offs = np.concatenate([[0], np.cumsum([len(e) for e in exp_parts])])
                 assert np.array_equal(np.asarray(offs, dtype=np.int64), exp_offs.astype(np.int64)), "text offsets differ"
+            elif entry == "decode_device":
+                # random ids in [-3, size + 2] except size: the non-empty entries are wp_decode's tokens, and there are
+                # as many empty entries as ids wp_decode skips
+                size = len(v)
+                k = rng.choice([0, 1, 2047, 2049, rng.randrange(1, 100000)])
+                ids = np.array([rng.randrange(-3, size + 3) for _ in range(k)], np.int32)
+                ids[ids == size] = size + 1
+                d_ids = torch.from_numpy(ids).cuda() if k else torch.empty(0, dtype=torch.int32, device="cuda")
+                d_chars, d_offs, _, n_skipped = v.decode_device(d_ids)
+                chars, offs = d_chars.cpu().numpy().tobytes(), d_offs.cpu().numpy()
+                entries = [chars[int(offs[i]):int(offs[i + 1])] for i in range(k)]
+                host = v.decode(ids)
+                assert [e for e in entries if e] == host, "decoded tokens differ from wp_decode"
+                assert n_skipped == entries.count(b"") == k - len(host), "skipped ids differ from wp_decode"
+                got = exp
             elif entry == "encode":
                 got = v.encode(text)
             elif entry == "encode_into":

@@ -18,7 +18,9 @@ plus the persistent handle :class:`Vocab` (the reference rebuilds its hash maps
 on every call, fast.cpp:21-35; a handle builds the device table once), whose
 batch calls the reference lacks: ``Vocab.encode_batch`` (host texts) and
 ``Vocab.encode_batch_device[_async]`` (a string column in GPU memory: uint8
-chars + int64 Arrow offsets in, ids + per-text id offsets in GPU memory out).
+chars + int64 Arrow offsets in, ids + per-text id offsets in GPU memory out),
+and ``Vocab.decode_device[_async]`` (ids in GPU memory to one token string per
+id in the same column layout).
 
 There is no CPU fallback: if the shared library is missing or no CUDA device is
 usable, calls raise.

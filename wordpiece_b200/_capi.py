@@ -88,6 +88,8 @@ EXPORTED_SYMBOLS = [
     "wp_set_kernel_timing",
     "wp_last_kernel_ms",
     "wp_decode",
+    "wp_decode_device",
+    "wp_decode_device_async",
     "wp_free",
     "wp_debug_longest_match",
     "wp_debug_table_slots",
@@ -173,6 +175,11 @@ def load_library() -> C.CDLL:
     L.wp_last_kernel_ms.restype = C.c_int
     L.wp_decode.argtypes = [vp, vp, sz, C.POINTER(vp), C.POINTER(vp), C.POINTER(sz), C.POINTER(sz)]
     L.wp_decode.restype = C.c_int
+    if hasattr(L, "wp_decode_device"):  # (as wp_encode_batch: an older build may lack it)
+        L.wp_decode_device.argtypes = [vp, vp, sz, vp, sz, vp, C.POINTER(sz), C.POINTER(sz), vp]
+        L.wp_decode_device.restype = C.c_int
+        L.wp_decode_device_async.argtypes = [vp, vp, sz, vp, sz, vp, vp]
+        L.wp_decode_device_async.restype = C.c_int
     L.wp_free.argtypes = [vp]
     L.wp_free.restype = None
     L.wp_debug_longest_match.argtypes = [vp, C.c_char_p, sz, C.c_int, C.POINTER(C.c_uint32), C.POINTER(C.c_int32)]
@@ -522,6 +529,60 @@ class Vocab:
         self._L.wp_free(buf)
         self._L.wp_free(offs)
         return [raw[int(o[i]):int(o[i + 1])] for i in range(n.value)]
+
+    @staticmethod
+    def _decode_column(d_ids, d_chars, d_char_offsets):
+        import torch
+
+        assert d_ids.is_cuda and d_ids.dtype == torch.int32 and d_ids.dim() == 1 and d_ids.is_contiguous()
+        n_ids = d_ids.numel()
+        if d_char_offsets is None:
+            d_char_offsets = torch.empty(n_ids + 1, dtype=torch.int64, device=d_ids.device)
+        assert d_char_offsets.is_cuda and d_char_offsets.dtype == torch.int64 and d_char_offsets.is_contiguous()
+        assert d_char_offsets.numel() >= n_ids + 1, "n ids have n + 1 char offsets"
+        if d_chars is not None:
+            assert d_chars.is_cuda and d_chars.dtype == torch.uint8 and d_chars.dim() == 1 and d_chars.is_contiguous()
+        return n_ids, d_char_offsets
+
+    def decode_device(self, d_ids, d_chars=None, d_char_offsets=None, stream=None):
+        """Device ids (torch int32 CUDA tensor) -> (d_chars, d_char_offsets, n_chars, n_skipped).  ``wp_decode_device``.
+
+        Entry i, ``d_chars[d_char_offsets[i]:d_char_offsets[i + 1]]``, is what ``decode`` gives id i, or empty where
+        ``decode`` skips the id: one entry per id, so a batch's id offsets index the entries directly.  Dropping the
+        empty entries gives ``decode(ids)``.  ``d_chars`` may be a preallocated uint8 tensor (capacity = numel);
+        otherwise the call asks for the size first and allocates exactly ``n_chars``.  Synchronises the stream."""
+        import torch
+
+        n_ids, d_char_offsets = self._decode_column(d_ids, d_chars, d_char_offsets)
+        if stream is None:
+            stream = torch.cuda.current_stream(d_ids.device).cuda_stream
+        cnt, skipped = C.c_size_t(), C.c_size_t()
+
+        def call(chars):
+            return self._L.wp_decode_device(self._h, d_ids.data_ptr(), n_ids, chars.data_ptr() if chars is not None else None,
+                                            chars.numel() if chars is not None else 0, d_char_offsets.data_ptr(),
+                                            C.byref(cnt), C.byref(skipped), stream)
+
+        st = call(d_chars)
+        if d_chars is None:
+            if st == WP_ERR_CAPACITY or st == WP_OK:  # (the size query; with 0 bytes needed it was the whole call)
+                d_chars = torch.empty(cnt.value, dtype=torch.uint8, device=d_ids.device)
+                if st == WP_ERR_CAPACITY:
+                    st = call(d_chars)
+        _check(st)
+        return d_chars, d_char_offsets, int(cnt.value), int(skipped.value)
+
+    def decode_device_async(self, d_ids, d_chars, d_char_offsets, stream=None) -> None:
+        """Fully asynchronous variant of ``decode_device``: the total lands in ``d_char_offsets[n]``, which reads -1
+        (UINT64_MAX) if an id equals the vocabulary size or ``d_chars`` is too small; then repeat the call through
+        ``decode_device`` for the status.  ``wp_decode_device_async``."""
+        import torch
+
+        n_ids, d_char_offsets = self._decode_column(d_ids, d_chars, d_char_offsets)
+        if stream is None:
+            stream = torch.cuda.current_stream(d_ids.device).cuda_stream
+        _check(self._L.wp_decode_device_async(self._h, d_ids.data_ptr(), n_ids, d_chars.data_ptr(), d_chars.numel(),
+                                              d_char_offsets.data_ptr(), stream))
 
 
 # ---- the reference's stateless entry points ---------------------------------

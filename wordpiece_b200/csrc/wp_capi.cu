@@ -65,7 +65,7 @@ wp_status fail(wp_status st, const std::string &msg) {
 // WORDPIECE_B200_POISON=1 (tests): every device allocation of the library is filled with 0xCD bytes, so that a
 // kernel that reads scratch it has not written shows up in a fresh process as it would on recycled memory.
 // (value = bit mask of allocation classes: 1 scratch, 2 ids / text staging, 4 pipeline slot input, 8 batch output,
-// 16 tables, 32 call counters, 64 pipeline slot ids, 128 device batch (packed column, its text index, check flag);
+// 16 tables (the decode table too), 32 call counters, 64 pipeline slot ids, 128 device batch (packed column, its text index, check flag);
 // "1" alone therefore poisons the scratch only, 255 everything)
 template <class T>
 cudaError_t dev_alloc(T **p, size_t bytes, int cls = 127) {
@@ -193,6 +193,12 @@ struct wp_vocab {
   DeviceBuffer<uint32_t> d_col_bound_seg{128};
   DeviceBuffer<unsigned int> d_col_bad{128};
   PinnedBuffer<unsigned int> h_col_bad;
+  // The decode table (wp_decode_device): per id {offset, length | DECODE_SKIP} and the decoded bytes, built on
+  // the first device decode call so that a handle that only encodes pays nothing for it
+  DeviceBuffer<uint2> d_dec_desc{16};
+  DeviceBuffer<uint8_t> d_dec_bytes{16};
+  bool dec_ready = false;
+  PinnedBuffer<unsigned long long> h_dec;  // the length pass's totals, for the synchronous call
   // every call on a handle shares its scratch, counters and word table: the kernels of one call must have
   // finished before those of the next begin, on whatever streams the caller enqueues them
   Event last_done;
@@ -1179,6 +1185,81 @@ wp_status create_common(wp_vocab *v, const char *const *tokens, const size_t *le
   return WP_OK;
 }
 
+// ---- device decode (wp_decode_device): one entry per id, gathered from the decode table
+
+// The decode table with exactly wp_decode's rules: "##" + word for a continuation token, the word for any other,
+// a skip mark for a malformed one.  Built and uploaded on the handle's first device decode call.
+wp_status ensure_decode_table(wp_vocab *v) {
+  if (v->dec_ready) return WP_OK;
+  const std::vector<wp::HostToken> &toks = v->host.tokens;
+  size_t total = 0, longest = 0;
+  for (const wp::HostToken &t : toks) {
+    if (t.is_malformed) continue;
+    const size_t len = t.word.size() + (t.is_prefix ? 0 : 2);
+    total += len;
+    longest = std::max(longest, len);
+  }
+  if (total > 0xFFFFFFFFull || longest >= wp::DECODE_SKIP)  // (32-bit offsets, 31-bit lengths)
+    return fail(WP_ERR_INVALID_ARG, "vocabulary too large for device decode (its decoded tokens exceed 4 GiB)");
+  std::vector<uint2> desc(toks.size());
+  std::string bytes;
+  bytes.reserve(total);
+  for (size_t i = 0; i < toks.size(); i++) {
+    const wp::HostToken &t = toks[i];
+    desc[i].x = static_cast<uint32_t>(bytes.size());
+    if (t.is_malformed) {  // fast.cpp:176-177
+      desc[i].y = wp::DECODE_SKIP;
+      continue;
+    }
+    if (!t.is_prefix) bytes += "##";  // fast.cpp:180-183
+    bytes += t.word;
+    desc[i].y = static_cast<uint32_t>(bytes.size()) - desc[i].x;
+  }
+  WP_CUDA(v->d_dec_desc.grow(std::max<size_t>(desc.size(), 1)));
+  WP_CUDA(v->d_dec_bytes.grow(std::max<size_t>(bytes.size(), 1)));
+  if (!desc.empty())
+    WP_CUDA(cudaMemcpy(v->d_dec_desc.p, desc.data(), desc.size() * sizeof(uint2), cudaMemcpyHostToDevice));
+  if (!bytes.empty()) WP_CUDA(cudaMemcpy(v->d_dec_bytes.p, bytes.data(), bytes.size(), cudaMemcpyHostToDevice));
+  v->dec_ready = true;
+  return WP_OK;
+}
+
+// Host-side checks shared by both device decode entry points
+wp_status check_decode_device(const wp_vocab *v, const int32_t *d_ids, size_t n_ids, const char *d_chars,
+                              size_t capacity, const uint64_t *d_char_offsets) {
+  if (!v || !d_char_offsets || (n_ids > 0 && !d_ids) || (capacity > 0 && !d_chars))
+    return fail(WP_ERR_INVALID_ARG, "null argument");
+  if (v->device < 0) return fail(WP_ERR_NO_DEVICE, kHostOnly);
+  if (n_ids / wp::decode_block_ids() >= 0xFFFFFFFFull) return fail(WP_ERR_INVALID_ARG, "too many ids for one call");
+  return WP_OK;
+}
+
+// The length pass of a decode of n_ids > 0 ids on `stream`, behind the handle's previous call (the decode uses
+// the handle's scratch: its totals, ticket and look-back words, zeroed here).  *A <- the arguments of both passes.
+wp_status enqueue_decode_total(wp_vocab *v, const int32_t *d_ids, size_t n_ids, char *d_chars, size_t capacity,
+                               uint64_t *d_char_offsets, cudaStream_t stream, wp::DecodeArgs *A, uint64_t *launches) {
+  const wp_status st = ensure_decode_table(v);
+  if (st != WP_OK) return st;
+  const size_t n_blocks = (n_ids + wp::decode_block_ids() - 1) / wp::decode_block_ids();
+  const size_t need = (4 + n_blocks) * sizeof(unsigned long long);
+  WP_CUDA(v->d_work.grow(need));
+  if (!v->last_done) WP_CUDA(cudaEventCreateWithFlags(&v->last_done.h, cudaEventDisableTiming));
+  WP_CUDA(cudaStreamWaitEvent(stream, v->last_done, 0));
+  WP_CUDA(cudaMemsetAsync(v->d_work.p, 0, need, stream));
+  *A = wp::DecodeArgs{};
+  A->ids = d_ids;
+  A->n_ids = n_ids;
+  A->desc = v->d_dec_desc.p;
+  A->bytes = v->d_dec_bytes.p;
+  A->vocab_size = static_cast<uint32_t>(v->host.tokens.size());
+  A->out = d_chars;
+  A->capacity = capacity;
+  A->offsets = reinterpret_cast<unsigned long long *>(d_char_offsets);
+  A->work = reinterpret_cast<unsigned long long *>(v->d_work.p);
+  WP_CUDA(wp::launch_decode_total(*A, v->sm_count, stream, launches));
+  return WP_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1741,6 +1822,63 @@ wp_status wp_decode(const wp_vocab *v, const int32_t *ids, size_t n_ids, char **
   *offsets_out = ob;
   *n_tokens = offs.size() - 1;
   if (n_skipped) *n_skipped = skipped;
+  return WP_OK;
+}
+
+wp_status wp_decode_device_async(wp_vocab *v, const int32_t *d_ids, size_t n_ids, char *d_chars, size_t capacity,
+                                 uint64_t *d_char_offsets, void *stream) {
+  wp_status st = check_decode_device(v, d_ids, n_ids, d_chars, capacity, d_char_offsets);
+  if (st != WP_OK) return st;
+  DeviceGuard g(v->device);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);  // NULL = the default stream, as everywhere in CUDA
+  if (n_ids == 0) {
+    WP_CUDA(cudaMemsetAsync(d_char_offsets, 0, sizeof(uint64_t), s));
+    return WP_OK;
+  }
+  wp::DecodeArgs A;
+  uint64_t launches = 0;
+  st = enqueue_decode_total(v, d_ids, n_ids, d_chars, capacity, d_char_offsets, s, &A, &launches);
+  g_launches.fetch_add(std::exchange(launches, 0), std::memory_order_relaxed);
+  if (st != WP_OK) return st;
+  WP_CUDA(wp::launch_decode(A, v->sm_count, s, &launches));
+  g_launches.fetch_add(launches, std::memory_order_relaxed);
+  WP_CUDA(cudaEventRecord(v->last_done, s));  // the scratch is free once the scatter is done
+  return WP_OK;
+}
+
+wp_status wp_decode_device(wp_vocab *v, const int32_t *d_ids, size_t n_ids, char *d_chars, size_t capacity,
+                           uint64_t *d_char_offsets, size_t *n_chars, size_t *n_skipped, void *stream) {
+  if (!n_chars) return fail(WP_ERR_INVALID_ARG, "null argument");
+  *n_chars = 0;
+  if (n_skipped) *n_skipped = 0;
+  wp_status st = check_decode_device(v, d_ids, n_ids, d_chars, capacity, d_char_offsets);
+  if (st != WP_OK) return st;
+  DeviceGuard g(v->device);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (n_ids == 0) {
+    WP_CUDA(cudaMemsetAsync(d_char_offsets, 0, sizeof(uint64_t), s));
+    WP_CUDA(cudaStreamSynchronize(s));
+    return WP_OK;
+  }
+  WP_CUDA(v->h_dec.grow(3));
+  wp::DecodeArgs A;
+  uint64_t launches = 0;
+  st = enqueue_decode_total(v, d_ids, n_ids, d_chars, capacity, d_char_offsets, s, &A, &launches);
+  g_launches.fetch_add(std::exchange(launches, 0), std::memory_order_relaxed);
+  if (st != WP_OK) return st;
+  WP_CUDA(cudaMemcpyAsync(v->h_dec.p, v->d_work.p, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+  WP_CUDA(cudaEventRecord(v->last_done, s));
+  WP_CUDA(cudaStreamSynchronize(s));
+  const unsigned long long bytes = v->h_dec.p[0], skipped = v->h_dec.p[1], bad = v->h_dec.p[2];
+  if (bad) return fail(WP_ERR_ID_RANGE, "token id equals vocabulary size");  // fast.cpp:175 .at()
+  *n_chars = static_cast<size_t>(bytes);
+  if (n_skipped) *n_skipped = static_cast<size_t>(skipped);
+  if (bytes > capacity) return fail(WP_ERR_CAPACITY, "char buffer too small");
+  // (the scratch still holds the totals and zeroed look-back words: nothing ran on it since the length pass)
+  WP_CUDA(wp::launch_decode(A, v->sm_count, s, &launches));
+  g_launches.fetch_add(launches, std::memory_order_relaxed);
+  WP_CUDA(cudaEventRecord(v->last_done, s));
+  WP_CUDA(cudaStreamSynchronize(s));
   return WP_OK;
 }
 

@@ -533,22 +533,22 @@ __device__ __noinline__ void classify_window(TileSmem &sm, const uint8_t *buf, i
 }
 
 // block-wide exclusive scan of one value per thread; returns the exclusive prefix, *total = sum
-template <int NWARPS>
-__device__ __forceinline__ uint32_t block_exclusive_scan(uint32_t *warp_sums, uint32_t v, uint32_t *total) {
+template <int NWARPS, class T = uint32_t>
+__device__ __forceinline__ T block_exclusive_scan(T *warp_sums, T v, T *total) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  uint32_t incl = v;
+  T incl = v;
 #pragma unroll
   for (int o = 1; o < 32; o <<= 1) {
-    const uint32_t y = __shfl_up_sync(FULL, incl, o);
+    const T y = __shfl_up_sync(FULL, incl, o);
     if (lane >= o) incl += y;
   }
   __syncthreads();  // warp_sums may still be in use by an earlier scan
   if (lane == 31) warp_sums[warp] = incl;
   __syncthreads();
-  uint32_t wbase = 0, tot = 0;
+  T wbase = 0, tot = 0;
 #pragma unroll
   for (int wi = 0; wi < NWARPS; wi++) {
-    const uint32_t ws = warp_sums[wi];
+    const T ws = warp_sums[wi];
     if (wi < warp) wbase += ws;
     tot += ws;
   }
@@ -2369,6 +2369,181 @@ cudaError_t launch_format(const int32_t *ids, size_t n, char *out, unsigned long
 }
 
 uint32_t format_block_ids() { return FORMAT_IDS; }
+
+// ============================================================== decode
+//
+// ids -> one entry per id of the token text fast::decode gives it (fast.cpp:165-187), empty where the reference
+// skips the id.  The shape of K4: a length pass (total bytes, skipped ids, the id == size flag), then blocks by
+// ticket that scan their ids' lengths, publish the block total, write their offsets and copy their bytes.  The
+// bytes of one block go out through a shared-memory stage in WINDOWS of DECODE_STAGE bytes aligned to 16 bytes of
+// the output: for each window every id copies the part of its token that falls inside it, then the window is
+// stored with 16-byte stores (byte stores only at the two ends of the block's range, which neighbours share).
+// Any block output size takes the same path: a block of 2 048 tokens of 400 bytes is 50 windows.
+
+constexpr int DECODE_THREADS = 256;
+constexpr int DECODE_ITEMS = 8;
+constexpr int DECODE_IDS = DECODE_THREADS * DECODE_ITEMS;  // 2048 ids per block iteration
+constexpr int DECODE_STAGE = 16384;                        // bytes per window (= DECODE_IDS offsets of 8 bytes)
+constexpr int DECODE_BLOCKS = 4;                           // CTAs per SM (launch bound and grid)
+static_assert(DECODE_STAGE == DECODE_IDS * 8, "the stage holds the block's relative offsets before its bytes");
+
+// bytes of id's entry (0 if skipped); *bad |= id == size
+__device__ __forceinline__ uint2 decode_entry(const DecodeArgs &A, int32_t id, bool *bad) {
+  if (id < 0 || static_cast<uint32_t>(id) >= A.vocab_size) {
+    *bad |= static_cast<uint32_t>(id) == A.vocab_size;
+    return make_uint2(0u, 0u);
+  }
+  WP_CHECK(static_cast<uint32_t>(id) < A.vocab_size);
+  const uint2 d = A.desc[id];
+  return (d.y & DECODE_SKIP) ? make_uint2(0u, 0u) : d;
+}
+
+__global__ void __launch_bounds__(DECODE_THREADS) wp_decode_total_kernel(DecodeArgs A) {
+  __shared__ unsigned long long sums[2][DECODE_THREADS / 32];
+  unsigned long long bytes = 0, skipped = 0;
+  bool bad = false;
+  for (unsigned long long i = static_cast<unsigned long long>(blockIdx.x) * DECODE_THREADS + threadIdx.x; i < A.n_ids;
+       i += static_cast<unsigned long long>(gridDim.x) * DECODE_THREADS) {
+    const uint32_t len = decode_entry(A, A.ids[i], &bad).y;
+    bytes += len;
+    skipped += len == 0u;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    bytes += __shfl_xor_sync(FULL, bytes, o);
+    skipped += __shfl_xor_sync(FULL, skipped, o);
+  }
+  bad = __syncthreads_or(bad);
+  if ((threadIdx.x & 31) == 0) {
+    sums[0][threadIdx.x >> 5] = bytes;
+    sums[1][threadIdx.x >> 5] = skipped;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    unsigned long long b = 0, s = 0;
+    for (int w = 0; w < DECODE_THREADS / 32; w++) {
+      b += sums[0][w];
+      s += sums[1][w];
+    }
+    if (b) atomicAdd(&A.work[0], b);
+    if (s) atomicAdd(&A.work[1], s);
+    if (bad) atomicOr(&A.work[2], 1ull);
+  }
+}
+
+struct DecodeSmem {
+  __align__(16) uint8_t stage[DECODE_STAGE];
+  unsigned long long warp_sums[DECODE_THREADS / 32];
+  uint32_t block_index;
+  unsigned long long base;
+};
+
+__global__ void __launch_bounds__(DECODE_THREADS, DECODE_BLOCKS) wp_decode_kernel(DecodeArgs A) {
+  __shared__ DecodeSmem sm;
+  const int tid = threadIdx.x;
+  const int lane = tid & 31;
+  const unsigned long long n = A.n_ids;
+  // (an async call that needs more than capacity, or met an id == size, writes nothing but the void count)
+  if (A.work[2] != 0ull || A.work[0] > A.capacity) {
+    if (blockIdx.x == 0 && tid == 0) A.offsets[n] = ~0ull;
+    return;
+  }
+  unsigned long long *const block_state = A.work + 4;
+  unsigned int *const ticket = reinterpret_cast<unsigned int *>(A.work + 3);
+  unsigned long long *const rel = reinterpret_cast<unsigned long long *>(sm.stage);
+  const uint32_t n_blocks = static_cast<uint32_t>((n + DECODE_IDS - 1) / DECODE_IDS);
+  for (;;) {
+    __syncthreads();
+    if (tid == 0) sm.block_index = atomicAdd(ticket, 1u);
+    __syncthreads();
+    const uint32_t b = sm.block_index;
+    if (b >= n_blocks) break;
+    const unsigned long long block_first = static_cast<unsigned long long>(b) * DECODE_IDS;
+    const uint32_t count = static_cast<uint32_t>(n - block_first < DECODE_IDS ? n - block_first : DECODE_IDS);
+    const uint32_t first = tid * DECODE_ITEMS;  // within the block
+    uint2 e[DECODE_ITEMS];
+    unsigned long long mine = 0;
+    bool bad = false;
+#pragma unroll
+    for (int j = 0; j < DECODE_ITEMS; j++) {
+      e[j] = first + j < count ? decode_entry(A, A.ids[block_first + first + j], &bad) : make_uint2(0u, 0u);
+      mine += e[j].y;
+    }
+    unsigned long long total;
+    unsigned long long at = block_exclusive_scan<DECODE_THREADS / 32>(sm.warp_sums, mine, &total);
+    if (tid == 0) lookback_publish(A.work + 4, b, total);
+#pragma unroll
+    for (int j = 0; j < DECODE_ITEMS; j++) {
+      if (first + j < count) {
+        WP_CHECK(first + j < DECODE_IDS);
+        rel[first + j] = at;
+      }
+      at += e[j].y;
+    }
+    __syncthreads();
+    if (tid < 32) {
+      const unsigned long long base = lookback_walk(block_state, b, total, lane);
+      if (lane == 0) sm.base = base;
+    }
+    __syncthreads();
+    const unsigned long long base = sm.base;
+    for (uint32_t i = tid; i < count; i += DECODE_THREADS) {
+      WP_CHECK(block_first + i < n);
+      A.offsets[block_first + i] = base + rel[i];
+    }
+    if (block_first + count == n && tid == 0) A.offsets[n] = base + total;
+    // the block's bytes [base, base + total) of the output, in windows aligned to 16 bytes of the output address
+    WP_CHECK(base + total <= A.capacity);
+    const uintptr_t lo = reinterpret_cast<uintptr_t>(A.out) + base, hi = lo + total;
+    at -= mine;  // back to this thread's first entry
+    for (uintptr_t w = lo & ~static_cast<uintptr_t>(15); w < hi; w += DECODE_STAGE) {
+      __syncthreads();  // (the stage: the offsets above, or the previous window, have been stored)
+      const uintptr_t w_end = w + DECODE_STAGE < hi ? w + DECODE_STAGE : hi;
+      unsigned long long s = at;
+#pragma unroll
+      for (int j = 0; j < DECODE_ITEMS; j++) {
+        const uintptr_t t0 = lo + s, t1 = t0 + e[j].y;
+        const uintptr_t c0 = t0 > w ? t0 : w, c1 = t1 < w_end ? t1 : w_end;
+        const uint8_t *src = A.bytes + e[j].x + (c0 - t0);
+#pragma unroll 4
+        for (uintptr_t c = c0; c < c1; c++, src++) {
+          WP_CHECK(c - w < DECODE_STAGE && src < A.bytes + e[j].x + e[j].y);
+          sm.stage[c - w] = *src;
+        }
+        s += e[j].y;
+      }
+      __syncthreads();
+      for (uintptr_t u = w + 16u * tid; u < w_end; u += 16u * DECODE_THREADS) {
+        WP_CHECK(u - w + 16u <= DECODE_STAGE);
+        if (u >= lo && u + 16u <= hi) {
+          *reinterpret_cast<uint4 *>(u) = *reinterpret_cast<const uint4 *>(sm.stage + (u - w));
+        } else {
+          for (uintptr_t k = u; k < u + 16u; k++)
+            if (k >= lo && k < hi) {
+              WP_CHECK(k - reinterpret_cast<uintptr_t>(A.out) < A.capacity);
+              *reinterpret_cast<uint8_t *>(k) = sm.stage[k - w];
+            }
+        }
+      }
+    }
+  }
+}
+
+uint32_t decode_block_ids() { return DECODE_IDS; }
+
+cudaError_t launch_decode_total(const DecodeArgs &A, int sm_count, cudaStream_t stream, uint64_t *launches) {
+  if (sm_count <= 0) sm_count = 148;
+  wp_decode_total_kernel<<<sm_count * 8, DECODE_THREADS, 0, stream>>>(A);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_decode(const DecodeArgs &A, int sm_count, cudaStream_t stream, uint64_t *launches) {
+  if (sm_count <= 0) sm_count = 148;
+  wp_decode_kernel<<<sm_count * DECODE_BLOCKS, DECODE_THREADS, 0, stream>>>(A);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
 
 // ------------------------------------------------------------ word-table seed
 // Every encode call that records words starts from a working table that holds exactly the static words.

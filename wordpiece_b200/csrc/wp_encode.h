@@ -186,4 +186,27 @@ cudaError_t launch_format_total(const int32_t *ids, size_t n, unsigned long long
 cudaError_t launch_format(const int32_t *ids, size_t n, char *out, unsigned long long *block_state, unsigned int *ticket,
                           int sm_count, cudaStream_t stream, uint64_t *launches);
 
+// Device decode (wp_decode_device): ids -> one entry per id of the token's decoded bytes (empty if skipped).
+// The decode table: desc[id] = {offset into bytes, length | DECODE_SKIP}; built on the host (wp_capi.cu).
+constexpr uint32_t DECODE_SKIP = 0x80000000u;  // malformed token: the reference skips the id (fast.cpp:176-177)
+struct DecodeArgs {
+  const int32_t *ids;
+  unsigned long long n_ids;
+  const uint2 *desc;                   // vocabulary size entries
+  const uint8_t *bytes;                // every kept token's bytes ("##" + word for continuation tokens), concatenated
+  uint32_t vocab_size;
+  char *out;                           // capacity bytes
+  unsigned long long capacity;
+  unsigned long long *offsets;         // n_ids + 1 entries
+  // scratch (zeroed): [0] total bytes, [1] skipped ids, [2] an id == size was seen, [3] ticket, [4 ...] one
+  // look-back word per decode_block_ids() ids
+  unsigned long long *work;
+};
+uint32_t decode_block_ids();
+// Adds the output bytes and the skipped ids to work[0], work[1], and sets work[2] if an id equals the size.
+cudaError_t launch_decode_total(const DecodeArgs &A, int sm_count, cudaStream_t stream, uint64_t *launches);
+// Writes offsets[0 .. n_ids] and the bytes, or, if work[2] is set or work[0] > capacity, only offsets[n_ids] =
+// UINT64_MAX.
+cudaError_t launch_decode(const DecodeArgs &A, int sm_count, cudaStream_t stream, uint64_t *launches);
+
 }  // namespace wp
