@@ -194,7 +194,8 @@ wp_status wp_encode_batch_device_async(wp_vocab *v, const void *d_chars, size_t 
                                        void *stream);
 
 /* Counters of the last completed encode call on the handle (every encode entry point sets them; for a pipelined
- * call they are summed over its parts).  Decode calls (wp_decode, wp_decode_device[_async]) leave them as they are. */
+ * call they are summed over its parts).  Decode calls (wp_decode, wp_decode_device[_async]) and row calls
+ * (wp_rows_device[_async]) leave them as they are. */
 wp_status wp_last_stats(wp_vocab *v, wp_stats *out);
 
 /* Per-kernel device time (diagnostics for bench.py's roofline): when enabled, every following encode call
@@ -238,6 +239,50 @@ wp_status wp_decode_device(wp_vocab *v, const int32_t *d_ids, size_t n_ids, char
  * `capacity` and the column is incomplete; repeat the call through wp_decode_device to get the status. */
 wp_status wp_decode_device_async(wp_vocab *v, const int32_t *d_ids, size_t n_ids, char *d_chars, size_t capacity,
                                  uint64_t *d_char_offsets, void *stream);
+
+/* ---- model-input rows ---------------------------------------------------
+ * Per-text ids in device memory (e.g. the d_ids / d_id_offsets of wp_encode_batch_device) -> the fixed-length rows a
+ * BERT-family model takes, in device memory.  Each row is max_len (L) int32 ids:
+ *     [CLS]? content [SEP]? pad ... pad
+ * SEP follows the content directly (not the end of the row); the mask row is 1 on the CLS, content and SEP positions
+ * and 0 on the padding.  The content width is W = L - [CLS present] - [SEP present] and must be at least 1.
+ *   stride == 0       truncate: one row per text, holding its first min(n_t, W) ids.
+ *   1 <= stride <= W  overflow windows: a text of n_t ids has 1 row if n_t <= W, else 1 + ceil((n_t - W) / stride);
+ *                     row k holds the text's ids [k * stride, min(k * stride + W, n_t)), so the last row ends at n_t.
+ *                     `stride` is the distance between the STARTS of consecutive windows (cuDF subword_tokenize's
+ *                     meaning); HuggingFace's `stride` is the overlap, W - stride here.
+ * An empty text gives one row with no content.  Ids are copied verbatim, never interpreted (-1 stays -1). */
+#define WP_ROWS_CLS 1u
+#define WP_ROWS_SEP 2u
+typedef struct wp_rows_spec {
+  uint32_t max_len; /* L, special tokens included */
+  uint32_t stride;  /* 0: truncate; else window starts `stride` content ids apart, 1 <= stride <= W */
+  int32_t pad_id, cls_id, sep_id;
+  uint32_t flags;   /* WP_ROWS_CLS | WP_ROWS_SEP: which of cls_id / sep_id the rows carry */
+} wp_rows_spec;
+
+/* Text t's ids are d_ids[d_id_offsets[t] .. d_id_offsets[t + 1]) (n_texts + 1 uint64 offsets that ascend and end at
+ * most at n_ids; d_id_offsets[0] need not be 0).  Writes n_texts + 1 uint64 d_row_offsets: text t's rows are rows
+ * d_row_offsets[t] .. d_row_offsets[t + 1] (d_row_offsets[0] = 0), which with the rule above describes every row.
+ * Rows are row-major: row r is d_rows[r * L .. (r + 1) * L), mask row r is d_mask[r * L .. (r + 1) * L).  d_rows
+ * holds row_capacity rows and may be any 4-byte-aligned pointer; d_mask (optional, NULL = no mask) holds as many
+ * rows of L bytes at any alignment.
+ * Synchronises `stream` (NULL = the default stream).  WP_ERR_INVALID_ARG for a null argument, a spec with W < 1, a
+ * stride > W or unknown flags, a misaligned d_rows, row_capacity * L * 4 overflowing, or id offsets that descend
+ * or end past n_ids (found on the device).  WP_ERR_CAPACITY if row_capacity < the rows needed: then *n_rows and
+ * d_row_offsets are still exact and nothing is written to d_rows / d_mask (d_rows may be NULL with row_capacity 0:
+ * a size query).  Host-only handle: WP_ERR_NO_DEVICE.  n_texts == 0: d_row_offsets[0] = 0, *n_rows = 0 and no
+ * kernel runs.  Calls on one handle are ordered with its encode and decode calls (they share its scratch). */
+wp_status wp_rows_device(wp_vocab *v, const int32_t *d_ids, size_t n_ids, const uint64_t *d_id_offsets, size_t n_texts,
+                         const wp_rows_spec *spec, int32_t *d_rows, uint8_t *d_mask, size_t row_capacity,
+                         uint64_t *d_row_offsets, size_t *n_rows, void *stream);
+
+/* Fully asynchronous form, with the contract of wp_encode_device_async: d_row_offsets[n_texts] is the row total, or
+ * UINT64_MAX if the id offsets are malformed or row_capacity is short.  In the UINT64_MAX case nothing is written to
+ * d_rows / d_mask and the other offsets are unspecified; repeat the call through wp_rows_device for the status. */
+wp_status wp_rows_device_async(wp_vocab *v, const int32_t *d_ids, size_t n_ids, const uint64_t *d_id_offsets,
+                               size_t n_texts, const wp_rows_spec *spec, int32_t *d_rows, uint8_t *d_mask,
+                               size_t row_capacity, uint64_t *d_row_offsets, void *stream);
 
 void wp_free(void *p);
 

@@ -1,7 +1,8 @@
 #!/usr/bin/env python3
 """Randomised parity sweep on a B200: hostile texts and vocabularies (tests/textgen.py) through randomly
 chosen entry points, range sizes and memo settings, every result compared with the CPU oracle (the device decode leg:
-random ids of the vocabulary, compared with the host wp_decode).
+random ids of the vocabulary, compared with the host wp_decode; the rows leg: the device batch's ids cut into model
+rows with a random spec, compared with the numpy model of tests/test_gpu_rows_device.py).
     python tools/fuzz_gpu.py [--seconds 120] [--seed0 1000]
 Prints one line per failure (with the seed to reproduce) and a summary; exit code 1 if anything differed."""
 from __future__ import annotations
@@ -23,6 +24,7 @@ import torch  # noqa: E402
 import textgen  # noqa: E402
 import wordpiece_b200  # noqa: E402
 from _oracle import Oracle  # noqa: E402
+from test_gpu_rows_device import model as rows_model  # noqa: E402
 
 
 def main():
@@ -61,13 +63,13 @@ def main():
             os.environ.pop("WORDPIECE_B200_PIPE_CHUNK", None)
         os.environ["WORDPIECE_B200_TICKET"] = "1" if rng.random() < 0.1 else "0"
         entry = rng.choice(["encode", "encode_into", "encode_into_pinned", "encode_device", "encode_text", "encode_batch",
-                            "encode_batch_device", "decode_device"])
+                            "encode_batch_device", "decode_device", "rows_device"])
         v = wordpiece_b200.Vocab(vocab, device=0)
         if rng.random() < 0.3:  # a handle that has already encoded something else (scratch, memo and shared memory in use)
             other, _ = textgen.case(seed + 77777, min(n, 200000), **kw)
             v.encode(other)
         try:
-            if entry in ("encode_batch", "encode_batch_device"):
+            if entry in ("encode_batch", "encode_batch_device", "rows_device"):
                 # the text cut at arbitrary BYTE positions (also inside a UTF-8 sequence, inside a word): every piece
                 # must get the ids the oracle gives that piece alone
                 k_cuts = rng.choice([0, 1, 3, 17, 200, 3000])
@@ -93,6 +95,21 @@ def main():
                                              device="cuda")
                     d_ids, d_offs, k = v.encode_batch_device(d_chars, d_offsets)
                     got, offs = d_ids[:k].cpu().numpy(), d_offs.cpu().numpy()
+                if entry == "rows_device":
+                    # a random spec over those ids: L, stride in [0, W], CLS / SEP present or not
+                    cls_id = rng.choice([None, 101, -5])
+                    sep_id = rng.choice([None, 102])
+                    max_len = (cls_id is not None) + (sep_id is not None) + rng.choice([1, 2, 7, 64, 509, 512])
+                    width = max_len - (cls_id is not None) - (sep_id is not None)
+                    stride = rng.choice([0, 1, width, rng.randint(0, width)])
+                    spec = dict(stride=stride, pad_id=rng.choice([0, -1]), cls_id=cls_id, sep_id=sep_id)
+                    if rows_model(got, offs, max_len, rows=[], **spec)[2][-1] * max_len > 20_000_000:
+                        spec["stride"] = 0  # (keeps the model's index matrix small on a long text)
+                    r, m, ro, n_rows = v.rows_device(d_ids[:k], d_offs, max_len, mask=rng.random() < 0.8, **spec)
+                    e_rows, e_mask, e_offs = rows_model(got, offs, max_len, **spec)
+                    assert n_rows == e_rows.shape[0] and np.array_equal(ro.cpu().numpy(), e_offs), "row offsets differ"
+                    assert np.array_equal(r.cpu().numpy(), e_rows), f"rows differ (L {max_len}, {spec})"
+                    assert m is None or np.array_equal(m.cpu().numpy(), e_mask), f"mask differs (L {max_len}, {spec})"
                 exp_offs = np.concatenate([[0], np.cumsum([len(e) for e in exp_parts])])
                 assert np.array_equal(np.asarray(offs, dtype=np.int64), exp_offs.astype(np.int64)), "text offsets differ"
             elif entry == "decode_device":

@@ -19,8 +19,11 @@ on every call, fast.cpp:21-35; a handle builds the device table once), whose
 batch calls the reference lacks: ``Vocab.encode_batch`` (host texts) and
 ``Vocab.encode_batch_device[_async]`` (a string column in GPU memory: uint8
 chars + int64 Arrow offsets in, ids + per-text id offsets in GPU memory out),
-and ``Vocab.decode_device[_async]`` (ids in GPU memory to one token string per
-id in the same column layout).
+``Vocab.decode_device[_async]`` (ids in GPU memory to one token string per
+id in the same column layout), and ``Vocab.rows_device[_async]`` /
+``Vocab.encode_rows_device`` (per-text ids, or a string column, to the
+fixed-length rows, special tokens, padding, overflow windows and attention
+mask a BERT-family model takes, in GPU memory).
 
 There is no CPU fallback: if the shared library is missing or no CUDA device is
 usable, calls raise.

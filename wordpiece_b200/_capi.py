@@ -47,6 +47,28 @@ class _StatsStruct(C.Structure):
     ]
 
 
+WP_ROWS_CLS = 1
+WP_ROWS_SEP = 2
+
+
+class RowsSpec(C.Structure):
+    """``wp_rows_spec``: row length, window stride (0 = truncate), pad / cls / sep ids, WP_ROWS_* flags."""
+
+    _fields_ = [
+        ("max_len", C.c_uint32),
+        ("stride", C.c_uint32),
+        ("pad_id", C.c_int32),
+        ("cls_id", C.c_int32),
+        ("sep_id", C.c_int32),
+        ("flags", C.c_uint32),
+    ]
+
+    @classmethod
+    def make(cls, max_len, stride=0, pad_id=0, cls_id=None, sep_id=None) -> "RowsSpec":
+        flags = (WP_ROWS_CLS if cls_id is not None else 0) | (WP_ROWS_SEP if sep_id is not None else 0)
+        return cls(max_len, stride, pad_id, 0 if cls_id is None else cls_id, 0 if sep_id is None else sep_id, flags)
+
+
 @dataclass
 class Stats:
     n_bytes: int
@@ -90,6 +112,8 @@ EXPORTED_SYMBOLS = [
     "wp_decode",
     "wp_decode_device",
     "wp_decode_device_async",
+    "wp_rows_device",
+    "wp_rows_device_async",
     "wp_free",
     "wp_debug_longest_match",
     "wp_debug_table_slots",
@@ -180,6 +204,11 @@ def load_library() -> C.CDLL:
         L.wp_decode_device.restype = C.c_int
         L.wp_decode_device_async.argtypes = [vp, vp, sz, vp, sz, vp, vp]
         L.wp_decode_device_async.restype = C.c_int
+    if hasattr(L, "wp_rows_device"):
+        L.wp_rows_device.argtypes = [vp, vp, sz, vp, sz, C.POINTER(RowsSpec), vp, vp, sz, vp, C.POINTER(sz), vp]
+        L.wp_rows_device.restype = C.c_int
+        L.wp_rows_device_async.argtypes = [vp, vp, sz, vp, sz, C.POINTER(RowsSpec), vp, vp, sz, vp, vp]
+        L.wp_rows_device_async.restype = C.c_int
     L.wp_free.argtypes = [vp]
     L.wp_free.restype = None
     L.wp_debug_longest_match.argtypes = [vp, C.c_char_p, sz, C.c_int, C.POINTER(C.c_uint32), C.POINTER(C.c_int32)]
@@ -583,6 +612,98 @@ class Vocab:
             stream = torch.cuda.current_stream(d_ids.device).cuda_stream
         _check(self._L.wp_decode_device_async(self._h, d_ids.data_ptr(), n_ids, d_chars.data_ptr(), d_chars.numel(),
                                               d_char_offsets.data_ptr(), stream))
+
+    # ---- model-input rows ---------------------------------------------
+    @staticmethod
+    def _rows_args(d_ids, d_id_offsets, d_rows, d_mask, d_row_offsets, max_len):
+        """(n_texts, row capacity, d_row_offsets) after checking the tensors; d_row_offsets allocated if None."""
+        import torch
+
+        assert d_ids.is_cuda and d_ids.dtype == torch.int32 and d_ids.dim() == 1 and d_ids.is_contiguous()
+        assert d_id_offsets.is_cuda and d_id_offsets.dtype == torch.int64 and d_id_offsets.dim() == 1
+        assert d_id_offsets.is_contiguous() and d_id_offsets.numel() >= 1, "n texts have n + 1 id offsets"
+        n_texts = d_id_offsets.numel() - 1
+        if d_row_offsets is None:
+            d_row_offsets = torch.empty(n_texts + 1, dtype=torch.int64, device=d_ids.device)
+        assert d_row_offsets.is_cuda and d_row_offsets.dtype == torch.int64 and d_row_offsets.is_contiguous()
+        assert d_row_offsets.numel() >= n_texts + 1, "n texts have n + 1 row offsets"
+        capacity = 0
+        if d_rows is not None:
+            assert d_rows.is_cuda and d_rows.dtype == torch.int32 and d_rows.is_contiguous()
+            capacity = d_rows.numel() // max(max_len, 1)
+        if d_mask is not None:
+            assert d_mask.is_cuda and d_mask.dtype == torch.uint8 and d_mask.is_contiguous()
+            assert d_mask.numel() >= capacity * max_len, "the mask holds as many rows as d_rows"
+        return n_texts, capacity, d_row_offsets
+
+    def rows_device(self, d_ids, d_id_offsets, max_len, stride=0, pad_id=0, cls_id=None, sep_id=None, mask=True,
+                    d_rows=None, d_mask=None, stream=None):
+        """Per-text ids in GPU memory -> fixed-length model-input rows.  ``wp_rows_device``.
+
+        Text t's ids are ``d_ids[d_id_offsets[t]:d_id_offsets[t + 1]]`` (int32 and int64 CUDA tensors, e.g. what
+        ``encode_batch_device`` returns).  Every row is ``max_len`` ids: ``[cls_id]? content [sep_id]? pad_id ...``
+        (cls / sep present when given), content width W = max_len minus the specials.  ``stride`` 0 truncates each
+        text to one row; 1 <= stride <= W cuts it into windows whose starts are ``stride`` ids apart (cuDF's meaning;
+        HuggingFace's overlap is W - stride).  Returns ``(d_rows [n_rows, max_len] int32, d_mask [n_rows, max_len]
+        uint8 or None, d_row_offsets int64 [n_texts + 1], n_rows)``; text t's rows are
+        ``d_row_offsets[t]:d_row_offsets[t + 1]``.  ``d_rows`` / ``d_mask`` may be preallocated contiguous tensors
+        (capacity = d_rows.numel() // max_len rows); otherwise the call asks for the row count first and allocates
+        exactly.  ``mask=False`` writes no mask.  Synchronises the stream."""
+        import torch
+
+        if not mask:
+            d_mask = None
+        elif d_mask is None and d_rows is not None:
+            d_mask = torch.empty(d_rows.numel() // max(max_len, 1) * max_len, dtype=torch.uint8, device=d_rows.device)
+        n_texts, capacity, d_row_offsets = self._rows_args(d_ids, d_id_offsets, d_rows, d_mask, None, max_len)
+        if stream is None:
+            stream = torch.cuda.current_stream(d_ids.device).cuda_stream
+        spec = RowsSpec.make(max_len, stride, pad_id, cls_id, sep_id)
+        cnt = C.c_size_t()
+
+        def call(rows, msk, cap):
+            return self._L.wp_rows_device(self._h, d_ids.data_ptr(), d_ids.numel(), d_id_offsets.data_ptr(), n_texts,
+                                          C.byref(spec), rows.data_ptr() if rows is not None else None,
+                                          msk.data_ptr() if msk is not None else None, cap, d_row_offsets.data_ptr(),
+                                          C.byref(cnt), stream)
+
+        st = call(d_rows, d_mask, capacity)
+        if d_rows is None and st in (WP_OK, WP_ERR_CAPACITY):  # the size query (with 0 rows it was the whole call)
+            d_rows = torch.empty((cnt.value, max_len), dtype=torch.int32, device=d_ids.device)
+            if mask and d_mask is None:
+                d_mask = torch.empty((cnt.value, max_len), dtype=torch.uint8, device=d_ids.device)
+            if st == WP_ERR_CAPACITY:
+                st = call(d_rows, d_mask, cnt.value)
+        _check(st)
+        n_rows = int(cnt.value)
+        d_rows = d_rows.view(-1)[: n_rows * max_len].view(n_rows, max_len)
+        if d_mask is not None:
+            d_mask = d_mask.view(-1)[: n_rows * max_len].view(n_rows, max_len)
+        return d_rows, d_mask, d_row_offsets, n_rows
+
+    def rows_device_async(self, d_ids, d_id_offsets, d_rows, d_row_offsets, max_len, stride=0, pad_id=0, cls_id=None,
+                          sep_id=None, d_mask=None, stream=None) -> None:
+        """Fully asynchronous variant of ``rows_device`` into preallocated tensors: the row total lands in
+        ``d_row_offsets[n_texts]``, which reads -1 (UINT64_MAX) if the id offsets are malformed or ``d_rows`` is too
+        small (then nothing is written to ``d_rows`` / ``d_mask``); repeat the call through ``rows_device`` for the
+        status.  ``wp_rows_device_async``."""
+        import torch
+
+        n_texts, capacity, d_row_offsets = self._rows_args(d_ids, d_id_offsets, d_rows, d_mask, d_row_offsets, max_len)
+        if stream is None:
+            stream = torch.cuda.current_stream(d_ids.device).cuda_stream
+        spec = RowsSpec.make(max_len, stride, pad_id, cls_id, sep_id)
+        _check(self._L.wp_rows_device_async(self._h, d_ids.data_ptr(), d_ids.numel(), d_id_offsets.data_ptr(), n_texts,
+                                            C.byref(spec), d_rows.data_ptr(), d_mask.data_ptr() if d_mask is not None else None,
+                                            capacity, d_row_offsets.data_ptr(), stream))
+
+    def encode_rows_device(self, d_chars, d_offsets, max_len, stride=0, pad_id=0, cls_id=None, sep_id=None, mask=True,
+                           stream=None):
+        """A string column in GPU memory -> model-input rows: ``encode_batch_device`` then ``rows_device`` (see
+        both).  Returns ``(d_rows, d_mask, d_row_offsets, n_rows)``."""
+        d_ids, d_id_offsets, n_ids = self.encode_batch_device(d_chars, d_offsets, stream=stream)
+        return self.rows_device(d_ids[:n_ids], d_id_offsets, max_len, stride=stride, pad_id=pad_id, cls_id=cls_id,
+                                sep_id=sep_id, mask=mask, stream=stream)
 
 
 # ---- the reference's stateless entry points ---------------------------------

@@ -198,7 +198,7 @@ struct wp_vocab {
   DeviceBuffer<uint2> d_dec_desc{16};
   DeviceBuffer<uint8_t> d_dec_bytes{16};
   bool dec_ready = false;
-  PinnedBuffer<unsigned long long> h_dec;  // the length pass's totals, for the synchronous call
+  PinnedBuffer<unsigned long long> h_totals;  // the first kernel's totals of a synchronous device decode or row call
   // every call on a handle shares its scratch, counters and word table: the kernels of one call must have
   // finished before those of the next begin, on whatever streams the caller enqueues them
   Event last_done;
@@ -1260,6 +1260,63 @@ wp_status enqueue_decode_total(wp_vocab *v, const int32_t *d_ids, size_t n_ids, 
   return WP_OK;
 }
 
+// ---- model-input rows (wp_rows_device): per-text ids -> fixed-length rows, counted, scanned and filled by row
+
+// Host-side checks shared by both row entry points: null arguments and the spec before the device, so that a
+// host-only handle reports them too
+wp_status check_rows_device(const wp_vocab *v, const int32_t *d_ids, size_t n_ids, const uint64_t *d_id_offsets,
+                            size_t n_texts, const wp_rows_spec *spec, const int32_t *d_rows, size_t row_capacity,
+                            const uint64_t *d_row_offsets) {
+  if (!v || !spec || !d_id_offsets || !d_row_offsets || (n_ids > 0 && !d_ids) || (row_capacity > 0 && !d_rows))
+    return fail(WP_ERR_INVALID_ARG, "null argument");
+  if (reinterpret_cast<uintptr_t>(d_rows) % alignof(int32_t) != 0)
+    return fail(WP_ERR_INVALID_ARG, "d_rows is not 4-byte aligned");
+  if (spec->flags & ~(WP_ROWS_CLS | WP_ROWS_SEP)) return fail(WP_ERR_INVALID_ARG, "unknown wp_rows_spec flags");
+  const uint32_t specials = ((spec->flags & WP_ROWS_CLS) ? 1u : 0u) + ((spec->flags & WP_ROWS_SEP) ? 1u : 0u);
+  if (spec->max_len <= specials) return fail(WP_ERR_INVALID_ARG, "max_len leaves no content position (W < 1)");
+  if (spec->stride > spec->max_len - specials) return fail(WP_ERR_INVALID_ARG, "stride exceeds the content width W");
+  if (row_capacity > SIZE_MAX / sizeof(int32_t) / spec->max_len)
+    return fail(WP_ERR_INVALID_ARG, "row_capacity * max_len overflows");
+  if (v->device < 0) return fail(WP_ERR_NO_DEVICE, kHostOnly);
+  if (n_texts / wp::rows_block_texts() >= 0xFFFFFFFFull) return fail(WP_ERR_INVALID_ARG, "too many texts for one call");
+  return WP_OK;
+}
+
+// The scan of a row call of n_texts > 0 texts on `stream`, behind the handle's previous call (it uses the handle's
+// scratch: the total, the malformed flag, the ticket and the look-back words, zeroed here).  *A <- the arguments of
+// both kernels.
+wp_status enqueue_rows_scan(wp_vocab *v, const int32_t *d_ids, size_t n_ids, const uint64_t *d_id_offsets,
+                            size_t n_texts, const wp_rows_spec *spec, int32_t *d_rows, uint8_t *d_mask,
+                            size_t row_capacity, uint64_t *d_row_offsets, cudaStream_t stream, wp::RowsArgs *A,
+                            uint64_t *launches) {
+  const size_t n_blocks = (n_texts + wp::rows_block_texts() - 1) / wp::rows_block_texts();
+  const size_t need = (3 + n_blocks) * sizeof(unsigned long long);
+  WP_CUDA(v->d_work.grow(need));
+  if (!v->last_done) WP_CUDA(cudaEventCreateWithFlags(&v->last_done.h, cudaEventDisableTiming));
+  WP_CUDA(cudaStreamWaitEvent(stream, v->last_done, 0));
+  WP_CUDA(cudaMemsetAsync(v->d_work.p, 0, need, stream));
+  *A = wp::RowsArgs{};
+  A->ids = d_ids;
+  A->n_ids = n_ids;
+  A->id_offsets = reinterpret_cast<const unsigned long long *>(d_id_offsets);
+  A->n_texts = n_texts;
+  A->cls = (spec->flags & WP_ROWS_CLS) ? 1u : 0u;
+  A->sep = (spec->flags & WP_ROWS_SEP) ? 1u : 0u;
+  A->max_len = spec->max_len;
+  A->width = spec->max_len - A->cls - A->sep;
+  A->stride = spec->stride;
+  A->pad_id = spec->pad_id;
+  A->cls_id = spec->cls_id;
+  A->sep_id = spec->sep_id;
+  A->rows = d_rows;
+  A->mask = d_mask;
+  A->capacity = row_capacity;
+  A->row_offsets = reinterpret_cast<unsigned long long *>(d_row_offsets);
+  A->work = reinterpret_cast<unsigned long long *>(v->d_work.p);
+  WP_CUDA(wp::launch_rows_scan(*A, v->sm_count, stream, launches));
+  return WP_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1860,22 +1917,81 @@ wp_status wp_decode_device(wp_vocab *v, const int32_t *d_ids, size_t n_ids, char
     WP_CUDA(cudaStreamSynchronize(s));
     return WP_OK;
   }
-  WP_CUDA(v->h_dec.grow(3));
+  WP_CUDA(v->h_totals.grow(3));
   wp::DecodeArgs A;
   uint64_t launches = 0;
   st = enqueue_decode_total(v, d_ids, n_ids, d_chars, capacity, d_char_offsets, s, &A, &launches);
   g_launches.fetch_add(std::exchange(launches, 0), std::memory_order_relaxed);
   if (st != WP_OK) return st;
-  WP_CUDA(cudaMemcpyAsync(v->h_dec.p, v->d_work.p, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+  WP_CUDA(cudaMemcpyAsync(v->h_totals.p, v->d_work.p, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
   WP_CUDA(cudaEventRecord(v->last_done, s));
   WP_CUDA(cudaStreamSynchronize(s));
-  const unsigned long long bytes = v->h_dec.p[0], skipped = v->h_dec.p[1], bad = v->h_dec.p[2];
+  const unsigned long long bytes = v->h_totals.p[0], skipped = v->h_totals.p[1], bad = v->h_totals.p[2];
   if (bad) return fail(WP_ERR_ID_RANGE, "token id equals vocabulary size");  // fast.cpp:175 .at()
   *n_chars = static_cast<size_t>(bytes);
   if (n_skipped) *n_skipped = static_cast<size_t>(skipped);
   if (bytes > capacity) return fail(WP_ERR_CAPACITY, "char buffer too small");
   // (the scratch still holds the totals and zeroed look-back words: nothing ran on it since the length pass)
   WP_CUDA(wp::launch_decode(A, v->sm_count, s, &launches));
+  g_launches.fetch_add(launches, std::memory_order_relaxed);
+  WP_CUDA(cudaEventRecord(v->last_done, s));
+  WP_CUDA(cudaStreamSynchronize(s));
+  return WP_OK;
+}
+
+wp_status wp_rows_device_async(wp_vocab *v, const int32_t *d_ids, size_t n_ids, const uint64_t *d_id_offsets,
+                               size_t n_texts, const wp_rows_spec *spec, int32_t *d_rows, uint8_t *d_mask,
+                               size_t row_capacity, uint64_t *d_row_offsets, void *stream) {
+  wp_status st = check_rows_device(v, d_ids, n_ids, d_id_offsets, n_texts, spec, d_rows, row_capacity, d_row_offsets);
+  if (st != WP_OK) return st;
+  DeviceGuard g(v->device);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (n_texts == 0) {
+    WP_CUDA(cudaMemsetAsync(d_row_offsets, 0, sizeof(uint64_t), s));
+    return WP_OK;
+  }
+  wp::RowsArgs A;
+  uint64_t launches = 0;
+  st = enqueue_rows_scan(v, d_ids, n_ids, d_id_offsets, n_texts, spec, d_rows, d_mask, row_capacity, d_row_offsets, s,
+                         &A, &launches);
+  g_launches.fetch_add(std::exchange(launches, 0), std::memory_order_relaxed);
+  if (st != WP_OK) return st;
+  WP_CUDA(wp::launch_rows_fill(A, v->sm_count, s, &launches));
+  g_launches.fetch_add(launches, std::memory_order_relaxed);
+  WP_CUDA(cudaEventRecord(v->last_done, s));  // the scratch is free once the fill has read the total
+  return WP_OK;
+}
+
+wp_status wp_rows_device(wp_vocab *v, const int32_t *d_ids, size_t n_ids, const uint64_t *d_id_offsets, size_t n_texts,
+                         const wp_rows_spec *spec, int32_t *d_rows, uint8_t *d_mask, size_t row_capacity,
+                         uint64_t *d_row_offsets, size_t *n_rows, void *stream) {
+  if (!n_rows) return fail(WP_ERR_INVALID_ARG, "null argument");
+  *n_rows = 0;
+  wp_status st = check_rows_device(v, d_ids, n_ids, d_id_offsets, n_texts, spec, d_rows, row_capacity, d_row_offsets);
+  if (st != WP_OK) return st;
+  DeviceGuard g(v->device);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (n_texts == 0) {
+    WP_CUDA(cudaMemsetAsync(d_row_offsets, 0, sizeof(uint64_t), s));
+    WP_CUDA(cudaStreamSynchronize(s));
+    return WP_OK;
+  }
+  WP_CUDA(v->h_totals.grow(2));
+  wp::RowsArgs A;
+  uint64_t launches = 0;
+  st = enqueue_rows_scan(v, d_ids, n_ids, d_id_offsets, n_texts, spec, d_rows, d_mask, row_capacity, d_row_offsets, s,
+                         &A, &launches);
+  g_launches.fetch_add(std::exchange(launches, 0), std::memory_order_relaxed);
+  if (st != WP_OK) return st;
+  WP_CUDA(cudaMemcpyAsync(v->h_totals.p, v->d_work.p, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+  WP_CUDA(cudaEventRecord(v->last_done, s));
+  WP_CUDA(cudaStreamSynchronize(s));
+  const unsigned long long rows = v->h_totals.p[0], bad = v->h_totals.p[1];
+  if (bad) return fail(WP_ERR_INVALID_ARG, "id offsets descend or end past n_ids");
+  *n_rows = static_cast<size_t>(rows);
+  if (rows > row_capacity) return fail(WP_ERR_CAPACITY, "row buffer too small");
+  // (the scratch still holds the total and the flag: nothing ran on it since the scan)
+  WP_CUDA(wp::launch_rows_fill(A, v->sm_count, s, &launches));
   g_launches.fetch_add(launches, std::memory_order_relaxed);
   WP_CUDA(cudaEventRecord(v->last_done, s));
   WP_CUDA(cudaStreamSynchronize(s));

@@ -2545,6 +2545,230 @@ cudaError_t launch_decode(const DecodeArgs &A, int sm_count, cudaStream_t stream
   return cudaGetLastError();
 }
 
+// ============================================================== model-input rows
+//
+// Per-text ids (ids + Arrow id offsets) -> fixed-length rows of max_len ids: [cls]? content [sep]? pad ..., and a
+// mask that is 1 on cls, content and sep.  Text t of n_t ids has r_t = 1 row if stride == 0 or n_t <= W, else
+// 1 + ceil((n_t - W) / stride); row k holds the text's ids [k stride, min(k stride + W, n_t)).  The shape of the
+// decode pair: a scan kernel hands out blocks of 2 048 texts by ticket, counts their rows, scans them (64-bit block
+// scan, decoupled look-back) and writes the row offsets; the fill kernel is driven by ROW, so that one text of
+// millions of rows spreads over the whole GPU.  Each CTA takes tiles of ROWS_TILE consecutive rows: one 32-way
+// search over the row offsets finds the tile's first text, the tile's texts (at most ROWS_TILE, every text has a
+// row) are staged in shared memory, and each warp writes whole rows.  A row is a span of the flat output: its
+// interior goes out in 16-byte stores, only its ends (< 16 bytes each) in 4-byte (ids) or 1-byte (mask) stores.
+
+constexpr int ROWS_THREADS = 256;
+constexpr int ROWS_ITEMS = 8;
+constexpr int ROWS_TEXTS = ROWS_THREADS * ROWS_ITEMS;  // 2048 texts per scan block
+constexpr int ROWS_SCAN_BLOCKS = 4;                    // scan CTAs per SM (launch bound and grid)
+constexpr int ROWS_TILE = 128;                         // rows per fill tile
+constexpr int ROWS_FILL_BLOCKS = 6;                    // fill CTAs per SM (launch bound and grid)
+
+// rows of text t; *bad |= its offsets descend or end past n_ids (such a text counts one row: the call is void)
+__device__ __forceinline__ unsigned long long rows_of_text(const RowsArgs &A, unsigned long long t, bool *bad) {
+  WP_CHECK(t < A.n_texts);
+  const unsigned long long a = A.id_offsets[t], b = A.id_offsets[t + 1];
+  if (a > b || b > A.n_ids) {
+    *bad = true;
+    return 1ull;
+  }
+  const unsigned long long n = b - a;
+  return A.stride == 0u || n <= A.width ? 1ull : 1ull + (n - A.width + A.stride - 1u) / A.stride;
+}
+
+struct RowsScanSmem {
+  unsigned long long rel[ROWS_TEXTS];  // the block's row offsets relative to its first row
+  unsigned long long warp_sums[ROWS_THREADS / 32];
+  uint32_t block_index;
+  unsigned long long base;
+};
+
+__global__ void __launch_bounds__(ROWS_THREADS, ROWS_SCAN_BLOCKS) wp_rows_scan_kernel(RowsArgs A) {
+  __shared__ RowsScanSmem sm;
+  const int tid = threadIdx.x;
+  const int lane = tid & 31;
+  const unsigned long long n = A.n_texts;
+  unsigned long long *const block_state = A.work + 3;
+  unsigned int *const ticket = reinterpret_cast<unsigned int *>(A.work + 2);
+  const uint32_t n_blocks = static_cast<uint32_t>((n + ROWS_TEXTS - 1) / ROWS_TEXTS);
+  bool bad = false;
+  for (;;) {
+    __syncthreads();
+    if (tid == 0) sm.block_index = atomicAdd(ticket, 1u);
+    __syncthreads();
+    const uint32_t b = sm.block_index;
+    if (b >= n_blocks) break;
+    const unsigned long long block_first = static_cast<unsigned long long>(b) * ROWS_TEXTS;
+    const uint32_t count = static_cast<uint32_t>(n - block_first < ROWS_TEXTS ? n - block_first : ROWS_TEXTS);
+    const uint32_t first = tid * ROWS_ITEMS;  // within the block
+    unsigned long long r[ROWS_ITEMS], mine = 0;
+#pragma unroll
+    for (int j = 0; j < ROWS_ITEMS; j++) {
+      r[j] = first + j < count ? rows_of_text(A, block_first + first + j, &bad) : 0ull;
+      mine += r[j];
+    }
+    unsigned long long total;
+    unsigned long long at = block_exclusive_scan<ROWS_THREADS / 32>(sm.warp_sums, mine, &total);
+    if (tid == 0) lookback_publish(block_state, b, total);
+#pragma unroll
+    for (int j = 0; j < ROWS_ITEMS; j++) {
+      if (first + j < count) {
+        WP_CHECK(first + j < ROWS_TEXTS);
+        sm.rel[first + j] = at;
+      }
+      at += r[j];
+    }
+    __syncthreads();
+    if (tid < 32) {
+      const unsigned long long base = lookback_walk(block_state, b, total, lane);
+      if (lane == 0) sm.base = base;
+    }
+    __syncthreads();
+    const unsigned long long base = sm.base;
+    for (uint32_t i = tid; i < count; i += ROWS_THREADS) {
+      WP_CHECK(block_first + i < n);
+      A.row_offsets[block_first + i] = base + sm.rel[i];
+    }
+    if (block_first + count == n && tid == 0) {
+      A.row_offsets[n] = base + total;
+      A.work[0] = base + total;
+    }
+  }
+  bad = __syncthreads_or(bad);
+  if (bad && tid == 0) atomicOr(&A.work[1], 1ull);
+}
+
+struct RowsFillSmem {
+  unsigned long long row_off[ROWS_TILE + 1];  // row and id offsets of the texts t0 .. t0 + n_local
+  unsigned long long id_off[ROWS_TILE + 1];
+  unsigned long long t0;                      // the text of the tile's first row
+};
+
+// 16 mask bytes starting at column c: byte i is 1 if c + i < valid
+__device__ __forceinline__ uint4 mask_unit(uint32_t c, uint32_t valid) {
+  const uint32_t ones = valid > c ? (valid - c < 16u ? valid - c : 16u) : 0u;
+  uint32_t w[4];
+#pragma unroll
+  for (int k = 0; k < 4; k++) {
+    const uint32_t m = ones > 4u * k ? (ones - 4u * k < 4u ? ones - 4u * k : 4u) : 0u;
+    w[k] = m == 4u ? 0x01010101u : 0x01010101u & ((1u << (8u * m)) - 1u);
+  }
+  return make_uint4(w[0], w[1], w[2], w[3]);
+}
+
+__global__ void __launch_bounds__(ROWS_THREADS, ROWS_FILL_BLOCKS) wp_rows_fill_kernel(RowsArgs A) {
+  __shared__ RowsFillSmem sm;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const unsigned long long total = A.work[0];
+  // (an async call whose offsets are malformed, or that needs more rows than capacity, writes only the void count)
+  if (A.work[1] != 0ull || total > A.capacity) {
+    if (blockIdx.x == 0 && tid == 0) A.row_offsets[A.n_texts] = ~0ull;
+    return;
+  }
+  const uint32_t L = A.max_len;
+  const unsigned long long n_tiles = (total + ROWS_TILE - 1) / ROWS_TILE;
+  for (unsigned long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    const unsigned long long r0 = tile * ROWS_TILE;
+    const unsigned long long r1 = total - r0 < ROWS_TILE ? total : r0 + ROWS_TILE;
+    __syncthreads();  // (the previous tile's texts are no longer read)
+    if (warp == 0) {
+      // the first j in [1, n_texts) with row_offsets[j] > r0 (n_texts if none): a 32-way search; the row offsets
+      // ascend strictly (every text has a row), so text j - 1 holds row r0
+      unsigned long long lo = 1, hi = A.n_texts;
+      while (hi > lo) {
+        const unsigned long long span = hi - lo;
+        const unsigned long long p = lo + span * lane / 32;
+        WP_CHECK(p < A.n_texts);
+        const uint32_t gt = __ballot_sync(FULL, A.row_offsets[p] > r0);
+        const int k = gt ? __ffs(gt) - 1 : 32;  // lanes probe ascending positions: the first lane past r0
+        const unsigned long long nhi = k < 32 ? lo + span * k / 32 : hi;
+        lo = k > 0 ? lo + span * (k - 1) / 32 + 1 : lo;
+        hi = nhi;
+      }
+      if (lane == 0) sm.t0 = lo - 1;
+    }
+    __syncthreads();
+    const unsigned long long t0 = sm.t0;
+    const uint32_t n_local = static_cast<uint32_t>(A.n_texts - t0 < ROWS_TILE ? A.n_texts - t0 : ROWS_TILE);
+    for (uint32_t i = tid; i <= n_local; i += ROWS_THREADS) {
+      WP_CHECK(t0 + i <= A.n_texts);
+      sm.row_off[i] = A.row_offsets[t0 + i];
+      sm.id_off[i] = A.id_offsets[t0 + i];
+    }
+    __syncthreads();
+    for (unsigned long long r = r0 + warp; r < r1; r += ROWS_THREADS / 32) {
+      // the row's text: the last i with row_off[i] <= r (row_off[0] <= r0 <= r < r1 <= row_off[n_local])
+      uint32_t lo = 0, hi = n_local;
+      while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (sm.row_off[mid] <= r) lo = mid;
+        else hi = mid;
+      }
+      const unsigned long long k = r - sm.row_off[lo];
+      const unsigned long long n_t = sm.id_off[lo + 1] - sm.id_off[lo];
+      const unsigned long long from = sm.id_off[lo] + k * A.stride;  // (k = 0 when stride == 0)
+      WP_CHECK(k * A.stride <= n_t);
+      const uint32_t len = static_cast<uint32_t>(n_t - k * A.stride < A.width ? n_t - k * A.stride : A.width);
+      const uint32_t valid = A.cls + len + A.sep;
+      auto value = [&](uint32_t c) -> int32_t {
+        if (c < A.cls) return A.cls_id;
+        const uint32_t j = c - A.cls;
+        if (j < len) {
+          WP_CHECK(from + j < A.n_ids);
+          return __ldg(A.ids + from + j);
+        }
+        return j == len && A.sep ? A.sep_id : A.pad_id;
+      };
+      WP_CHECK(r < A.capacity);
+      // ids: [0, head) and [body, L) one by one, [head, body) in 16-byte units
+      int32_t *const row = A.rows + r * L;
+      uint32_t head = ((16u - (reinterpret_cast<uintptr_t>(row) & 15u)) & 15u) >> 2;
+      head = head < L ? head : L;
+      const uint32_t body = head + ((L - head) & ~3u);
+      for (uint32_t e = lane; e < head + (L - body); e += 32) {
+        const uint32_t c = e < head ? e : body + (e - head);
+        WP_CHECK(c < L);
+        row[c] = value(c);
+      }
+      for (uint32_t c = head + 4u * lane; c < body; c += 128u) {
+        WP_CHECK(c + 4u <= L);
+        *reinterpret_cast<int4 *>(row + c) = make_int4(value(c), value(c + 1), value(c + 2), value(c + 3));
+      }
+      if (A.mask != nullptr) {
+        uint8_t *const mrow = A.mask + r * L;
+        uint32_t mhead = (16u - (reinterpret_cast<uintptr_t>(mrow) & 15u)) & 15u;
+        mhead = mhead < L ? mhead : L;
+        const uint32_t mbody = mhead + ((L - mhead) & ~15u);
+        for (uint32_t e = lane; e < mhead + (L - mbody); e += 32) {
+          const uint32_t c = e < mhead ? e : mbody + (e - mhead);
+          WP_CHECK(c < L);
+          mrow[c] = c < valid ? 1u : 0u;
+        }
+        for (uint32_t c = mhead + 16u * lane; c < mbody; c += 512u) {
+          WP_CHECK(c + 16u <= L);
+          *reinterpret_cast<uint4 *>(mrow + c) = mask_unit(c, valid);
+        }
+      }
+    }
+  }
+}
+
+uint32_t rows_block_texts() { return ROWS_TEXTS; }
+
+cudaError_t launch_rows_scan(const RowsArgs &A, int sm_count, cudaStream_t stream, uint64_t *launches) {
+  if (sm_count <= 0) sm_count = 148;
+  wp_rows_scan_kernel<<<sm_count * ROWS_SCAN_BLOCKS, ROWS_THREADS, 0, stream>>>(A);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_rows_fill(const RowsArgs &A, int sm_count, cudaStream_t stream, uint64_t *launches) {
+  if (sm_count <= 0) sm_count = 148;
+  wp_rows_fill_kernel<<<sm_count * ROWS_FILL_BLOCKS, ROWS_THREADS, 0, stream>>>(A);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
 // ------------------------------------------------------------ word-table seed
 // Every encode call that records words starts from a working table that holds exactly the static words.
 __global__ void wp_seed_words_kernel(const WordSlot *__restrict__ image, uint32_t image_slots, WordSlot *work,

@@ -209,4 +209,30 @@ cudaError_t launch_decode_total(const DecodeArgs &A, int sm_count, cudaStream_t 
 // UINT64_MAX.
 cudaError_t launch_decode(const DecodeArgs &A, int sm_count, cudaStream_t stream, uint64_t *launches);
 
+// Model-input rows (wp_rows_device): per-text ids -> rows of max_len ids, [cls]? content [sep]? pad ..., and a mask.
+struct RowsArgs {
+  const int32_t *ids;
+  unsigned long long n_ids;
+  const unsigned long long *id_offsets;  // n_texts + 1 entries, ascending, the last <= n_ids
+  unsigned long long n_texts;
+  uint32_t max_len;                      // L
+  uint32_t width;                        // W = L - cls - sep >= 1: content ids per row
+  uint32_t stride;                       // 0: one truncated row per text; else 1 <= stride <= W
+  uint32_t cls, sep;                     // 1 if the row has the token, else 0
+  int32_t pad_id, cls_id, sep_id;
+  int32_t *rows;                         // capacity rows of L ids (4-byte aligned)
+  uint8_t *mask;                         // capacity rows of L bytes, or nullptr
+  unsigned long long capacity;           // rows
+  unsigned long long *row_offsets;       // n_texts + 1 entries
+  // scratch (zeroed): [0] total rows, [1] malformed offsets were seen, [2] ticket, [3 ...] one look-back word per
+  // rows_block_texts() texts
+  unsigned long long *work;
+};
+uint32_t rows_block_texts();
+// Writes row_offsets[0 .. n_texts] (exact if the offsets are well formed), the total to work[0], and sets work[1]
+// if the id offsets descend or end past n_ids.
+cudaError_t launch_rows_scan(const RowsArgs &A, int sm_count, cudaStream_t stream, uint64_t *launches);
+// Writes the rows and the mask, or, if work[1] is set or work[0] > capacity, only row_offsets[n_texts] = UINT64_MAX.
+cudaError_t launch_rows_fill(const RowsArgs &A, int sm_count, cudaStream_t stream, uint64_t *launches);
+
 }  // namespace wp
